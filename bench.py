@@ -373,6 +373,18 @@ def run_gpu_arm(args):
         dp_parity = {"rays": 4096, "tol": 1e-4,
                      "rel_l2": hn_train.dp_parity_check(model, fg, rays_all[:4096].to(dev), rgbs_all[:4096].to(dev), tol=1e-4)}
     opt = hn_train.FusedAdam(fg, lr=5e-4, eps=1e-8)   # Adam of utils/__init__.py:29-31 / opt.py:53-56, one launch
+    # Every timed step trains from this initial state (weights, Adam moments and step count, restored outside the events).
+    # The backward kernels reduce with float atomics, so a step is reproducible only up to rounding, and a chain of Adam
+    # steps amplifies that rounding until two runs train different models; from one fixed state, the same arguments give
+    # the same outputs from run to run.
+    params0 = opt.flat.clone()
+    opt_state0 = {k: v.clone() if torch.is_tensor(v) else v for k, v in opt.state_dict().items()}
+
+    @torch.no_grad()
+    def restore_train_state():
+        opt.flat.copy_(params0)
+        torch.autograd.graph.increment_version(fg.params)   # the models' packed-weight caches key on the version counters
+        opt.load_state_dict(opt_state0)
 
     # inputs: this rank's contiguous shard of the global batch, resident in HBM (value) and in pinned host memory (e2e)
     lo, hi = hn_train.shard_bounds(GLOBAL_RAYS, rank, world)
@@ -396,15 +408,17 @@ def run_gpu_arm(args):
         step(rays_d, rgbs_d)
     sync_all()
 
-    def timed_loop(fn, steps, profile=False):
-        """EXACTLY `steps` steps; device time by CUDA events on the launching stream, L2 flushed between steps
-        (outside the events); returns (seconds summed over steps, max over ranks; launches; per-kernel events)."""
+    def timed_loop(fn, steps, profile=False, before=None):
+        """EXACTLY `steps` steps; device time by CUDA events on the launching stream, `before` and an L2 flush between
+        steps (outside the events); returns (seconds summed over steps, max over ranks; launches; per-kernel events)."""
         evs = []
         launches0 = _lib.launches
         if profile:
             _lib.profile = []
         sync_all()
         for _ in range(steps):
+            if before is not None:
+                before()
             l2_flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
@@ -419,11 +433,20 @@ def run_gpu_arm(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item()), _lib.launches - launches0, prof
 
+    last = {}
+
+    def timed_step():
+        last["loss"] = step(rays_d, rgbs_d)
+
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
-    secs, launches, prof = timed_loop(lambda: step(rays_d, rgbs_d), args.steps, profile=True)
+    secs, launches, prof = timed_loop(timed_step, args.steps, profile=True, before=restore_train_state)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # what a caller of the train step holds after the last timed step, before the other legs train further: the loss,
+        # the all-reduced gradient and the Adam-updated parameters (flat buffers, FlatGrads order incl. padding; 5.9 MB each)
+        dump_outputs(args.dump_outputs, {"loss": last["loss"], "grads": fg.flat, "params": opt.flat})
 
     # end to end: host rows in, loss out, every step
     loss_h = torch.empty((), dtype=torch.float32).pin_memory()
@@ -637,6 +660,8 @@ def run_gpu_arm(args):
             "config": {"workload": WORKLOAD, "global_rays": GLOBAL_RAYS, "rays_per_gpu": hi - lo, "chunk_rays": chunk,
                        "samples": f"{N_COARSE}+{N_FINE}", "parallelism": f"dp{world} (ray shards, 1 flat NCCL all-reduce/step)",
                        "optimizer": "Adam step inside the timed region", "timing": "CUDA events per step, max over ranks",
+                       "train_state": "every timed step starts from the initial weights and Adam state (restored between steps, "
+                                      "outside the events)",
                        "l2": "256 MB buffer written between timed steps; per-step working set (>10 GB) exceeds L2",
                        "flop_accounting": "roofline.* count EXECUTED unpadded FLOPs (the fine level's 64 inherited depths skip "
                                           "the shared warp / sheet nets: 874.3 MFLOP per ray instead of the reference's 923.4)",
@@ -650,6 +675,14 @@ def run_gpu_arm(args):
         emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor of `arrays` as float32 to out_dir/<name>.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 _REAL_STDOUT = None
@@ -689,7 +722,12 @@ def main():
     ap.add_argument("--graph-chunk", type=int, default=16384, help="rays per chunk inside the CUDA graph of the end-to-end path")
     ap.add_argument("--no-graph", action="store_true", help="end-to-end path: launch the chunk loop eagerly instead of from a CUDA graph")
     ap.add_argument("--se3-steps", type=int, default=3, help="timed steps of the cfg5 leg (>= 3)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed train steps, write the last step's loss, gradient and updated parameters as "
+                         "float32 DIR/<name>.npy (inputs and draws are seeded: same arguments, same inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
