@@ -29,7 +29,7 @@ EXPORTS = [
 ]
 # microbenchmarks / descriptor probes: their own library and header (include/hypernerf_b200_probe.h), not the product ABI
 PROBE_LIB_PATH = os.path.join(_HERE, "libhypernerf_b200_probe.so")
-PROBE_EXPORTS = ["hn_set_sm_partition", "hn_umma_probe", "hn_umma_probe2", "hn_umma_rate", "hn_umma_rate2", "hn_umma_rate3", "hn_umma_rate4",
+PROBE_EXPORTS = ["hn_umma_probe", "hn_umma_probe2", "hn_umma_rate", "hn_umma_rate2", "hn_umma_rate3", "hn_umma_rate4",
                  "hn_epi_rate", "hn_tmem_rate", "hn_overlap_rate"]
 
 
@@ -76,8 +76,6 @@ def lib():
     L.hn_abi_version.restype = C.c_int
     L.hn_last_error.restype = C.c_char_p
     L.hn_query.argtypes = [C.POINTER(ModelDesc), i64, C.POINTER(Sizes)]
-    L.hn_set_sm_partition.argtypes = [i32, i32]      # declared in the probe header: a scheduling experiment, not the ABI
-    L.hn_set_sm_partition.restype = C.c_int
     L.hn_pack_weights.argtypes = [C.POINTER(ModelDesc), vp, C.POINTER(C.c_int64), i32, vp, vp]
     L.hn_sample_coarse.argtypes = [vp, vp, vp, vp, vp, i64, i32, vp, vp, vp]
     L.hn_sample_pdf.argtypes = [vp, vp, vp, i64, vp, vp, vp, i64, i32, i32, i32, vp, vp, vp, vp]

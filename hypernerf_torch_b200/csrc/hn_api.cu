@@ -31,19 +31,7 @@ int num_sms() {
   return cached;
 }
 
-// SM partition (hn_set_sm_partition): caps on the persistent grids of the forward / data-gradient kernels and of the
-// weight-gradient kernel, so that a weight-gradient launch on a second stream runs beside them on the SMs they leave free.
-static int g_mlp_ctas = 0, g_wgrad_ctas = 0;
-int mlp_grid_cap() { const int n = num_sms(); return g_mlp_ctas > 0 && g_mlp_ctas < n ? g_mlp_ctas : n; }
-int wgrad_grid_cap() { const int n = num_sms(); return g_wgrad_ctas > 0 && g_wgrad_ctas < n ? g_wgrad_ctas : n; }
-
 }  // namespace hn
 
-extern "C" int hn_set_sm_partition(int mlp_ctas, int wgrad_ctas) {
-  if (mlp_ctas < 0 || wgrad_ctas < 0) return hn::set_error(-1, "hn_set_sm_partition: negative CTA count");
-  hn::g_mlp_ctas = mlp_ctas;
-  hn::g_wgrad_ctas = wgrad_ctas;
-  return 0;
-}
 extern "C" int hn_abi_version(void) { return HN_ABI_VERSION; }
 extern "C" const char* hn_last_error(void) { return hn::g_err; }

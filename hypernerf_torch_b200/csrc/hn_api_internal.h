@@ -10,6 +10,4 @@ namespace hn {
 int set_error(int code, const char* msg);
 int set_cuda_error(cudaError_t e, const char* where);  // returns 0 when e == cudaSuccess
 int num_sms();                                         // cached SM count of the current device
-int mlp_grid_cap();                                    // num_sms() or the hn_set_sm_partition cap (forward / data gradient)
-int wgrad_grid_cap();                                  // the same for the weight-gradient kernel
 }  // namespace hn

@@ -17,31 +17,22 @@
 // ring; 5-6 stages in the data gradient) and the UMMA issuer (one elected thread) and gives its registers away.
 // TMEM: 512 columns = 2 sub-tiles x 256 fp32 accumulator columns.  Stash stores are streaming (st.global.cs).
 #include <math.h>
-#include <stdlib.h>
 #include <algorithm>
 #include <string.h>
-#include <mutex>
 #include <type_traits>
 #include <unordered_map>
-#include <cuda.h>          // CUtensorMap (types only; the encoder is resolved through cudaGetDriverEntryPoint)
-#include <cudaTypedefs.h>
 #include "hn_api_internal.h"
 #include "hn_mlp_program.h"
 #include "hn_ptx.cuh"
 
 // This file is compiled twice into libhypernerf_b200.so (Makefile).  The second compilation (hn_mlp_fv.o:
-// -DHN_MLP_FWD_VARIANT=1 -DHN_EPI_SPLIT=2 + register budgets) holds the FORWARD kernels with two epilogue warpgroups per
-// sub-tile, in their own namespace, and exports only hn_mlp_fwd_fv / hn_mlp_fwd_trunk_fv, which the first compilation's
-// hn_mlp_fwd / hn_mlp_fwd_trunk call for INFERENCE launches (HN_FWD_VARIANT_LINKED; HN_FWD_VARIANT = 0 / 1 / 2 in the
-// environment: never / every forward / inference only, the default).  Measured per 1 M samples in isolation: inference
-// forward 2.03 -> 1.93 ms, training forward 2.50 -> 2.42 ms, data gradient +2 % (hence per kernel, not a global switch);
-// a full-frame render goes from 2.27 to 2.40 Mrays/s, while inside the power-capped training step the split training
-// forward is a wash (690 k against 691 k rays/s over three alternating runs, the trunk-only launch 3 % slower), so training
-// keeps the single-warpgroup kernels.  The stash / gate-word layout does not depend on the epilogue split (all GPU tests pass
-// with HN_FWD_VARIANT=1: the backward kernels of the first compilation read what these forwards wrote).
-#ifndef HN_FWD_VARIANT_DEFAULT
-#define HN_FWD_VARIANT_DEFAULT 2
-#endif
+// -DHN_MLP_FWD_VARIANT=1) holds the INFERENCE forward kernels with two epilogue warpgroups per sub-tile (hn_mlp_program.h:
+// kEpiSplit), in their own namespace, and exports only hn_mlp_fwd_fv / hn_mlp_fwd_trunk_fv, which the first compilation's
+// hn_mlp_fwd / hn_mlp_fwd_trunk call for every launch without a stash.  Measured per 1 M samples in isolation: inference
+// forward 2.03 -> 1.93 ms, training forward 2.50 -> 2.42 ms, data gradient +2 %; a full-frame render goes from 2.27 to
+// 2.40 Mrays/s, while inside the power-capped training step the split training forward is a wash (690 k against 691 k
+// rays/s over three alternating runs, the trunk-only launch 3 % slower), so training keeps the single-warpgroup kernels.
+// The stash / gate-word layout does not depend on the epilogue split.
 #ifdef HN_MLP_FWD_VARIANT
 namespace hn_fv { using namespace hn; }
 #define hn hn_fv
@@ -78,7 +69,7 @@ struct Shape {
   static constexpr int PE_X = 3 + 6 * XF, PE_H = H * (1 + 2 * HF), IN_T = PE_X + PE_H, KT = pad16(IN_T);
   static constexpr int PE_V = 3 + 6 * VF, KV = STATIC ? pad16(PE_V) : kKV;
   static constexpr bool TIN_ACT = !STATIC && trunk_in_act(KT);   // trunk input vector in ACT (hn_mlp_program.h: kMaxTrunkInInb)
-  // bias folding (hn_mlp_program.h: HN_FOLD_BIAS): the last two columns of INB's last chunk pair hold 1.0; they sit in
+  // bias folding (hn_mlp_program.h): the last two columns of INB's last chunk pair hold 1.0; they sit in
   // the zero padding of the widest input vector when every vector that reaches the last chunk has >= 2 pad columns
   static constexpr int INB_CHUNKS = STATIC ? inb_chunks_of(KW, IN_W, 0, 0, KV, PE_V) : inb_chunks_of(KW, IN_W, KT, IN_T, KV, PE_V);
   static constexpr int N_RGB0A = pad16(kRgbW + 1);
@@ -99,99 +90,29 @@ using CfgSE3 = Shape<8, 8, kSe3Freqs, 0, 10, 6, 6, false, true>;   // config 5: 
 // stash stores) runs under sub-tile 1's UMMAs and vice versa.  Price: every weight stage is fetched from L2 once per
 // 128 instead of once per 256 samples, i.e. the weight ring has to sustain twice the rate over the same ~1 100-cycle
 // refill latency.  Lock step: both sub-tiles consume each stage back to back.
-// HN_PINGPONG bits: 1 = training forward, 2 = data gradient, 4 = inference forward.  Measured per 1 M samples once
-// the stash stores stopped evicting the weights from L2 (streaming stores): data gradient (80 KB ring) 2.55 -> 2.31 ms,
-// training forward (48 KB ring) 2.50 -> 2.42 ms, inference forward (48 KB ring, short drains, bias K steps streamed
-// twice) 1.89 -> 2.34 ms.  Before the streaming stores none of the three gained anything.
-#ifndef HN_PINGPONG
-#define HN_PINGPONG 3
-#endif
-// L2 cache policies on the bulk loads: bit 0 = evict_last for the weight stream of the forward / data-gradient kernels,
-// bit 1 = evict_first for the stash slabs the weight-gradient kernel streams through.  Measured with the streaming
-// stash stores in place: no effect on forward / data gradient, weight gradient 2.92 -> 2.97 ms; off.
-#ifndef HN_L2_HINTS
-#define HN_L2_HINTS 0
-#endif
-// HN_FOLD_BIAS_TRAIN = 1: the stash-writing forward also carries its biases in the UMMAs (one extra K = 16 step per op)
-// instead of 8 LDS + 32 FADD per 32 accumulator columns in the drain.
-#ifndef HN_FOLD_BIAS_TRAIN
-#define HN_FOLD_BIAS_TRAIN 0
-#endif
-constexpr bool kFoldBiasTrain = kFoldBias && HN_FOLD_BIAS_TRAIN != 0;
-// HN_CONST_BIAS: where the epilogue takes its biases from when they do not ride in the UMMAs.
-//   0: staged in shared memory per layer (LDS.128 broadcasts)  1: the training forward reads them from constant memory
-//   2: the inference forward too (no bias K steps at all)
-// Measured (profiles/overlap_rate.py): next to a busy tensor pipe the 8 LDS.128 + 32 FADD per 32 columns double a drain
-// (2 380 -> 4 840 cycles per 128 x 256 accumulator) because the broadcasts queue behind the UMMAs' operand reads in the
-// shared-memory pipe; constant-bank loads (LDC, uniform address) do not touch it.
-// HN_LD_MID = k (1..3): the drain issues the next block's TMEM load after k of the 4 chunks of the current block; 0: right
-// after the wait (source order; ptxas then places it)
-#ifndef HN_LD_MID
-#define HN_LD_MID 0
-#endif
-#ifndef HN_CONST_BIAS
-#define HN_CONST_BIAS 0
-#endif
-constexpr int kConstBias = HN_CONST_BIAS;
-constexpr int kMaxBiasFloats = 4608;   // >= the forward bias array of any built configuration (hyper model: 4 144 floats)
-constexpr int kConstSlots = 3;         // blobs whose biases are resident at the same time (coarse, fine, one more model)
-__constant__ float c_bias[kConstSlots * kMaxBiasFloats];
-// HN_WS = 1: lock-step schedules issue weight-stationary UMMAs (hn_ptx.cuh: umma_ws_*): one shared-memory read of every
-// weight stage per CTA instead of one per sub-tile.
-#ifndef HN_WS
-#define HN_WS 0
-#endif
-// HN_TMA_STASH = 1: the wide layers' stash slabs (activations in the training forward, pre-activation gradients in the data
-// gradient) are not stored by the epilogue threads: the bf16 tile the epilogue writes into ACT for the next layer's UMMAs IS
-// the slab (ACT chunk c, rows [64 h, 64 h + 64) = 1 KB = half tile h's chunk c), so one lane per epilogue warp hands it to the
-// copy engine in 1 KB bulk copies (cp.async.bulk shared -> global, evict-first) once the sub-tile's drain is complete.
-// Timing-only builds that drop the stores altogether bound what this could buy: forward 2.50 -> 2.24 ms, data gradient
-// 2.30 -> 2.00 ms per 1 M samples.  Measured with the copies in place (parity tests green): forward 2.50 -> 2.62 ms, data
-// gradient 2.30 -> 2.28 ms — the cost of the stash is not the epilogue's store instructions but the traffic itself (the copy
-// engine's shared-memory reads compete with the UMMAs' operand reads like the stores' did with the drain).  Off.
-#ifndef HN_TMA_STASH
-#define HN_TMA_STASH 0
-#endif
-constexpr bool kTmaStash = HN_TMA_STASH != 0 && kEpiSplit == 1 && !kPair;
-constexpr bool kPingPongFwdTrain = ((HN_PINGPONG & 1) || kPair) && kSubTiles == 2;
-constexpr bool kPingPongBwd = ((HN_PINGPONG & 2) || kPair) && kSubTiles == 2;
-constexpr bool kPingPongFwdInfer = ((HN_PINGPONG & 4) || kPair) && kSubTiles == 2;
+// The training forward and the data gradient run out of phase, the inference forward in lock step.  Measured per 1 M
+// samples once the stash stores stopped evicting the weights from L2 (streaming stores): data gradient (80 KB ring)
+// 2.55 -> 2.31 ms, training forward (48 KB ring) 2.50 -> 2.42 ms out of phase; inference forward (48 KB ring, short
+// drains, bias K steps streamed twice) 1.89 -> 2.34 ms, so it stays in lock step.
 template <bool PP>
 struct Sched {
   static constexpr int CHAINS = PP ? kSubTiles : 1;          // independently synchronised sub-tile groups
   static constexpr int SUBS = kSubTiles / CHAINS;            // sub-tiles per chain
 };
-// Warp roles.  The epilogue warpgroups come FIRST and the feeder warpgroup (weight producer, UMMA issuer, pair relay)
-// LAST: the SM's warp arbiter favours the highest warp id, and once a drain loop of one sub-tile runs concurrently with
-// the other sub-tile's UMMAs (ping-pong / pair schedules) low-numbered feeder warps were starved of issue slots
-// (measured: the leader's issuer waited 42 % of its time for the other CTA's relay warp).
+// Warp roles.  The epilogue warpgroups come FIRST and the feeder warpgroup (weight producer, UMMA issuer) LAST: the SM's
+// warp arbiter favours the highest warp id, and once a drain loop of one sub-tile runs concurrently with the other
+// sub-tile's UMMAs low-numbered feeder warps were starved of issue slots.
 constexpr int kEpiWarps = 4 * kSubTiles * kEpiSplit;
-// split-epilogue register budgets after setmaxnreg (feeder / primary / secondary warpgroups; 128 F + 256 P + 256 S <= 640 x 96).
-// The first split build (40 / 144 / 72) starved the weight producer (it spills below 72 registers): forward 2.76 ms per 1 M
-// samples; with 72 / 136 / 64 the split epilogue is the faster forward (Makefile: FV_FLAGS).
-#ifndef HN_FEEDER_REGS        // single epilogue warpgroup per sub-tile: 128 F + 256 P <= 384 x 168 (88 / 208 and 104 / 200: no gain)
-#define HN_FEEDER_REGS 72
-#endif
-#ifndef HN_PRIMARY_REGS
-#define HN_PRIMARY_REGS 216
-#endif
-#ifndef HN_SPLIT_FEEDER_REGS
-#define HN_SPLIT_FEEDER_REGS 40
-#endif
-#ifndef HN_SPLIT_PRIMARY_REGS
-#define HN_SPLIT_PRIMARY_REGS 144
-#endif
-#ifndef HN_SPLIT_SECONDARY_REGS
-#define HN_SPLIT_SECONDARY_REGS 72
-#endif
-// register budgets after setmaxnreg (65 536 per SM): feeders, primary and secondary epilogue warpgroups
-constexpr int kRegsFeeder = kEpiSplit == 2 ? HN_SPLIT_FEEDER_REGS : (kSubTiles == 2 ? HN_FEEDER_REGS : 40);   // 128 x 72 + 256 x 216 = 64 512 = the launch allocation (384 x 168)
-// (setmaxnreg moves registers inside the CTA's LAUNCH allocation only: 640 threads x 96 = 61 440 with the split epilogue,
-// 384 x 168 = 64 512 without; the budgets below add up to no more than that)
-constexpr int kRegsPrimary = kEpiSplit == 2 ? HN_SPLIT_PRIMARY_REGS : (kSubTiles == 2 ? HN_PRIMARY_REGS : 208);
-constexpr int kRegsSecondary = HN_SPLIT_SECONDARY_REGS;
-static_assert(kEpiSplit != 2 || 128 * kRegsFeeder + 256 * kRegsPrimary + 256 * kRegsSecondary <= 640 * 96, "register budget");
-constexpr int kProducerWarp = kEpiWarps, kIssuerWarp = kEpiWarps + 1, kRelayWarp = kEpiWarps + 2;
+// Register budgets after setmaxnreg (feeder / primary / secondary warpgroups).  setmaxnreg moves registers inside the CTA's
+// LAUNCH allocation only: 384 threads x 168 = 64 512 with one epilogue warpgroup per sub-tile (128 x 72 + 256 x 216;
+// 88 / 208 and 104 / 200: no gain), 640 x 96 = 61 440 with the split epilogue (128 x 72 + 256 x 136 + 256 x 64).  The
+// weight producer spills below 72 registers (a split build with 40 / 144 / 72 ran the forward in 2.76 ms per 1 M samples).
+constexpr int kRegsFeeder = 72;
+constexpr int kRegsPrimary = kEpiSplit == 2 ? 136 : 216;
+constexpr int kRegsSecondary = 64;
+static_assert(kEpiSplit == 2 ? 128 * kRegsFeeder + 256 * kRegsPrimary + 256 * kRegsSecondary <= 640 * 96
+                             : 128 * kRegsFeeder + 256 * kRegsPrimary <= 384 * 168, "register budget");
+constexpr int kProducerWarp = kEpiWarps, kIssuerWarp = kEpiWarps + 1;
 
 template <int INB_CHUNKS_, int STAGES_>
 struct SmemPlan {
@@ -202,29 +123,20 @@ struct SmemPlan {
   static constexpr int INB = ACT + kSubTiles * ACT_BYTES;
   static constexpr int RING = INB + kSubTiles * INB_BYTES;        // STAGES x kStageBytes
   static constexpr int BIAS = RING + STAGES * kStageBytes;        // 2 x 256 fp32: this / next layer's bias
-  static constexpr int BARS = BIAS + 2 * 256 * 4;                 // full[], empty[], acc_full[2], act_ready[2], peer_full[]
-  static constexpr int TMEMP = BARS + (3 * STAGES + 4) * 8;
+  static constexpr int BARS = BIAS + 2 * 256 * 4;                 // full[], empty[], acc_full[2], act_ready[2]
+  static constexpr int TMEMP = BARS + (2 * STAGES + 4) * 8;
   static constexpr int TOTAL = TMEMP + 16;
   static_assert(TOTAL <= 227 * 1024, "shared memory budget");
 };
 // forward: INB holds the PE input vectors (UMMA operands of the first / skip / view layers)
 template <class C>
 using Smem = SmemPlan<C::INB_CHUNKS, kRingStages>;
-// backward-data: INB only holds the 16-column head gradient of the static model, so the weight ring gets the space.
-// With 3 stages of 512 cycles of UMMA work a refill (commit -> producer -> L2 -> complete_tx, ~1 100 cycles after the
-// stage's last UMMA retires) lands ~80 cycles after the issuer needs the slot again: 12 % of the issuer's time was
-// spent waiting for stages.
-#ifndef HN_PAIR_BWD_RING
-#define HN_PAIR_BWD_RING 0   // experiment: give the pair-mode data gradient the deep ring as well
-#endif
-constexpr int kBwdRingStages = kSubTiles == 2 && (!kPair || HN_PAIR_BWD_RING) ? 5 : kRingStages;
-// (the hyper model's data gradient keeps nothing in INB at all: 6 stages)
+// backward-data: INB only holds the 16-column head gradient of the static model, so the weight ring gets the space:
+// 5 stages, 6 for the hyper model, whose data gradient keeps nothing in INB at all.  With 3 stages of 512 cycles of UMMA
+// work a refill (commit -> producer -> L2 -> complete_tx, ~1 100 cycles after the stage's last UMMA retires) lands ~80
+// cycles after the issuer needs the slot again: 12 % of the issuer's time was spent waiting for stages.
 template <class C>
-using SmemBwd = SmemPlan<C::STATIC ? 2 : 0, (C::STATIC || kBwdRingStages != 5) ? kBwdRingStages : 6>;
-
-// pair mode: 3-D tensor maps over the packed blob viewed as [128-byte block][8 rows][8 bf16]; map i moves a contiguous
-// run of 2^i blocks (128 B .. 32 KB) in one request
-struct PairMaps { CUtensorMap m[kPair ? 9 : 1]; };
+using SmemBwd = SmemPlan<C::STATIC ? 2 : 0, C::STATIC ? 5 : 6>;
 
 // run-time model flags of the fused kernels (from hn_model_desc::flags)
 enum ModelFlags : int { MF_AXIS = 1, MF_COND = 2 };   // hyper point = GLO vector; GLO condition columns in the view vector
@@ -232,11 +144,8 @@ static bool has_warp(const hn_model_desc& d) { return (d.flags & (HN_FLAG_WARP_T
 
 struct FwdParams {
   Program prog;
-  PairMaps maps;
-  uint32_t w_row0;          // pair mode: first 16-byte row of `weights` inside the blob the tensor maps cover
   const uint8_t* weights;   // packed blob base + fwd_off
   const float* bias;        // packed blob base + bias_off
-  int cbias;                // first float of this blob's bias array inside c_bias (kConstBias)
   const float* glo;         // (E, G) fp32 copy of the GLO table
   const float* points; const float* viewdirs; const int64_t* ids; const float* noise;
   const float* warped_in;   // trunk-only program (hn_mlp_fwd_trunk): (n, 3 + H) warped points + hyper coordinates, else NULL
@@ -263,8 +172,6 @@ struct FwdParams {
 
 struct BwdParams {
   Program prog;
-  PairMaps maps;
-  uint32_t w_row0;
   const uint8_t* weights;   // packed blob base + bwd_off
   const int64_t* ids;
   const float* sigma; const float* rgb; const float* warped;
@@ -308,9 +215,6 @@ using RingState = RingStateT<kRingStages>;
 template <bool PP, class RS>
 __device__ __forceinline__ void produce_tile(const Program& prog, const uint8_t* __restrict__ weights, uint8_t* ring,
                                              uint64_t* full, uint64_t* empty, RS& rs, long long& t_wait) {
-#if HN_L2_HINTS & 1
-  const uint64_t keep = l2_policy_evict_last();   // the 1.6 MB of weights are re-read by every CTA for every tile
-#endif
   for (int li = 0; li < prog.nlayers; ++li) {
     const Layer& L = prog.layers[li];
     for (int chain = 0; chain < Sched<PP>::CHAINS; ++chain) {   // ping-pong: every sub-tile makes its own pass over the layer
@@ -325,11 +229,7 @@ __device__ __forceinline__ void produce_tile(const Program& prog, const uint8_t*
           mbar_wait(&empty[rs.slot], rs.phase ^ 1);
           t_wait += HN_T0() - t0;
           mbar_arrive_expect_tx(&full[rs.slot], bytes);
-#if HN_L2_HINTS & 1
-          bulk_g2s_hint(ring + rs.slot * kStageBytes, src + (size_t)c * op.n * 16, bytes, &full[rs.slot], keep);
-#else
           bulk_g2s(ring + rs.slot * kStageBytes, src + (size_t)c * op.n * 16, bytes, &full[rs.slot]);
-#endif
           rs.next();
         }
       }
@@ -372,143 +272,13 @@ __device__ __forceinline__ void issue_layer(const Program& prog, const Layer& L,
         uint32_t acc = (c > 0) | acc0;
         for (uint32_t j = 0; j < cnt; j += 2) {
           const uint64_t bd = desc64(b_lo);
-#if HN_WS
-          // lock step: the second sub-tile takes the weights from the collector buffer (.ws only exists for N = 64 / 128 / 256)
-          if (Sched<PP>::SUBS == 2 && (n == 64 || n == 128 || n == 256)) {
-            umma_ws_fill_bf16(d0, desc64(a_lo), bd, idesc, acc);
-            umma_ws_lastuse_bf16(d0 + 256, desc64(a_lo + a_sub), bd, idesc, acc);
-          } else
-#endif
-          {
 #pragma unroll
           for (int sub = 0; sub < Sched<PP>::SUBS; ++sub) umma_bf16(d0 + sub * 256, desc64(a_lo + sub * a_sub), bd, idesc, acc);
-          }
           a_lo += 2 * (kChunkBytes >> 4);
           b_lo += 2 * n;
           acc = 1;
         }
         umma_commit(&empty[rs.slot]);
-      }
-      __syncwarp();
-      rs.next();
-    }
-  }
-}
-
-// ---- pair mode (HN_PAIR): see hn_mlp_program.h -------------------------------------------------------------------
-// HN_PAIR_DIRECT = 1: the non-leader CTA's weight copies complete_tx on the LEADER's full[] barrier (its shared::cluster
-// address), so the issuer learns from one local barrier that both halves of a stage have landed; 0: relay thread +
-// remote arrive on peer_full[].
-#ifndef HN_PAIR_DIRECT
-#define HN_PAIR_DIRECT 1
-#endif
-// HN_PAIR_MAP2D = 1: the pair mode's tensor maps view the blob as [128-byte line][lines] instead of [block][8 rows][8 bf16]
-#ifndef HN_PAIR_MAP2D
-#define HN_PAIR_MAP2D 1
-#endif
-// Producer of CTA `rank`: per stage, its half (rows [rank N/2, (rank+1) N/2) of every 8-column chunk) of the weights.
-template <class RS>
-__device__ __forceinline__ void produce_tile_pair(const Program& prog, const PairMaps& maps, uint32_t w_row0,
-                                                  const uint8_t* __restrict__ weights, uint8_t* ring,
-                                                  uint64_t* full, uint64_t* empty, RS& rs, uint32_t rank, long long& t_wait) {
-  for (int li = 0; li < prog.nlayers; ++li) {
-    const Layer& L = prog.layers[li];
-    for (int chain = 0; chain < kSubTiles; ++chain) {   // pair mode is always ping-pong
-      for (int oi = L.op0; oi < L.op0 + L.nops; ++oi) {
-        const MmaOp& op = prog.ops[oi];
-        const int nchunks = op.k >> 3;
-        const uint32_t half_bytes = (uint32_t)(op.n >> 1) * 16;   // one chunk's rows held by this CTA
-        // pair layout of the packed weights: [rank][chunk][N/2 rows][8] -> this CTA's chunks are contiguous
-        const uint32_t nh = op.n >> 1;
-        const uint32_t row_base = (op.w_off16 - (uint32_t)op.n * op.kc0)                 // the logical matrix
-                                  + rank * (uint32_t)op.kc_total * nh + (uint32_t)op.kc0 * nh;   // 16-byte rows inside `weights`
-        for (int c = 0; c < nchunks; c += op.cps) {
-          const int cnt = min((int)op.cps, nchunks - c);
-          { long long t0 = HN_T0(); mbar_wait(&empty[rs.slot], rs.phase ^ 1); t_wait += HN_T0() - t0; }
-          uint8_t* dst = ring + rs.slot * kStageBytes;
-          const uint32_t bytes = cnt * half_bytes;
-          const uint32_t row0 = row_base + (uint32_t)c * (op.n >> 1);
-#if HN_PAIR_DIRECT
-          // both CTAs' halves complete_tx on the leader's full[slot]; the leader expects the bytes of both
-          if (rank == 0) mbar_arrive_expect_tx(&full[rs.slot], 2 * bytes);
-          uint32_t blk = (w_row0 + row0) >> 3, nblk = bytes >> 7, off = 0;   // 128-byte blocks
-          while (nblk) {
-            const int i = 31 - __clz(nblk > 256u ? 256u : nblk);             // largest power of two that fits
-#if HN_PAIR_MAP2D
-            tma_g2s_2d_pair(dst + off, &maps.m[i], (int32_t)blk, &full[rs.slot]);
-#else
-            tma_g2s_3d_pair(dst + off, &maps.m[i], (int32_t)blk, &full[rs.slot]);
-#endif
-            blk += 1u << i; nblk -= 1u << i; off += 128u << i;
-          }
-#else
-          mbar_arrive_expect_tx(&full[rs.slot], bytes);
-          bulk_g2s(dst, weights + (size_t)row0 * 16, bytes, &full[rs.slot]);
-#endif
-          rs.next();
-        }
-      }
-    }
-  }
-}
-// Relay of the non-leader CTA: tells the leader's issuer when this CTA's half of a stage has landed.
-template <class RS>
-__device__ __forceinline__ void relay_tile_pair(const Program& prog, uint64_t* full, uint32_t leader_peer_full, RS& rs) {
-  for (int li = 0; li < prog.nlayers; ++li) {
-    const Layer& L = prog.layers[li];
-    for (int chain = 0; chain < kSubTiles; ++chain) {   // pair mode is always ping-pong
-      for (int oi = L.op0; oi < L.op0 + L.nops; ++oi) {
-        const MmaOp& op = prog.ops[oi];
-        const int nchunks = op.k >> 3;
-        for (int c = 0; c < nchunks; c += op.cps) {
-          mbar_wait(&full[rs.slot], rs.phase);
-          mbar_arrive_remote(leader_peer_full + rs.slot * 8);
-          rs.next();
-        }
-      }
-    }
-  }
-}
-// Leader's issuer: one layer of one chain (= sub-tile `sub0` of both CTAs), cta_group::2, M = 256.
-template <class RS>
-__device__ __forceinline__ void issue_layer_pair(const Program& prog, const Layer& L, int sub0, uint32_t act_s, uint32_t inb_s,
-                                                 uint32_t act_stride, uint32_t inb_stride, uint32_t ring_s, uint32_t tmem_base,
-                                                 uint64_t* full, uint64_t* peer_full, uint64_t* empty, RS& rs,
-                                                 long long& t_wait, long long& t_peer) {
-  for (int oi = L.op0; oi < L.op0 + L.nops; ++oi) {
-    const MmaOp& op = prog.ops[oi];
-    const uint32_t n = op.n, nh = n >> 1, nchunks = op.k >> 3, cps = op.cps;
-    const uint32_t idesc = make_idesc_bf16(2 * kTileRows, n, 0, 0);
-    const bool from_act = op.src == SRC_ACT;
-    const uint32_t a_sub = (from_act ? act_stride : inb_stride) >> 4;
-    const uint32_t a_base = ((((from_act ? act_s : inb_s) + op.a_chunk * kChunkBytes) >> 4) | ((uint32_t)(kChunkBytes >> 4) << 16)) + sub0 * a_sub;
-    const uint32_t d0 = tmem_base + op.tmem_col + sub0 * 256;
-    const uint32_t acc0 = op.acc_init;
-    for (uint32_t c = 0; c < nchunks; c += cps) {
-      const uint32_t cnt = min(cps, nchunks - c);
-      long long t0 = HN_T0();
-#if HN_PAIR_DIRECT
-      mbar_wait_cluster(&full[rs.slot], rs.phase);
-      t_wait += HN_T0() - t0;
-      (void)peer_full; (void)t_peer;
-#else
-      mbar_wait(&full[rs.slot], rs.phase);
-      long long t1 = HN_T0();
-      mbar_wait_cluster(&peer_full[rs.slot], rs.phase);
-      t_wait += t1 - t0; t_peer += HN_T0() - t1;
-#endif
-      tc_fence_after();
-      if (elect_one_sync()) {
-        uint32_t a_lo = a_base + c * (uint32_t)(kChunkBytes >> 4);
-        uint32_t b_lo = ((ring_s + rs.slot * kStageBytes) >> 4) | (nh << 16);   // B half: K-major, LBO = N/2 * 16 B
-        uint32_t acc = (c > 0) | acc0;
-        for (uint32_t j = 0; j < cnt; j += 2) {
-          umma2_bf16(d0, desc64(a_lo), desc64(b_lo), idesc, acc);
-          a_lo += 2 * (kChunkBytes >> 4);
-          b_lo += 2 * nh;
-          acc = 1;
-        }
-        umma2_commit_mc(&empty[rs.slot], 3);   // frees the slot in both CTAs
       }
       __syncwarp();
       rs.next();
@@ -659,13 +429,13 @@ __device__ __forceinline__ void se3_apply_bwd(const float* x, const float* w, co
   }
 }
 
-// zero padding of a K-wide input vector with IN real features; with folded biases a vector that reaches INB's last
-// chunk carries the two ones columns in its tail
+// zero padding of a K-wide input vector with IN real features; a vector that reaches INB's last chunk carries the two
+// ones columns of the folded biases in its tail
 template <class C, int K, int IN>
 __device__ __forceinline__ void finish_features(float* f) {
 #pragma unroll
   for (int i = IN; i < K; ++i) f[i] = 0.f;
-  if constexpr (kFoldBias && K / 8 == C::INB_CHUNKS) {
+  if constexpr (K / 8 == C::INB_CHUNKS) {
     static_assert(IN <= K - 2, "no room for the ones columns");
     f[K - 2] = 1.f; f[K - 1] = 1.f;
   }
@@ -673,7 +443,7 @@ __device__ __forceinline__ void finish_features(float* f) {
 // the ones chunk pair of INB when the vector just stored (K columns) does not reach it
 template <class C, int K>
 __device__ __forceinline__ void store_ones_pair(uint8_t* inb_row) {
-  if constexpr (kFoldBias && K / 8 < C::INB_CHUNKS) {
+  if constexpr (K / 8 < C::INB_CHUNKS) {
     if constexpr (K / 8 < C::INB_CHUNKS - 1) *reinterpret_cast<uint4*>(inb_row + (C::INB_CHUNKS - 2) * kChunkBytes) = make_uint4(0, 0, 0, 0);
     *reinterpret_cast<uint4*>(inb_row + (C::INB_CHUNKS - 1) * kChunkBytes) = make_uint4(0, 0, 0, 0x3F803F80u);   // bf16 1.0, 1.0
   }
@@ -702,10 +472,8 @@ __device__ __forceinline__ void store_features(const float* f, uint8_t* buf_row,
 // the ones chunk pair of INB on its own (trunk-only rows of a model whose trunk input lives in ACT)
 template <class C>
 __device__ __forceinline__ void store_ones_only(uint8_t* inb_row) {
-  if constexpr (kFoldBias) {
-    *reinterpret_cast<uint4*>(inb_row + (C::INB_CHUNKS - 2) * kChunkBytes) = make_uint4(0, 0, 0, 0);
-    *reinterpret_cast<uint4*>(inb_row + (C::INB_CHUNKS - 1) * kChunkBytes) = make_uint4(0, 0, 0, 0x3F803F80u);   // bf16 1.0, 1.0
-  }
+  *reinterpret_cast<uint4*>(inb_row + (C::INB_CHUNKS - 2) * kChunkBytes) = make_uint4(0, 0, 0, 0);
+  *reinterpret_cast<uint4*>(inb_row + (C::INB_CHUNKS - 1) * kChunkBytes) = make_uint4(0, 0, 0, 0x3F803F80u);   // bf16 1.0, 1.0
 }
 
 // Trunk input vector of the template (models.py:458-478): [posenc_orig(xyz, XF) | posenc_orig(hyper, HF) | 0], written as
@@ -753,44 +521,33 @@ __device__ __forceinline__ void warp_arrive(uint64_t* bar) {
   __syncwarp();
   if ((threadIdx.x & 31) == 0) mbar_arrive(bar);
 }
-// pair mode: the activation barrier lives in the leader CTA; `leader_bar` is its shared::cluster address
-__device__ __forceinline__ void warp_arrive_leader(uint32_t leader_bar) {
-  __syncwarp();
-  if ((threadIdx.x & 31) == 0) mbar_arrive_remote(leader_bar);
-}
 // named barrier of one chain's epilogue threads (ids 1, 2; barrier 0 is __syncthreads)
 template <bool PP>
 __device__ __forceinline__ void epi_named_barrier(int chain) {
   asm volatile("bar.sync %0, %1;" ::"r"(1 + chain), "n"(128 * Sched<PP>::SUBS * kEpiSplit) : "memory");
 }
 
-// bias of a head column: already inside the accumulator when the biases ride in the UMMAs
-// BM: 0 = already inside the accumulator (bias K steps), 1 = shared-memory staging buffer, 2 = constant memory
-template <int BM>
-__device__ __forceinline__ float head_bias(const float* bias_s, int cb, int i) {
-  return BM == 0 ? 0.f : (BM == 2 ? c_bias[cb + i] : bias_s[i]);
+// bias of a head column: FOLD = already inside the accumulator (bias K steps), else from the shared-memory staging buffer
+template <bool FOLD>
+__device__ __forceinline__ float head_bias(const float* bias_s, int i) {
+  return FOLD ? 0.f : bias_s[i];
 }
 
-// chunks [Q0, Q1) of one 32-column block (a chunk = 8 columns): bias, ReLU, bf16 pack, st.shared (+ stash store); ge / go
-// collect the sign bits for the block's gate word
-template <bool RELU, bool STASH, int BM, int Q0, int Q1>
-__device__ __forceinline__ void fwd_store_chunks(const uint32_t* r, const float* bias_s, int cb, uint8_t* act_row, uint4* save_row,
-                                                 int chunk0, int save_chunk, uint32_t& ge, uint32_t& go) {
+// one 32-column block (4 chunks of 8 columns): bias, ReLU, bf16 pack, st.shared (+ stash store and gate word: the sign
+// bits of the even / odd columns, hn_ptx.cuh: gate_push)
+template <bool RELU, bool STASH, bool FOLD>
+__device__ __forceinline__ void fwd_store32(const uint32_t* r, const float* bias_s, uint8_t* act_row, uint4* save_row,
+                                            int chunk0, int save_chunk, uint32_t* gate_dst) {
+  uint32_t ge = 0, go = 0;
 #pragma unroll
-  for (int q = Q0; q < Q1; ++q) {
+  for (int q = 0; q < 4; ++q) {
     float v[8];
-    if constexpr (BM == 0) {   // the accumulator already holds W x + b
+    if constexpr (FOLD) {   // the accumulator already holds W x + b
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = __uint_as_float(r[8 * q + j]);
-    } else {
-    float4 b0, b1;
-    if constexpr (BM == 2) {   // constant-bank loads, uniform address
-      b0 = *reinterpret_cast<const float4*>(&c_bias[cb + 8 * q]);
-      b1 = *reinterpret_cast<const float4*>(&c_bias[cb + 8 * q + 4]);
-    } else {                   // smem broadcast
-      b0 = *reinterpret_cast<const float4*>(bias_s + 8 * q);
-      b1 = *reinterpret_cast<const float4*>(bias_s + 8 * q + 4);
-    }
+    } else {                // smem broadcast
+    const float4 b0 = *reinterpret_cast<const float4*>(bias_s + 8 * q);
+    const float4 b1 = *reinterpret_cast<const float4*>(bias_s + 8 * q + 4);
     v[0] = __uint_as_float(r[8 * q + 0]) + b0.x; v[1] = __uint_as_float(r[8 * q + 1]) + b0.y;
     v[2] = __uint_as_float(r[8 * q + 2]) + b0.z; v[3] = __uint_as_float(r[8 * q + 3]) + b0.w;
     v[4] = __uint_as_float(r[8 * q + 4]) + b1.x; v[5] = __uint_as_float(r[8 * q + 5]) + b1.y;
@@ -809,81 +566,47 @@ __device__ __forceinline__ void fwd_store_chunks(const uint32_t* r, const float*
       o.z = pack_bf16(v[4], v[5]); o.w = pack_bf16(v[6], v[7]);
     }
     *reinterpret_cast<uint4*>(act_row + (chunk0 + q) * kChunkBytes) = o;
-    if (STASH && !kTmaStash) stash_store(&save_row[(save_chunk + chunk0 + q) * (kHalfChunkBytes / 16)], o);
+    if (STASH) stash_store(&save_row[(save_chunk + chunk0 + q) * (kHalfChunkBytes / 16)], o);
   }
-}
-template <bool RELU, bool STASH, int BM>
-__device__ __forceinline__ void fwd_store32(const uint32_t* r, const float* bias_s, int cb, uint8_t* act_row, uint4* save_row,
-                                            int chunk0, int save_chunk, uint32_t* gate_dst) {
-  uint32_t ge = 0, go = 0;   // sign bits of the even / odd columns of this 32-column block (hn_ptx.cuh: gate_push)
-  fwd_store_chunks<RELU, STASH, BM, 0, 4>(r, bias_s, cb, act_row, save_row, chunk0, save_chunk, ge, go);
-  if (RELU && STASH) __stcs(&gate_dst[(chunk0 >> 2) * kHalfRows], gate_word_of(ge, go));
-}
-// the same with the NEXT block's TMEM load issued in the middle of this block's work (HN_LD_MID): where exactly the load
-// sits relative to the stores changes the drain by several percent (ptxas otherwise floats it freely)
-template <bool RELU, bool STASH, int BM>
-__device__ __forceinline__ void fwd_store32_ld(const uint32_t* r, const float* bias_s, int cb, uint8_t* act_row, uint4* save_row,
-                                               int chunk0, int save_chunk, uint32_t* gate_dst, bool more, uint32_t next_taddr,
-                                               uint32_t* next) {
-  uint32_t ge = 0, go = 0;
-  fwd_store_chunks<RELU, STASH, BM, 0, HN_LD_MID>(r, bias_s, cb, act_row, save_row, chunk0, save_chunk, ge, go);
-  asm volatile("" ::: "memory");
-  if (more) tmem_ld32(next_taddr, next);
-  asm volatile("" ::: "memory");
-  fwd_store_chunks<RELU, STASH, BM, HN_LD_MID, 4>(r, bias_s, cb, act_row, save_row, chunk0, save_chunk, ge, go);
   if (RELU && STASH) __stcs(&gate_dst[(chunk0 >> 2) * kHalfRows], gate_word_of(ge, go));
 }
 
 // ncols: multiple of 32
-template <bool RELU, bool STASH, int BM>
-__device__ __forceinline__ void fwd_cols(uint32_t taddr, const float* bias_s, int cb, uint8_t* act_row, uint4* save_row,
+template <bool RELU, bool STASH, bool FOLD>
+__device__ __forceinline__ void fwd_cols(uint32_t taddr, const float* bias_s, uint8_t* act_row, uint4* save_row,
                                          int save_chunk, int ncols, uint32_t* gate_dst) {
   if constexpr (kEpiSplit == 2) {
-    // two warpgroups per sub-tile overlap each other's TMEM latency: one buffer keeps the secondary warpgroup at 72 registers
+    // two warpgroups per sub-tile overlap each other's TMEM latency: one buffer keeps the secondary warpgroup at 64 registers
     uint32_t r[32];
     for (int c0 = 0; c0 < ncols; c0 += 32) {
       tmem_ld32(taddr + c0, r);
       tmem_ld_wait();
-      fwd_store32<RELU, STASH, BM>(r, bias_s + c0, cb + c0, act_row, save_row, c0 >> 3, save_chunk, gate_dst);
+      fwd_store32<RELU, STASH, FOLD>(r, bias_s + c0, act_row, save_row, c0 >> 3, save_chunk, gate_dst);
     }
     return;
   }
   uint32_t ra[32], rb[32];
   tmem_ld32(taddr, ra);
-#if HN_LD_MID > 0
-  for (int c0 = 0; c0 < ncols; c0 += 64) {
-    tmem_ld_wait();
-    const bool more = c0 + 32 < ncols;
-    fwd_store32_ld<RELU, STASH, BM>(ra, bias_s + c0, cb + c0, act_row, save_row, c0 >> 3, save_chunk, gate_dst, more,
-                                    taddr + c0 + 32, rb);
-    if (more) {
-      tmem_ld_wait();
-      fwd_store32_ld<RELU, STASH, BM>(rb, bias_s + c0 + 32, cb + c0 + 32, act_row, save_row, (c0 + 32) >> 3, save_chunk, gate_dst,
-                                      c0 + 64 < ncols, taddr + c0 + 64, ra);
-    }
-  }
-  return;
-#endif
   for (int c0 = 0; c0 < ncols; c0 += 64) {
     tmem_ld_wait();
     const bool more = c0 + 32 < ncols;
     if (more) tmem_ld32(taddr + c0 + 32, rb);
-    fwd_store32<RELU, STASH, BM>(ra, bias_s + c0, cb + c0, act_row, save_row, c0 >> 3, save_chunk, gate_dst);
+    fwd_store32<RELU, STASH, FOLD>(ra, bias_s + c0, act_row, save_row, c0 >> 3, save_chunk, gate_dst);
     if (more) {
       tmem_ld_wait();
       if (c0 + 64 < ncols) tmem_ld32(taddr + c0 + 64, ra);
-      fwd_store32<RELU, STASH, BM>(rb, bias_s + c0 + 32, cb + c0 + 32, act_row, save_row, (c0 + 32) >> 3, save_chunk, gate_dst);
+      fwd_store32<RELU, STASH, FOLD>(rb, bias_s + c0 + 32, act_row, save_row, (c0 + 32) >> 3, save_chunk, gate_dst);
     }
   }
 }
 
-// the column share of one of the kEpiSplit warpgroups that drain a sub-tile (hn_mlp_program.h: HN_EPI_SPLIT)
-template <bool RELU, bool STASH, int BM>
-__device__ __forceinline__ void fwd_cols_share(int share, uint32_t taddr, const float* bias_s, int cb, uint8_t* act_row,
+// the column share of one of the kEpiSplit warpgroups that drain a sub-tile (hn_mlp_program.h: kEpiSplit)
+template <bool RELU, bool STASH, bool FOLD>
+__device__ __forceinline__ void fwd_cols_share(int share, uint32_t taddr, const float* bias_s, uint8_t* act_row,
                                                uint4* save_row, int save_chunk, int ncols, uint32_t* gate_dst) {
   const int n = ncols / kEpiSplit, c0 = share * n;
-  fwd_cols<RELU, STASH, BM>(taddr + c0, bias_s + c0, cb + c0, act_row + (c0 >> 3) * kChunkBytes, save_row,
-                            save_chunk + (c0 >> 3), n, gate_dst != nullptr ? gate_dst + (c0 >> 5) * kHalfRows : nullptr);
+  fwd_cols<RELU, STASH, FOLD>(taddr + c0, bias_s + c0, act_row + (c0 >> 3) * kChunkBytes, save_row,
+                              save_chunk + (c0 >> 3), n, gate_dst != nullptr ? gate_dst + (c0 >> 5) * kHalfRows : nullptr);
 }
 
 // backward: ReLU gates from the gate words the forward wrote (one uint32 per row per 32 columns, hn_ptx.cuh), so the
@@ -912,7 +635,7 @@ __device__ __forceinline__ void bwd_store32(const uint32_t* r, uint32_t w, uint8
   for (int q = 0; q < 4; ++q) {
     const uint4 v = make_uint4(o[4 * q], o[4 * q + 1], o[4 * q + 2], o[4 * q + 3]);
     *reinterpret_cast<uint4*>(dst_row + (chunk0 + q) * kChunkBytes) = v;
-    if (save_row != nullptr && !kTmaStash) stash_store(&save_row[(save_chunk + chunk0 + q) * (kHalfChunkBytes / 16)], v);
+    if (save_row != nullptr) stash_store(&save_row[(save_chunk + chunk0 + q) * (kHalfChunkBytes / 16)], v);
   }
 }
 // NCOLS: multiple of 32 (<= 256), compile time so that gw[] and both row buffers stay in registers
@@ -948,7 +671,7 @@ __device__ __forceinline__ void bwd_masked_layer(uint32_t tlane, const uint32_t*
   bwd_cols<true, NCOLS>(tlane, gw, dst_row, save_row, save_chunk);
 }
 
-// the column share of one of the kEpiSplit warpgroups of a sub-tile (hn_mlp_program.h: HN_EPI_SPLIT)
+// the column share of one of the kEpiSplit warpgroups of a sub-tile (hn_mlp_program.h: kEpiSplit)
 template <int NCOLS>
 __device__ __forceinline__ void bwd_masked_share(int share, uint32_t tlane, const uint32_t* __restrict__ gate_row, int gate_word,
                                                  uint8_t* dst_row, uint4* save_row, int save_chunk, uint64_t* acc_full,
@@ -965,21 +688,6 @@ __device__ __forceinline__ void bwd_linear_share(int share, uint32_t tlane, uint
   bwd_cols<false, N>(tlane + c0, nullptr, dst_row + (c0 >> 3) * kChunkBytes, save_row, save_chunk + (c0 >> 3));
 }
 
-// HN_TMA_STASH: chunks [0, nchunks) of sub-tile `sub`'s ACT tile -> slab `slab_chunk` of its two half tiles.  Called by every
-// epilogue warp of the sub-tile after a barrier that follows the drain; lane 0 of warp quarter q takes chunks q, q + 4, ...
-__device__ __forceinline__ void stash_tile_bulk(const uint8_t* act_sub, uint8_t* stash, size_t half0, int total_chunks, int slab_chunk,
-                                                int nchunks, int quarter, int lane, uint64_t policy) {
-  if (lane == 0) {
-    for (int c = quarter; c < nchunks; c += 4) {
-#pragma unroll
-      for (int h = 0; h < 2; ++h)
-        bulk_s2g_hint(stash + ((half0 + h) * (size_t)total_chunks + slab_chunk + c) * kHalfChunkBytes,
-                      act_sub + c * kChunkBytes + h * kHalfChunkBytes, kHalfChunkBytes, policy);
-    }
-    bulk_commit_group();
-  }
-}
-
 __device__ __forceinline__ float softplus_f(float x) { return x > 20.f ? x : log1pf(expf(x)); }
 __device__ __forceinline__ float sigmoid_f(float x) { return 1.f / (1.f + expf(-x)); }
 
@@ -989,13 +697,12 @@ __device__ __forceinline__ float sigmoid_f(float x) { return 1.f / (1.f + expf(-
 // STASH = false (inference, hn_mlp_fwd with saved == NULL) compiles every stash store out: even predicated-off
 // st.global instructions in the drain loop cost 23 % of the kernel (2.67 -> 2.06 ms per 1 M samples, measured).
 template <class C, bool STASH>
-__global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const __grid_constant__ FwdParams p) {
+__global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_constant__ FwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   using SM = Smem<C>;
-  // biases inside the UMMAs (hn_mlp_program.h: HN_FOLD_BIAS), else from constant memory (HN_CONST_BIAS) or staged in smem
-  constexpr bool FOLD = kFoldBias && (STASH ? kFoldBiasTrain : kConstBias < 2);
-  constexpr int BM = FOLD ? 0 : ((STASH ? kConstBias >= 1 : kConstBias >= 2) ? 2 : 1);
-  constexpr bool PP = STASH ? kPingPongFwdTrain : kPingPongFwdInfer;
+  // biases inside the UMMAs in inference (hn_mlp_program.h: bias folding), staged in smem by the stash-writing forward
+  constexpr bool FOLD = !STASH;
+  constexpr bool PP = STASH;   // out of phase in training, lock step in inference (see Sched)
   uint8_t* act = smem + SM::ACT;
   uint8_t* inb = smem + SM::INB;
   uint8_t* ring = smem + SM::RING;
@@ -1007,21 +714,15 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(smem + SM::TMEMP);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
-  uint64_t* peer_full = act_ready + 2;        // [kRingStages], pair mode: the other CTA's half of a stage has landed
-  const uint32_t rank = kPair ? cluster_ctarank() : 0;
   if (threadIdx.x == 0) {
-    for (int i = 0; i < kRingStages; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); mbar_init(&peer_full[i], 1); }
-    // one arrival per epilogue warp of the chain (pair mode: of both CTAs, the other CTA's arrive remotely)
-    for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&act_ready[i], 4 * Sched<PP>::SUBS * kEpiSplit * (kPair ? 2 : 1)); }
+    for (int i = 0; i < kRingStages; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
+    // one arrival per epilogue warp of the chain
+    for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&act_ready[i], 4 * Sched<PP>::SUBS * kEpiSplit); }
     fence_barrier_init();
   }
-  if (warp == kIssuerWarp) {
-    if (kPair) { tmem_alloc2(tmem_ptr, 256 * kSubTiles); tmem_relinquish2(); }
-    else { tmem_alloc(tmem_ptr, 256 * kSubTiles); tmem_relinquish(); }
-  }
+  if (warp == kIssuerWarp) { tmem_alloc(tmem_ptr, 256 * kSubTiles); tmem_relinquish(); }
   tc_fence_before();
   __syncthreads();
-  if (kPair) cluster_sync_all();   // barriers of both CTAs are initialised before any remote arrive / multicast commit
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   const Program& prog = p.prog;
@@ -1031,37 +732,24 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
     if (warp == kProducerWarp && lane == 0) {
       RingState rs;
       long long tw = 0;
-      for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
-        if (kPair) produce_tile_pair(prog, p.maps, p.w_row0, p.weights, ring, full, empty, rs, rank, tw);
-        else produce_tile<PP>(prog, p.weights, ring, full, empty, rs, tw);
-      }
+      for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) produce_tile<PP>(prog, p.weights, ring, full, empty, rs, tw);
       if (p.dbg) p.dbg[blockIdx.x * 8 + 0] = tw;
-    } else if (kPair && !HN_PAIR_DIRECT && warp == kRelayWarp && lane == 0 && rank == 1) {
-      RingState rs;
-      const uint32_t leader_peer_full = mapa_u32(peer_full, 0);
-      for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) relay_tile_pair(prog, full, leader_peer_full, rs);
-    } else if (warp == kIssuerWarp && (!kPair || rank == 0)) {  // whole warp, converged: see elect_one_sync()
+    } else if (warp == kIssuerWarp) {  // whole warp, converged: see elect_one_sync()
       RingState rs;
       uint32_t ph_ready = 0;
-      long long t_ready = 0, t_full = 0, t_peer = 0;
+      long long t_ready = 0, t_full = 0;
       const long long t_begin = HN_T0();
       const uint32_t act_s = smem_u32(act), inb_s = smem_u32(inb), ring_s = smem_u32(ring);
       for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
         for (int li = 0; li < prog.nlayers; ++li) {
           for (int chain = 0; chain < Sched<PP>::CHAINS; ++chain) {
             long long t0 = HN_T0();
-            if (kPair) mbar_wait_cluster(&act_ready[chain], ph_ready); else mbar_wait(&act_ready[chain], ph_ready);
+            mbar_wait(&act_ready[chain], ph_ready);
             t_ready += HN_T0() - t0;
             tc_fence_after();
-            if (kPair) {
-              issue_layer_pair(prog, prog.layers[li], chain * Sched<PP>::SUBS, act_s, inb_s, SM::ACT_BYTES, SM::INB_BYTES, ring_s,
-                               tmem_base, full, peer_full, empty, rs, t_full, t_peer);
-              if (elect_one_sync()) umma2_commit_mc(&acc_full[chain], 3);   // accumulators of both CTAs are complete
-            } else {
-              issue_layer<PP>(prog, prog.layers[li], chain * Sched<PP>::SUBS, act_s, inb_s, SM::ACT_BYTES, SM::INB_BYTES, ring_s, tmem_base,
-                          full, empty, rs, t_full);
-              if (elect_one_sync()) umma_commit(&acc_full[chain]);
-            }
+            issue_layer<PP>(prog, prog.layers[li], chain * Sched<PP>::SUBS, act_s, inb_s, SM::ACT_BYTES, SM::INB_BYTES, ring_s, tmem_base,
+                        full, empty, rs, t_full);
+            if (elect_one_sync()) umma_commit(&acc_full[chain]);
             __syncwarp();
           }
           ph_ready ^= 1;
@@ -1069,7 +757,6 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
       }
       if (p.dbg && lane == 0) {
         p.dbg[blockIdx.x * 8 + 1] = t_ready; p.dbg[blockIdx.x * 8 + 2] = t_full; p.dbg[blockIdx.x * 8 + 3] = HN_T0() - t_begin;
-        if (kPair && !HN_PAIR_DIRECT) p.dbg[blockIdx.x * 8 + 0] = t_peer;   // relay variant: issuer's wait for the other CTA's half stage
       }
     }
   } else {
@@ -1087,11 +774,9 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
     const int chain = PP ? sub : 0;
     uint64_t* my_acc = &acc_full[chain];
     uint64_t* my_ready = &act_ready[chain];
-    const uint32_t leader_ready = kPair ? mapa_u32(my_ready, 0) : 0;
     uint32_t ph_acc = 0;
     long long t_acc = 0, t_pro = 0;
     const long long t_begin = HN_T0();
-    const uint64_t stash_policy = (STASH && kTmaStash) ? l2_policy_evict_first() : 0;   // like st.global.cs: see stash_store
     for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
       const long long t_tile = HN_T0();
       const int64_t g = (int64_t)tile * kCtaRows + sub * kTileRows + row;
@@ -1156,7 +841,7 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
       }   // PRIMARY
       fence_proxy_async_smem();
       tc_fence_before();
-      { if (kPair) warp_arrive_leader(leader_ready); else warp_arrive(my_ready); }
+      warp_arrive(my_ready);
       t_pro += HN_T0() - t_tile;
 
       for (int li = 0; li < prog.nlayers; ++li) {
@@ -1165,23 +850,16 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
         // a per-block __ldg would go to L2 every time); double-buffered by layer parity
         float* bias = PP ? sbias + chain * 256 : sbias + (li & 1) * 256;
         const long long t_layer = HN_T0();
-        const int cb = p.cbias + L.bias_off;    // this layer's biases inside c_bias (BM == 2)
-        if constexpr (BM == 1) {
+        if constexpr (!FOLD) {
           if (PP) epi_named_barrier<PP>(chain);   // single buffer per chain: everyone is done with the previous layer's bias
           for (int i = et; i < L.n_out; i += 128 * Sched<PP>::SUBS * kEpiSplit) bias[i] = __ldg(p.bias + L.bias_off + i);
           epi_named_barrier<PP>(chain);
         }
         { long long t0 = HN_T0(); mbar_wait(my_acc, ph_acc); ph_acc ^= 1; t_acc += HN_T0() - t0; }
         tc_fence_after();
-        if constexpr (STASH && kTmaStash) {
-          // the copy engine has had this layer's UMMA phase to read the previous layer's tile out of ACT; nobody overwrites
-          // it before the lanes that issued those copies have seen them complete
-          bulk_wait_read_all();
-          epi_named_barrier<PP>(chain);
-        }
         const long long t_drain = HN_T0();
         if (L.epi == FE_RELU) {
-          fwd_cols_share<true, STASH, BM>(share, tlane, bias, cb, act_row, save_row, L.save_chunk, L.n_out,
+          fwd_cols_share<true, STASH, FOLD>(share, tlane, bias, act_row, save_row, L.save_chunk, L.n_out,
                                       STASH ? gate_row + (size_t)L.gate_word * kHalfRows : nullptr);
         } else if (L.epi == FE_WSHEAD) {
           if constexpr (PRIMARY && !C::STATIC && !C::NOWARP) {
@@ -1195,7 +873,7 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
             // head columns 0..2 = w, 3..5 = v: rigid transform of the sample point by exp of the screw (warping.py:229-238)
             float wv[6], x[3];
 #pragma unroll
-            for (int i = 0; i < 6; ++i) wv[i] = __uint_as_float(r[i]) + head_bias<BM>(bias, cb, i);
+            for (int i = 0; i < 6; ++i) wv[i] = __uint_as_float(r[i]) + head_bias<FOLD>(bias, i);
 #pragma unroll
             for (int i = 0; i < 3; ++i) x[i] = wp[i];
             se3_apply(x, wv, wv + 3, wp);
@@ -1205,9 +883,9 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
             }
           } else {
 #pragma unroll
-          for (int i = 0; i < 3; ++i) wp[i] += __uint_as_float(r[i]) + head_bias<BM>(bias, cb, i);
+          for (int i = 0; i < 3; ++i) wp[i] += __uint_as_float(r[i]) + head_bias<FOLD>(bias, i);
 #pragma unroll
-          for (int i = 0; i < C::H; ++i) wp[3 + i] = __uint_as_float(r[3 + i]) + head_bias<BM>(bias, cb, 3 + i);
+          for (int i = 0; i < C::H; ++i) wp[3 + i] = __uint_as_float(r[3 + i]) + head_bias<FOLD>(bias, 3 + i);
           }
           if constexpr (C::H == C::G) {
             if (p.mflags & MF_AXIS) {   // axis-aligned slicing: the hyper point is the GLO vector (models.py:533-534)
@@ -1233,19 +911,19 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
           // recomputed from the warped point this thread still holds, for the input part that accumulates on top
           if constexpr (PRIMARY && C::TIN_ACT) store_trunk_input<C>(wp_keep, act_row, inb_row, nullptr, 0);
         } else if (L.epi == FE_LINEAR) {
-          fwd_cols_share<false, STASH, BM>(share, tlane, bias, cb, act_row, save_row, L.save_chunk, L.n_out, nullptr);
+          fwd_cols_share<false, STASH, FOLD>(share, tlane, bias, act_row, save_row, L.save_chunk, L.n_out, nullptr);
         } else if (L.epi == FE_SIGMA) {
           // static baseline: raw sigma = Linear(W, 1)(h8) (nerf.py:109); rendering.py:150 uses relu(sigma + noise)
           if constexpr (PRIMARY) {
           uint32_t r[16];
           tmem_ld16(tlane, r);
           tmem_ld_wait();
-          float a = __uint_as_float(r[0]) + head_bias<BM>(bias, cb, 0);
+          float a = __uint_as_float(r[0]) + head_bias<FOLD>(bias, 0);
           if (p.noise != nullptr) a += __ldg(p.noise + gq) * p.noise_std;
           if (valid) p.sigma[gq] = fmaxf(a, 0.f);
           }
         } else if (L.epi == FE_BOTT) {
-          fwd_cols_share<false, STASH, BM>(share, tlane, bias, cb, act_row, save_row, L.save_chunk, L.n_out, nullptr);
+          fwd_cols_share<false, STASH, FOLD>(share, tlane, bias, act_row, save_row, L.save_chunk, L.n_out, nullptr);
           // view-direction condition (models.py:410-419; viewdirs = raw directions, models.py:717-720)
           if constexpr (PRIMARY) {
           float f[C::KV], dir[3];
@@ -1271,13 +949,13 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
           }
         } else if (L.epi == FE_RGB0A) {
           if constexpr (!C::STATIC) {
-          fwd_cols_share<true, STASH, BM>(share, tlane, bias, cb, act_row, save_row, L.save_chunk, kRgbW,
+          fwd_cols_share<true, STASH, FOLD>(share, tlane, bias, act_row, save_row, L.save_chunk, kRgbW,
                                       STASH ? gate_row + (size_t)L.gate_word * kHalfRows : nullptr);
           if constexpr (PRIMARY) {
           uint32_t r[16];
           tmem_ld16(tlane + kRgbW, r);
           tmem_ld_wait();
-          float a = __uint_as_float(r[0]) + head_bias<BM>(bias, cb, kRgbW);
+          float a = __uint_as_float(r[0]) + head_bias<FOLD>(bias, kRgbW);
           if (p.noise != nullptr) a += __ldg(p.noise + gq) * p.noise_std;  // noise_regularize, model_utils.py:312-316
           if (valid) p.sigma[gq] = softplus_f(a);                         // models.py:491
           }
@@ -1288,23 +966,13 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
           tmem_ld_wait();
           if (valid) {
 #pragma unroll
-            for (int i = 0; i < 3; ++i) p.rgb[gq * 3 + i] = sigmoid_f(__uint_as_float(r[i]) + head_bias<BM>(bias, cb, i));
+            for (int i = 0; i < 3; ++i) p.rgb[gq * 3 + i] = sigmoid_f(__uint_as_float(r[i]) + head_bias<FOLD>(bias, i));
           }
         }
         if (li + 1 < prog.nlayers) {
           fence_proxy_async_smem();
           tc_fence_before();
-          { if (kPair) warp_arrive_leader(leader_ready); else warp_arrive(my_ready); }
-        }
-        if constexpr (STASH && kTmaStash) {
-          // the tile this layer left in ACT for the next layer's UMMAs is its stash slab: hand it to the copy engine
-          const bool wide = L.epi == FE_RELU || L.epi == FE_BOTT || L.epi == FE_LINEAR || L.epi == FE_RGB0A;
-          if (wide && L.save_chunk != kNone) {
-            if (li + 1 == prog.nlayers) fence_proxy_async_smem();
-            epi_named_barrier<PP>(chain);   // every row of the sub-tile is written (and fenced towards the async proxy)
-            stash_tile_bulk(act + sub * SM::ACT_BYTES, p.saved, (size_t)tile * (2 * kSubTiles) + sub * 2, p.x_total, L.save_chunk,
-                            (L.epi == FE_RGB0A ? kRgbW : (int)L.n_out) >> 3, quarter, lane, stash_policy);
-          }
+          warp_arrive(my_ready);
         }
 #if HN_ROLE_TIMING
         // per-layer profile of CTA 0 (profiles/role_timing.py): [wait for the accumulator, drain] after the 8 role counters
@@ -1316,7 +984,6 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
         (void)t_layer; (void)t_drain;
       }
     }
-    if constexpr (STASH && kTmaStash) bulk_wait_all();   // the slabs are in global memory before the CTA retires
     if (p.dbg && threadIdx.x == 0) {
       const long long tt = HN_T0() - t_begin;
       p.dbg[blockIdx.x * 8 + 4] = t_acc; p.dbg[blockIdx.x * 8 + 5] = tt - t_acc - t_pro;
@@ -1329,8 +996,7 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_fwd_kernel(const 
   }
   tc_fence_before();
   __syncthreads();
-  if (kPair) cluster_sync_all();   // the leader's UMMAs read this CTA's shared memory and TMEM until the very end
-  if (warp == kIssuerWarp) { if (kPair) tmem_dealloc2(tmem_base, 256 * kSubTiles); else tmem_dealloc(tmem_base, 256 * kSubTiles); }
+  if (warp == kIssuerWarp) tmem_dealloc(tmem_base, 256 * kSubTiles);
 }
 
 // d(trunk input features) in this row's accumulator columns [0, KT) -> d(warped point, hyper coordinates) through the
@@ -1383,11 +1049,11 @@ __device__ __forceinline__ void trunk_in_bwd(uint32_t tlane, const float* wp, fl
 // backward-data
 // ======================================================================================================
 template <class C>
-__global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(const __grid_constant__ BwdParams p) {
+__global__ void __launch_bounds__(kMlpThreads, 1) mlp_dgrad_kernel(const __grid_constant__ BwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   using SM = SmemBwd<C>;
   using Ring = RingStateT<SM::STAGES>;
-  constexpr bool PP = kPingPongBwd;
+  constexpr bool PP = true;   // sub-tiles out of phase (see Sched)
   uint8_t* act = smem + SM::ACT;
   uint8_t* inb = smem + SM::INB;
   uint8_t* ring = smem + SM::RING;
@@ -1398,21 +1064,15 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(cons
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(smem + SM::TMEMP);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
-  uint64_t* peer_full = act_ready + 2;        // [kRingStages], pair mode: the other CTA's half of a stage has landed
-  const uint32_t rank = kPair ? cluster_ctarank() : 0;
   if (threadIdx.x == 0) {
-    for (int i = 0; i < SM::STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); mbar_init(&peer_full[i], 1); }
-    // one arrival per epilogue warp of the chain (pair mode: of both CTAs, the other CTA's arrive remotely)
-    for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&act_ready[i], 4 * Sched<PP>::SUBS * kEpiSplit * (kPair ? 2 : 1)); }
+    for (int i = 0; i < SM::STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
+    // one arrival per epilogue warp of the chain
+    for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&act_ready[i], 4 * Sched<PP>::SUBS * kEpiSplit); }
     fence_barrier_init();
   }
-  if (warp == kIssuerWarp) {
-    if (kPair) { tmem_alloc2(tmem_ptr, 256 * kSubTiles); tmem_relinquish2(); }
-    else { tmem_alloc(tmem_ptr, 256 * kSubTiles); tmem_relinquish(); }
-  }
+  if (warp == kIssuerWarp) { tmem_alloc(tmem_ptr, 256 * kSubTiles); tmem_relinquish(); }
   tc_fence_before();
   __syncthreads();
-  if (kPair) cluster_sync_all();   // barriers of both CTAs are initialised before any remote arrive / multicast commit
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   const Program& prog = p.prog;
@@ -1422,37 +1082,24 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(cons
     if (warp == kProducerWarp && lane == 0) {
       Ring rs;
       long long tw = 0;
-      for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
-        if (kPair) produce_tile_pair(prog, p.maps, p.w_row0, p.weights, ring, full, empty, rs, rank, tw);
-        else produce_tile<PP>(prog, p.weights, ring, full, empty, rs, tw);
-      }
+      for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) produce_tile<PP>(prog, p.weights, ring, full, empty, rs, tw);
       if (p.dbg) p.dbg[blockIdx.x * 8 + 0] = tw;
-    } else if (kPair && !HN_PAIR_DIRECT && warp == kRelayWarp && lane == 0 && rank == 1) {
-      Ring rs;
-      const uint32_t leader_peer_full = mapa_u32(peer_full, 0);
-      for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) relay_tile_pair(prog, full, leader_peer_full, rs);
-    } else if (warp == kIssuerWarp && (!kPair || rank == 0)) {  // whole warp, converged: see elect_one_sync()
+    } else if (warp == kIssuerWarp) {  // whole warp, converged: see elect_one_sync()
       Ring rs;
       uint32_t ph_ready = 0;
-      long long t_ready = 0, t_full = 0, t_peer = 0;
+      long long t_ready = 0, t_full = 0;
       const long long t_begin = HN_T0();
       const uint32_t act_s = smem_u32(act), inb_s = smem_u32(inb), ring_s = smem_u32(ring);
       for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
         for (int li = 0; li < prog.nlayers; ++li) {
           for (int chain = 0; chain < Sched<PP>::CHAINS; ++chain) {
             long long t0 = HN_T0();
-            if (kPair) mbar_wait_cluster(&act_ready[chain], ph_ready); else mbar_wait(&act_ready[chain], ph_ready);
+            mbar_wait(&act_ready[chain], ph_ready);
             t_ready += HN_T0() - t0;
             tc_fence_after();
-            if (kPair) {
-              issue_layer_pair(prog, prog.layers[li], chain * Sched<PP>::SUBS, act_s, inb_s, SM::ACT_BYTES, SM::INB_BYTES, ring_s,
-                               tmem_base, full, peer_full, empty, rs, t_full, t_peer);
-              if (elect_one_sync()) umma2_commit_mc(&acc_full[chain], 3);   // accumulators of both CTAs are complete
-            } else {
-              issue_layer<PP>(prog, prog.layers[li], chain * Sched<PP>::SUBS, act_s, inb_s, SM::ACT_BYTES, SM::INB_BYTES, ring_s, tmem_base,
-                          full, empty, rs, t_full);
-              if (elect_one_sync()) umma_commit(&acc_full[chain]);
-            }
+            issue_layer<PP>(prog, prog.layers[li], chain * Sched<PP>::SUBS, act_s, inb_s, SM::ACT_BYTES, SM::INB_BYTES, ring_s, tmem_base,
+                        full, empty, rs, t_full);
+            if (elect_one_sync()) umma_commit(&acc_full[chain]);
             __syncwarp();
           }
           ph_ready ^= 1;
@@ -1460,7 +1107,6 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(cons
       }
       if (p.dbg && lane == 0) {
         p.dbg[blockIdx.x * 8 + 1] = t_ready; p.dbg[blockIdx.x * 8 + 2] = t_full; p.dbg[blockIdx.x * 8 + 3] = HN_T0() - t_begin;
-        if (kPair && !HN_PAIR_DIRECT) p.dbg[blockIdx.x * 8 + 0] = t_peer;   // relay variant: issuer's wait for the other CTA's half stage
       }
     }
   } else {
@@ -1476,11 +1122,9 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(cons
     const int chain = PP ? sub : 0;
     uint64_t* my_acc = &acc_full[chain];
     uint64_t* my_ready = &act_ready[chain];
-    const uint32_t leader_ready = kPair ? mapa_u32(my_ready, 0) : 0;
     uint32_t ph_acc = 0;
     long long t_acc = 0, t_pro = 0;
     const long long t_begin = HN_T0();
-    const uint64_t stash_policy = kTmaStash ? l2_policy_evict_first() : 0;
     for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
       const long long t_tile = HN_T0();
       const int64_t g = (int64_t)tile * kCtaRows + sub * kTileRows + row;
@@ -1516,31 +1160,18 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(cons
       }
       fence_proxy_async_smem();
       tc_fence_before();
-      { if (kPair) warp_arrive_leader(leader_ready); else warp_arrive(my_ready); }
+      warp_arrive(my_ready);
       t_pro += HN_T0() - t_tile;
 
       float gx_skip[C::STATIC ? 1 : C::NWARPED] = {};   // skip-layer part of d(warped point, hyper coordinates)
-      // HN_TMA_STASH: the gradient tile a wide layer leaves in ACT is its dY slab (see stash_tile_bulk)
-      auto stash_tile = [&](const Layer& L, int ncols) {
-        if constexpr (kTmaStash) {
-          epi_named_barrier<PP>(chain);   // every row of the sub-tile is written (and fenced towards the async proxy)
-          stash_tile_bulk(act + sub * SM::ACT_BYTES, p.dsaved, (size_t)tile * (2 * kSubTiles) + sub * 2, p.d_total, L.save_chunk,
-                          ncols >> 3, quarter, lane, stash_policy);
-        }
-      };
       for (int li = 0; li < prog.nlayers; ++li) {
         const Layer& L = prog.layers[li];
-        if constexpr (kTmaStash) {   // the copy engine is done reading ACT before this layer's drain overwrites it
-          bulk_wait_read_all();
-          epi_named_barrier<PP>(chain);
-        }
         if (L.epi == BE_MASK) {
           if (L.n_out == kTrunkW) bwd_masked_share<kTrunkW>(share, tlane, gate_row, L.gate_word, act_row, save_row, L.save_chunk, my_acc, ph_acc, t_acc);
           else if (L.n_out == kWsW) bwd_masked_share<kWsW>(share, tlane, gate_row, L.gate_word, act_row, save_row, L.save_chunk, my_acc, ph_acc, t_acc);
           else bwd_masked_share<kRgbW>(share, tlane, gate_row, L.gate_word, act_row, save_row, L.save_chunk, my_acc, ph_acc, t_acc);
           fence_proxy_async_smem();
-          if (li + 1 < prog.nlayers) { tc_fence_before(); { if (kPair) warp_arrive_leader(leader_ready); else warp_arrive(my_ready); } }
-          stash_tile(L, L.n_out);
+          if (li + 1 < prog.nlayers) { tc_fence_before(); warp_arrive(my_ready); }
           continue;
         }
         if (!C::STATIC && L.epi == BE_RGB1) {
@@ -1553,8 +1184,7 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(cons
           if (valid) f[0] = __ldg(p.g_sigma + gq) * (-expm1f(-__ldg(p.sigma + gq)));
           store_features<16>(f, act_row + (kRgbW / 8) * kChunkBytes, save_row, L.save_chunk + kRgbW / 8);
           }
-          fence_proxy_async_smem(); tc_fence_before(); { if (kPair) warp_arrive_leader(leader_ready); else warp_arrive(my_ready); }
-          stash_tile(L, kRgbW);
+          fence_proxy_async_smem(); tc_fence_before(); warp_arrive(my_ready);
           continue;
         }
         { long long t0 = HN_T0(); mbar_wait(my_acc, ph_acc); ph_acc ^= 1; t_acc += HN_T0() - t0; }
@@ -1649,15 +1279,10 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(cons
         if (li + 1 < prog.nlayers) {
           fence_proxy_async_smem();
           tc_fence_before();
-          { if (kPair) warp_arrive_leader(leader_ready); else warp_arrive(my_ready); }
-        }
-        if (L.epi == BE_LINEAR || L.epi == BE_LINCOND) {
-          if (li + 1 == prog.nlayers) fence_proxy_async_smem();
-          stash_tile(L, L.n_out);
+          warp_arrive(my_ready);
         }
       }
     }
-    if constexpr (kTmaStash) bulk_wait_all();   // the slabs are in global memory before the CTA retires
     if (p.dbg && threadIdx.x == 0) {
       const long long tt = HN_T0() - t_begin;
       p.dbg[blockIdx.x * 8 + 4] = t_acc; p.dbg[blockIdx.x * 8 + 5] = tt - t_acc - t_pro;
@@ -1669,10 +1294,10 @@ __global__ void __launch_bounds__(kMlpThreads, kCtasPerSm) mlp_dgrad_kernel(cons
   }
   tc_fence_before();
   __syncthreads();
-  if (kPair) cluster_sync_all();   // the leader's UMMAs read this CTA's shared memory and TMEM until the very end
-  if (warp == kIssuerWarp) { if (kPair) tmem_dealloc2(tmem_base, 256 * kSubTiles); else tmem_dealloc(tmem_base, 256 * kSubTiles); }
+  if (warp == kIssuerWarp) tmem_dealloc(tmem_base, 256 * kSubTiles);
 }
 
+#ifndef HN_MLP_FWD_VARIANT   // the split-epilogue copy holds the inference forward kernels only
 // ======================================================================================================
 // weight gradient: for every job, D[N_j, K_j] += dY^T X over this CTA's half tiles (UMMA with both operands
 // MN-major straight out of the stash layout), bias gradient by column sums on the CUDA cores.
@@ -1688,16 +1313,10 @@ struct WgSmem {
 };
 // Job groups: CTAs of group g run only the jobs with WgradJob::group == g, over 1/(CTAs per group) of the half tiles
 // each.  Jobs are spread over the groups by their operand bytes per half tile (the kernel is HBM-bound), largest first.
-// HN_WGRAD_GROUPS overrides; default 8 groups for the ~30-job tables of the hyper model (measured at 0.5 / 1 / 2 M samples per
-// launch: 8 groups beat 4 by 5 / 2.5 / 3 %, 12 and 16 lose to load imbalance) and 4 for the short tables (static NeRF: 12 jobs,
-// 4 groups 502 k against 497 k rays/s with 8).
-static int wgrad_groups(int njobs) {
-  static const int g = [] {
-    const char* e = getenv("HN_WGRAD_GROUPS");
-    return (e && atoi(e) > 0) ? std::min(atoi(e), 16) : 0;   // unset, empty or 0: the rule below
-  }();
-  return g ? g : (njobs >= 24 ? 8 : 4);
-}
+// 8 groups for the ~30-job tables of the hyper model (measured at 0.5 / 1 / 2 M samples per launch: 8 groups beat 4 by
+// 5 / 2.5 / 3 %, 12 and 16 lose to load imbalance) and 4 for the short tables (static NeRF: 12 jobs, 4 groups 502 k against
+// 497 k rays/s with 8).
+static int wgrad_groups(int njobs) { return njobs >= 24 ? 8 : 4; }
 // Spreads the jobs over the groups (largest first) and the grid's CTAs over the groups: every CTA of a group streams the
 // group's bytes over 1 / (its CTAs) of the half tiles, so the CTA counts follow the groups' bytes (each next CTA goes to the
 // group with the most bytes per CTA).  Round-robin CTA assignment left the heaviest group 6 % above the mean at 8 groups
@@ -1715,9 +1334,8 @@ static void assign_wgrad_groups(WgradTable& t, int groups, int grid, int16_t* gr
     load[best] += cost(order[k]);
   }
   int ctas[16];
-  static const bool even = [] { const char* e = getenv("HN_WGRAD_EVEN_CTAS"); return e && e[0] == '1'; }();   // A/B: equal CTA counts
-  for (int g = 0; g < groups; ++g) ctas[g] = even ? (grid - g + groups - 1) / groups : 1;
-  for (int c = groups; c < grid && !even; ++c) {
+  for (int g = 0; g < groups; ++g) ctas[g] = 1;
+  for (int c = groups; c < grid; ++c) {
     int best = 0;
     for (int g = 1; g < groups; ++g)
       if (load[g] * ctas[best] > load[best] * ctas[g]) best = g;
@@ -1771,12 +1389,6 @@ __global__ void __launch_bounds__(192, 1) mlp_wgrad_kernel(const __grid_constant
 
   if (warp == 0) {
     if (lane == 0 && h0 < h1) {
-#if HN_L2_HINTS & 2
-      const uint64_t once = l2_policy_evict_first();   // the stash streams through once; dW (atomics) should stay in L2
-#define HN_WG_LOAD(dst, src, bytes, bar) bulk_g2s_hint(dst, src, bytes, bar, once)
-#else
-#define HN_WG_LOAD(dst, src, bytes, bar) bulk_g2s(dst, src, bytes, bar)
-#endif
       int slot = 0; uint32_t phase = 0;
       for (int ji = 0; ji < njobs; ++ji) {
         const WgradJob& J = p.tab.jobs[ji];
@@ -1787,10 +1399,10 @@ __global__ void __launch_bounds__(192, 1) mlp_wgrad_kernel(const __grid_constant
           uint8_t* st = smem + slot * kWgStageBytes;
           mbar_wait(&empty[slot], phase ^ 1);
           mbar_arrive_expect_tx(&full[slot], a_bytes + b0_bytes + b1_bytes);
-          HN_WG_LOAD(st, p.dsaved + ((size_t)h * p.d_total + J.dy_chunk) * kHalfChunkBytes, a_bytes, &full[slot]);
-          HN_WG_LOAD(st + kWgStageA, p.saved + ((size_t)h * p.x_total + J.x0_chunk) * kHalfChunkBytes, b0_bytes, &full[slot]);
+          bulk_g2s(st, p.dsaved + ((size_t)h * p.d_total + J.dy_chunk) * kHalfChunkBytes, a_bytes, &full[slot]);
+          bulk_g2s(st + kWgStageA, p.saved + ((size_t)h * p.x_total + J.x0_chunk) * kHalfChunkBytes, b0_bytes, &full[slot]);
           if (b1_bytes)
-            HN_WG_LOAD(st + kWgStageA + b0_bytes, p.saved + ((size_t)h * p.x_total + J.x1_chunk) * kHalfChunkBytes, b1_bytes,
+            bulk_g2s(st + kWgStageA + b0_bytes, p.saved + ((size_t)h * p.x_total + J.x1_chunk) * kHalfChunkBytes, b1_bytes,
                        &full[slot]);
           if (++slot == kWgStages) { slot = 0; phase ^= 1; }
         }
@@ -1952,11 +1564,8 @@ __global__ void pack_kernel(const __grid_constant__ PackParams p) {
   if (oi < p.tab.nops) {
     const PackOp& op = p.tab.ops[oi];
     const int npk = op.n * (op.k / 8);
-    for (int i0 = blockIdx.x * blockDim.x + threadIdx.x; i0 < npk; i0 += gridDim.x * blockDim.x) {
-      const int chunk = i0 / op.n, n = i0 % op.n;
-      // pair mode: [rank][chunk][N/2 rows] so that each CTA's half of consecutive chunks is one contiguous run
-      const int nh = op.n >> 1;
-      const int i = kPair ? ((n / nh) * (op.k / 8) + chunk) * nh + (n % nh) : i0;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < npk; i += gridDim.x * blockDim.x) {
+      const int chunk = i / op.n, n = i % op.n;
       float v[8];
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = 0.f;
@@ -1998,70 +1607,18 @@ __global__ void pack_kernel(const __grid_constant__ PackParams p) {
   }
 }
 
+#endif  // !HN_MLP_FWD_VARIANT
+
 // ------------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------------
 static unsigned long long* g_dbg = nullptr;
-// CTA tiles (256 rows); pair mode: both CTAs of a cluster always work, so the count is rounded up to even (the extra
-// tile re-evaluates the last sample with every output masked off; its stash rows exist and contribute zeros)
-static int64_t tiles_of(int64_t n) {
-  int64_t t = (n + kCtaRows - 1) / kCtaRows;
-  return kPair ? (t + 1) / 2 * 2 : t;
-}
-// pair mode: tensor maps over one packed blob (cached per blob pointer: the encoder is a host-side driver call)
-static int build_pair_maps(const void* blob, int64_t blob_bytes, PairMaps* out) {
-  if (!kPair) return 0;
-  static thread_local const void* cached_blob = nullptr;
-  static thread_local int64_t cached_bytes = 0;
-  static thread_local PairMaps cached;
-  if (blob == cached_blob && blob_bytes == cached_bytes) { *out = cached; return 0; }
-  static PFN_cuTensorMapEncodeTiled_v12000 enc = nullptr;
-  if (enc == nullptr) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q);
-    if (e != cudaSuccess || fn == nullptr || q != cudaDriverEntryPointSuccess)
-      return set_error(-20, "pair mode: cuTensorMapEncodeTiled is not available from this driver");
-    enc = (PFN_cuTensorMapEncodeTiled_v12000)fn;
-  }
-#if HN_PAIR_MAP2D
-  // 2-D view [64 bf16 = one 128-byte line][lines]: box = {64, 2^i} is a contiguous run of 2^i lines
-  const cuuint64_t dims[2] = {64, (cuuint64_t)(blob_bytes / 128)};
-  const cuuint64_t strides[1] = {128};
-  const cuuint32_t es[2] = {1, 1};
-  for (int i = 0; i < 9; ++i) {
-    const cuuint32_t box[2] = {64, (cuuint32_t)(1u << i)};
-    CUresult r = enc(&cached.m[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(blob), dims, strides, box, es,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(-21, "pair mode: cuTensorMapEncodeTiled failed");
-  }
-#else
-  const cuuint64_t dims[3] = {8, 8, (cuuint64_t)(blob_bytes / 128)};
-  const cuuint64_t strides[2] = {16, 128};
-  const cuuint32_t es[3] = {1, 1, 1};
-  for (int i = 0; i < 9; ++i) {
-    const cuuint32_t box[3] = {8, 8, (cuuint32_t)(1u << i)};
-    CUresult r = enc(&cached.m[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(blob), dims, strides, box, es,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(-21, "pair mode: cuTensorMapEncodeTiled failed");
-  }
-#endif
-  cached_blob = blob; cached_bytes = blob_bytes;
-  *out = cached;
-  return 0;
-}
+static int64_t tiles_of(int64_t n) { return (n + kCtaRows - 1) / kCtaRows; }   // CTA tiles (256 rows)
 
 template <class K, class P>
 static cudaError_t launch_mlp(K kernel, int grid, int smem, cudaStream_t stream, const P& params) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kMlpThreads); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = kPair ? 2 : 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, params);
+  kernel<<<grid, kMlpThreads, smem, stream>>>(params);
+  return cudaGetLastError();
 }
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize is set once per (kernel, device) instead of before every launch
@@ -2101,52 +1658,6 @@ static ModelPlan& cached_plan(const hn_model_desc& d, int level = -1, const int6
     }
   }
   return c.plan;
-}
-
-// ---- constant-memory bias slots (HN_CONST_BIAS) -------------------------------------------------------------------
-// c_bias holds the forward bias arrays of up to kConstSlots packed blobs per device.  A blob's array is copied in
-// (device to device, stream ordered) the first time a forward launch uses it after it was packed; hn_pack_weights
-// invalidates the slot of the blob it rewrites.  Slots are recycled least-recently-used; a slot last used on another
-// stream is handed over with a synchronisation of that stream (launches of one model on two streams at once are not a use
-// case of this library, but they must not read each other's biases).
-struct ConstSlot { const void* src = nullptr; cudaStream_t stream = nullptr; uint64_t stamp = 0; };
-static std::mutex g_const_mu;
-static ConstSlot g_const_slots[16][kConstSlots];
-static uint64_t g_const_stamp = 0;
-
-static void const_bias_invalidate(const void* src) {
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 16) return;
-  std::lock_guard<std::mutex> lock(g_const_mu);
-  for (auto& sl : g_const_slots[dev]) if (sl.src == src) sl.src = nullptr;
-}
-// returns the float offset of the blob's bias array inside c_bias, uploading it if needed; < 0 on error
-static int const_bias_offset(const float* src, int nfloats, cudaStream_t stream) {
-  if (nfloats > kMaxBiasFloats) return set_error(-22, "bias array larger than a constant-memory slot");
-  int dev = 0;
-  if (cudaError_t e = cudaGetDevice(&dev)) return -std::abs(set_cuda_error(e, "const bias: cudaGetDevice"));
-  if (dev < 0 || dev >= 16) return set_error(-23, "const bias: device index out of range");
-  std::lock_guard<std::mutex> lock(g_const_mu);
-  ConstSlot* slots = g_const_slots[dev];
-  int hit = -1, victim = 0;
-  for (int i = 0; i < kConstSlots; ++i) {
-    if (slots[i].src == src) hit = i;
-    if (slots[i].stamp < slots[victim].stamp) victim = i;
-  }
-  const int s = hit >= 0 ? hit : victim;
-  if (slots[s].stream != stream && slots[s].stamp != 0) {
-    // kernels of another stream may still be reading (hit) or must not see the overwrite (victim)
-    if (cudaError_t e = cudaStreamSynchronize(slots[s].stream)) { cudaGetLastError(); (void)e; }
-  }
-  if (hit < 0) {
-    cudaError_t e = cudaMemcpyToSymbolAsync(c_bias, src, (size_t)nfloats * 4, (size_t)s * kMaxBiasFloats * 4,
-                                            cudaMemcpyDeviceToDevice, stream);
-    if (e != cudaSuccess) return -std::abs(set_cuda_error(e, "const bias: cudaMemcpyToSymbolAsync"));
-    slots[s].src = src;
-  }
-  slots[s].stream = stream;
-  slots[s].stamp = ++g_const_stamp;
-  return s * kMaxBiasFloats;
 }
 
 }  // namespace hn
@@ -2203,7 +1714,6 @@ extern "C" int hn_pack_weights(const hn_model_desc* desc, const float* flat_para
   pp.glo_src = plan.info.glo_param >= 0 ? param_offsets[plan.info.glo_param] : 0;
   if (plan.info.glo_param >= 0 && pp.glo_src < 0) return set_error(-2, "hn_pack_weights: the GLO table of this configuration has no offset");
   pp.glo_floats = plan.info.glo_floats;
-  const_bias_invalidate((const uint8_t*)packed + plan.layout.bias_off);   // the blob's biases are about to change
   dim3 grid(16, plan.pack.nops + 1);
   pack_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(pp);
   return set_cuda_error(cudaGetLastError(), "hn_pack_weights");
@@ -2235,6 +1745,12 @@ static int shape_of(const hn_model_desc& d) {
     default: MACRO(CfgT); break;        \
   }
 
+template <class C, bool STASH>
+static int launch_fwd(const FwdParams& fp, int grid, void* stream) {
+  if (int rc = set_smem(mlp_fwd_kernel<C, STASH>, Smem<C>::TOTAL, "hn_mlp_fwd: smem attr")) return rc;
+  return set_cuda_error(launch_mlp(mlp_fwd_kernel<C, STASH>, grid, Smem<C>::TOTAL, (cudaStream_t)stream, fp), "hn_mlp_fwd");
+}
+
 // warped_in != NULL: trunk-only program (hn_mlp_fwd_trunk; always the case for a model without warp: warped_in = points)
 static int mlp_fwd_impl(const hn_model_desc* desc, const void* packed, const float* points, const float* warped_in,
                         const float* viewdirs, const int64_t* ids, const float* noise, float noise_std, int64_t B, int S,
@@ -2255,21 +1771,12 @@ static int mlp_fwd_impl(const hn_model_desc* desc, const void* packed, const flo
   if (B == 0) return 0;
   const ModelPlan& plan = cached_plan(*desc);
   FwdParams fp;
-  // programs without bias K steps: the stash-writing forward (biases in the epilogue) and, with HN_CONST_BIAS = 2, the
-  // inference forward as well
-  const bool nobias_prog = saved != nullptr ? !kFoldBiasTrain : kConstBias >= 2;
-  fp.prog = trunk ? (nobias_prog ? plan.fwd_trunk_train : plan.fwd_trunk) : (nobias_prog ? plan.fwd_train : plan.fwd);
+  // the stash-writing forward runs the programs without bias K steps and adds the biases in its epilogue
+  const bool train = saved != nullptr;
+  fp.prog = trunk ? (train ? plan.fwd_trunk_train : plan.fwd_trunk) : (train ? plan.fwd_train : plan.fwd);
   fp.warped_in = warped_in;
   fp.weights = (const uint8_t*)packed + plan.layout.fwd_off;
-  fp.w_row0 = (uint32_t)(plan.layout.fwd_off / 16);
-  if (int rc = build_pair_maps(packed, plan.layout.total, &fp.maps)) return rc;
   fp.bias = (const float*)((const uint8_t*)packed + plan.layout.bias_off);
-  fp.cbias = 0;
-  if (nobias_prog && kConstBias >= 1) {
-    const int nb = (int)((plan.layout.glo_off - plan.layout.bias_off) / 4);
-    fp.cbias = const_bias_offset(fp.bias, nb, (cudaStream_t)stream);
-    if (fp.cbias < 0) return fp.cbias;
-  }
   fp.glo = (const float*)((const uint8_t*)packed + plan.layout.glo_off);
   fp.points = points; fp.viewdirs = viewdirs; fp.ids = ids; fp.noise = noise; fp.noise_std = noise_std;
   fp.n = B * S; fp.S = S; fp.n_embed = desc->num_embeddings;
@@ -2285,40 +1792,32 @@ static int mlp_fwd_impl(const hn_model_desc* desc, const void* packed, const flo
   fp.g_total = plan.info.g_total;
   fp.gates = saved ? (uint32_t*)((uint8_t*)saved + (size_t)(2 * kSubTiles) * nt * plan.info.x_total * kHalfChunkBytes) : nullptr;
   fp.dbg = g_dbg;
-  int grid = (int)std::min<int64_t>(nt, (int64_t)mlp_grid_cap() * kCtasPerSm);
-#define HN_LAUNCH_FWD(CFG)                                                                                                   \
-  do {                                                                                                                       \
-    if (saved != nullptr) {                                                                                                  \
-      if (int rc = set_smem(mlp_fwd_kernel<CFG, true>, Smem<CFG>::TOTAL, "hn_mlp_fwd: smem attr")) return rc;                \
-      return set_cuda_error(launch_mlp(mlp_fwd_kernel<CFG, true>, grid, Smem<CFG>::TOTAL, (cudaStream_t)stream, fp), "hn_mlp_fwd"); \
-    }                                                                                                                        \
-    if (int rc = set_smem(mlp_fwd_kernel<CFG, false>, Smem<CFG>::TOTAL, "hn_mlp_fwd: smem attr")) return rc;                 \
-    return set_cuda_error(launch_mlp(mlp_fwd_kernel<CFG, false>, grid, Smem<CFG>::TOTAL, (cudaStream_t)stream, fp), "hn_mlp_fwd"); \
-  } while (0)
+  const int grid = (int)std::min<int64_t>(nt, num_sms());
+#ifdef HN_MLP_FWD_VARIANT   // the split-epilogue copy serves the launches without a stash only
+#define HN_LAUNCH_FWD(CFG) return launch_fwd<CFG, false>(fp, grid, stream)
+#else
+#define HN_LAUNCH_FWD(CFG) return train ? launch_fwd<CFG, true>(fp, grid, stream) : launch_fwd<CFG, false>(fp, grid, stream)
+#endif
   HN_DISPATCH_SHAPE(shape_of(*desc), HN_LAUNCH_FWD)
 #undef HN_LAUNCH_FWD
   return set_error(-1, "hn_mlp_fwd: unreachable");
 }
 
-#if defined(HN_FWD_VARIANT_LINKED) && !defined(HN_MLP_FWD_VARIANT)
+#if defined(HN_MLP_FV_LINKED) && !defined(HN_MLP_FWD_VARIANT)
 extern "C" int hn_mlp_fwd_fv(const hn_model_desc*, const void*, const float*, const float*, const int64_t*, const float*, float,
                              int64_t, int, const int32_t*, int, float*, float*, float*, void*, float*, void*);
 extern "C" int hn_mlp_fwd_trunk_fv(const hn_model_desc*, const void*, const float*, const float*, const int64_t*, const float*,
                                    float, int64_t, int, const int32_t*, int, float*, float*, float*, void*, void*);
-// HN_FWD_VARIANT in the environment: 0 = never, 1 = inference and training forward, 2 = inference forward only
-static bool fwd_variant_enabled(bool training) {
-  static const int mode = [] { const char* e = getenv("HN_FWD_VARIANT"); return (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : HN_FWD_VARIANT_DEFAULT; }();
-  return mode == 1 || (mode == 2 && !training);
-}
-#define HN_FWD_VARIANT_CALL(fn, ...) if (fwd_variant_enabled(saved != nullptr)) return fn(__VA_ARGS__)
+// every launch without a stash runs on the split-epilogue copy (hn_mlp_fv.o)
+#define HN_MLP_FV_CALL(fn, ...) if (saved == nullptr) return fn(__VA_ARGS__)
 #else
-#define HN_FWD_VARIANT_CALL(fn, ...)
+#define HN_MLP_FV_CALL(fn, ...)
 #endif
 
 extern "C" HN_FV_HIDDEN int hn_mlp_fwd(const hn_model_desc* desc, const void* packed, const float* points, const float* viewdirs,
                           const int64_t* ids, const float* noise, float noise_std, int64_t B, int S, const int32_t* pos,
                           int S_full, float* sigma, float* rgb, float* warped, void* saved, float* aux, void* stream) {
-  HN_FWD_VARIANT_CALL(hn_mlp_fwd_fv, desc, packed, points, viewdirs, ids, noise, noise_std, B, S, pos, S_full, sigma, rgb, warped,
+  HN_MLP_FV_CALL(hn_mlp_fwd_fv, desc, packed, points, viewdirs, ids, noise, noise_std, B, S, pos, S_full, sigma, rgb, warped,
                       saved, aux, stream);
   if (!points) return set_error(-2, "hn_mlp_fwd: null pointer");
   return mlp_fwd_impl(desc, packed, points, nullptr, viewdirs, ids, noise, noise_std, B, S, pos, S_full, sigma, rgb, warped,
@@ -2328,7 +1827,7 @@ extern "C" HN_FV_HIDDEN int hn_mlp_fwd(const hn_model_desc* desc, const void* pa
 extern "C" HN_FV_HIDDEN int hn_mlp_fwd_trunk(const hn_model_desc* desc, const void* packed, const float* warped_in, const float* viewdirs,
                                 const int64_t* ids, const float* noise, float noise_std, int64_t B, int S, const int32_t* pos,
                                 int S_full, float* sigma, float* rgb, float* warped, void* saved, void* stream) {
-  HN_FWD_VARIANT_CALL(hn_mlp_fwd_trunk_fv, desc, packed, warped_in, viewdirs, ids, noise, noise_std, B, S, pos, S_full, sigma, rgb,
+  HN_MLP_FV_CALL(hn_mlp_fwd_trunk_fv, desc, packed, warped_in, viewdirs, ids, noise, noise_std, B, S, pos, S_full, sigma, rgb,
                       warped, saved, stream);
   if (!warped_in) return set_error(-2, "hn_mlp_fwd_trunk: null pointer");
   return mlp_fwd_impl(desc, packed, nullptr, warped_in, viewdirs, ids, noise, noise_std, B, S, pos, S_full, sigma, rgb, warped,
@@ -2368,8 +1867,6 @@ static int mlp_bwd_impl(const hn_model_desc* desc, const void* packed, const int
     bp.prog = trunk ? plan.bwd_trunk : plan.bwd;
     bp.g_warped_out = g_warped_out;
     bp.weights = (const uint8_t*)packed + plan.layout.bwd_off;
-    bp.w_row0 = (uint32_t)(plan.layout.bwd_off / 16);
-    if (int rc = build_pair_maps(packed, plan.layout.total, &bp.maps)) return rc;
     bp.ids = ids; bp.sigma = sigma; bp.rgb = rgb; bp.warped = warped;
     bp.g_sigma = g_sigma; bp.g_rgb = g_rgb; bp.g_warped = g_warped;
     bp.points = points; bp.aux = aux;
@@ -2388,7 +1885,7 @@ static int mlp_bwd_impl(const hn_model_desc* desc, const void* packed, const int
     bp.x_total = plan.info.x_total; bp.d_total = plan.info.d_total;
     bp.d_rgbhead = plan.info.d_rgbhead; bp.d_sigma = plan.info.d_sigma;
     bp.dbg = g_dbg;
-    int grid = (int)std::min<int64_t>(nt, (int64_t)mlp_grid_cap() * kCtasPerSm);
+    const int grid = (int)std::min<int64_t>(nt, num_sms());
 #define HN_LAUNCH_BWD(CFG)                                                                                                  \
   do {                                                                                                                      \
     if (int rc = set_smem(mlp_dgrad_kernel<CFG>, SmemBwd<CFG>::TOTAL, "hn_mlp_bwd: dgrad smem attr")) return rc;            \
@@ -2406,7 +1903,7 @@ static int mlp_bwd_impl(const hn_model_desc* desc, const void* packed, const int
     wp.n_half = 2 * kSubTiles * nt;
     wp.x_total = plan.info.x_total; wp.d_total = plan.info.d_total;
     if (int rc = set_smem(mlp_wgrad_kernel, WgSmem::TOTAL, "hn_mlp_bwd: wgrad smem attr")) return rc;
-    int wgrid = (int)std::min<int64_t>(wp.n_half, (int64_t)wgrad_grid_cap());
+    const int wgrid = (int)std::min<int64_t>(wp.n_half, num_sms());
     wp.groups = wp.n_half >= 8 * (int64_t)wgrid ? std::min(wgrad_groups(wp.tab.njobs), wgrid) : 1;
     assign_wgrad_groups(wp.tab, wp.groups, wgrid, wp.group_start);
     mlp_wgrad_kernel<<<wgrid, 192, WgSmem::TOTAL, (cudaStream_t)stream>>>(wp);

@@ -51,7 +51,7 @@ struct Builder {
   Program* p;
   LogicalOps* lg;
   uint32_t w16 = 0;  // running weight offset (16-byte units)
-  int ones_col = -1; // forward programs with kFoldBias: INB column of the ones chunk pair (every op gets a bias K step)
+  int ones_col = -1; // folded-bias forward programs: INB column of the ones chunk pair (every op gets a bias K step)
   int lg_chunks = 0, lg_total = 0;   // chunk cursor inside / chunk count of the logical matrix being emitted
   void begin_layer(uint8_t epi, int n_out, int bias_off, uint16_t save_chunk, uint16_t mask_chunk, uint16_t gate_word = kNone) {
     Layer& L = p->layers[p->nlayers++];
@@ -64,8 +64,7 @@ struct Builder {
     o.kc0 = (uint16_t)kc0; o.kc_total = (uint16_t)kc_total;
     o.w_off16 = w16; o.n = (uint16_t)n; o.k = (uint16_t)k; o.a_chunk = (uint16_t)(a_col / 8);
     o.tmem_col = (uint16_t)tmem_col; o.src = s; o.acc_init = (uint8_t)acc_init; o.pad = 0;
-    const int rows_here = kPair ? n / 2 : n;   // pair mode: each CTA stages half of the N rows of every chunk
-    int cps = (kStageBytes / (rows_here * 16)) & ~1;
+    int cps = (kStageBytes / (n * 16)) & ~1;
     if (cps < 2) cps = 2;
     if (cps > k / 8) cps = k / 8;
     o.cps = (uint8_t)cps;
@@ -75,7 +74,7 @@ struct Builder {
   // One logical [n x k_total] weight matrix (+ 16 bias rows in the folded-bias forward programs), consumed by one or
   // more parts; the parts may sit in consecutive layers (split skip layer, see kMaxTrunkInInb).
   void begin_logical(int n, int k_total) {
-    const int kb = ones_col >= 0 ? 16 : 0;   // bias rows (hn_mlp_program.h: HN_FOLD_BIAS)
+    const int kb = ones_col >= 0 ? 16 : 0;   // bias rows (hn_mlp_program.h: bias folding)
     LogicalOp& l = lg->ops[lg->n++];
     l.w_off16 = w16; l.n = (uint16_t)n; l.k = (uint16_t)(k_total + kb);
     lg_chunks = 0; lg_total = (k_total + kb) / 8;
@@ -144,9 +143,8 @@ struct Packer {
     b.n0 = (uint16_t)n0; b.nn = (uint16_t)nn; b.k0 = (uint16_t)k0; b.kk = (uint16_t)kk;
     t->ops[cur].nblk++;
   }
-  // bias of output rows [n0, n0 + nn) of the current op into its last two K rows (kFoldBias)
+  // bias of output rows [n0, n0 + nn) of the current op into its last two K rows (folded-bias programs)
   void bias_rows(int param, int n0, int nn) {
-    if (!kFoldBias) return;
     const int k0 = t->ops[cur].k - 2;
     block(param, 0, 1, kBiasPairStride, n0, nn, k0, 2);
   }
@@ -175,7 +173,7 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
   // ------------------------------------------------------------------ forward program
   {
     Builder b{&plan->fwd, &plan->fwd_logical};
-    if (kFoldBias) b.ones_col = m.ones_col;
+    b.ones_col = m.ones_col;
     plan->fwd.flags = m.t_in_act ? PF_TIN_ACT : 0;
     int bias = 0;
     if (m.se3) {
@@ -708,7 +706,7 @@ static void build_plan_static(const hn_model_desc& d, ModelPlan* plan) {
   // ---------------------------------------------------------------- forward (nerf.py:84-123)
   {
     Builder b{&plan->fwd, &plan->fwd_logical};
-    if (kFoldBias) {   // same rule as make_dims / Shape<>::INB_CHUNKS in hn_mlp.cu
+    {   // same rule as make_dims / Shape<>::INB_CHUNKS in hn_mlp.cu
       const int mx = s.KX > s.KV ? s.KX : s.KV;
       const bool in_pad = ones_fit_in_pad(mx, s.KX, s.pe_x) && ones_fit_in_pad(mx, s.KV, s.pe_v);
       b.ones_col = (in_pad ? mx / 8 : mx / 8 + 2) * 8 - 16;

@@ -15,59 +15,30 @@
 
 namespace hn {
 
-// HN_SUBTILES = 2: one CTA per SM owns 256 samples as two 128-row sub-tiles that share every weight stage.
-// HN_SUBTILES = 1: two CTAs per SM of 128 samples each (half the shared memory / TMEM / registers per CTA): the two
-//                  CTAs run out of phase, so one's UMMAs overlap the other's epilogue and stash stores, at the price
-//                  of streaming the weights from L2 once per 128 instead of once per 256 samples.
-// Measured (profiles/README.md): with the 2 x 8 KB ring that fits next to a second CTA the weight stream starves the
-// UMMAs (fwd 2.83 -> 4.06 ms, dgrad 2.78 -> 3.92 ms per 1 M samples), so 2 is the shipped configuration.
-#ifndef HN_SUBTILES
-#define HN_SUBTILES 2
-#endif
-// HN_PAIR = 1: the fused kernels run on 2-CTA clusters.  A UMMA spans the pair (cta_group::2, M = 256 = one 128-row
-// sub-tile of each CTA) and takes half of every weight stage from each CTA's shared memory, so a pass over a layer's
-// weights serves 256 rows while each SM only ingests half of it; that makes the out-of-phase (ping-pong) schedule of
-// the two sub-tiles affordable: sub-tile 0's epilogue of both CTAs runs under sub-tile 1's UMMAs and vice versa.
-// Status: functionally complete (GPU parity tests pass with HN_PAIR=1; tests/helpers.py TILE_ROWS = 512) but not the
-// default.  Two variants were measured (profiles/README.md): (a) relay thread + remote arrive to tell the leader that
-// the peer's half stage landed, (b) HN_PAIR_DIRECT: tensor-map TMA loads whose cta_group::2 form signals the leader's
-// mbarrier directly, with a pair-friendly packed layout so that a half stage is one request.  In both the weight
-// refill round trip (UMMA commit multicast to both CTAs -> producers -> TMA -> complete_tx across the pair) is
-// ~3 000 cycles against ~1 200 in the single-CTA schedule, and the 48 KB ring that fits next to the 2 x 64 KB of
-// resident activations only holds ~1 500 cycles of UMMA work: the issuer waits ~40 % of its time for stages
-// (fwd 3.33 / dgrad 3.32 ms per 1 M samples against 2.77 / 2.71 in lock step).
-#ifndef HN_PAIR
-#define HN_PAIR 0
-#endif
-constexpr bool kPair = HN_PAIR && HN_SUBTILES == 2;
+// One CTA per SM owns 256 samples as two 128-row sub-tiles that share every weight stage.  (Two CTAs of 128 samples per
+// SM leave room for only a 2 x 8 KB weight ring, which starves the UMMAs: fwd 2.83 -> 4.06 ms, dgrad 2.78 -> 3.92 ms per
+// 1 M samples, profiles/README.md.)
 constexpr int kTileRows = 128;   // samples per sub-tile (= UMMA M = TMEM lanes)
-constexpr int kSubTiles = HN_SUBTILES;
-constexpr int kCtasPerSm = kSubTiles == 2 ? 1 : 2;
-// HN_EPI_SPLIT = 2: every sub-tile is drained by TWO warpgroups, each taking half of the accumulator columns of the wide
-// (ReLU / linear) layers.  A drain is latency bound per warp (one warp per scheduler issues ~0.2 instructions per clock:
-// TMEM load -> bias -> pack -> st.shared -> st.global chains), and in the out-of-phase schedule only one sub-tile drains at a
-// time, so half of the epilogue warps idled; the second warpgroup per sub-tile doubles the drain's memory-level parallelism.
-// The "primary" warpgroup of a sub-tile also does the per-row work (positional encodings, heads); the "secondary" one only
-// drains its column share and keeps the launch-time 96 registers.
-#ifndef HN_EPI_SPLIT
-#define HN_EPI_SPLIT 1
+constexpr int kSubTiles = 2;
+// The inference forward is compiled a second time (HN_MLP_FWD_VARIANT, hn_mlp.cu) with TWO epilogue warpgroups per
+// sub-tile, each taking half of the accumulator columns of the wide (ReLU / linear) layers.  A drain is latency bound per
+// warp (one warp per scheduler issues ~0.2 instructions per clock: TMEM load -> bias -> pack -> st.shared chains); the
+// second warpgroup per sub-tile doubles the drain's memory-level parallelism.  The "primary" warpgroup of a sub-tile also
+// does the per-row work (positional encodings, heads); the "secondary" one only drains its column share.
+#ifdef HN_MLP_FWD_VARIANT
+constexpr int kEpiSplit = 2;
+#else
+constexpr int kEpiSplit = 1;
 #endif
-constexpr int kEpiSplit = HN_EPI_SPLIT;
 constexpr int kMlpThreads = 128 + 128 * kSubTiles * kEpiSplit;   // epilogue warpgroups (kEpiSplit per sub-tile), then the feeder warpgroup: producer + UMMA issuer
 constexpr int kCtaRows = kTileRows * kSubTiles;
 constexpr int kHalfRows = 64;    // granularity of the saved-activation layout and of the wgrad K step
 constexpr int kChunkBytes = kTileRows * 16;      // one 8-column chunk of a 128-row smem operand
 constexpr int kHalfChunkBytes = kHalfRows * 16;  // one 8-column chunk of a 64-row global slab
-// weight ring: 48 KB beside the resident activations (two co-resident CTAs only have room for 2 x 8 KB)
-#ifndef HN_RING_STAGES
-#define HN_RING_STAGES (HN_SUBTILES == 2 ? 3 : 2)
-#endif
-#ifndef HN_STAGE_BYTES
-#define HN_STAGE_BYTES (HN_SUBTILES == 2 ? 16384 : 8192)
-#endif
-constexpr int kRingStages = HN_RING_STAGES;
-constexpr int kStageBytes = HN_STAGE_BYTES;
-// HN_FOLD_BIAS = 1: in the INFERENCE forward (no stash) every layer's bias rides in the UMMAs: one extra K = 16 step
+// weight ring: 3 x 16 KB beside the resident activations (6 x 8 KB measured slower)
+constexpr int kRingStages = 3;
+constexpr int kStageBytes = 16384;
+// Bias folding: in the INFERENCE forward (no stash) every layer's bias rides in the UMMAs: one extra K = 16 step
 // whose A operand is the last chunk pair of the input buffer INB — its last two columns hold 1.0 — and whose weight rows
 // are [0 x 14, bf16(b), bf16(b - bf16(b))] (two bf16 terms carry the fp32 bias to ~2^-17 relative).  The epilogue then
 // has no bias staging (global load -> shared, named barrier) and no LDS + FADD per column.  The ones live in the zero
@@ -75,10 +46,6 @@ constexpr int kStageBytes = HN_STAGE_BYTES;
 // chunk pair.  Measured per 1 M samples: inference 2.03 -> 1.90 ms; the training forward, whose drain is bound by the
 // stash stores and hides the bias adds under them, only pays for the extra K steps (2.76 -> 2.89 ms), so it runs the
 // same program without the bias steps (ModelPlan::fwd_train) and adds the biases in its epilogue.
-#ifndef HN_FOLD_BIAS
-#define HN_FOLD_BIAS 1
-#endif
-constexpr bool kFoldBias = HN_FOLD_BIAS != 0;
 constexpr bool ones_fit_in_pad(int kmax, int k, int in) { return k < kmax || in <= kmax - 2; }
 constexpr int kMaxOps = 64;
 constexpr int kMaxLayers = 28;
@@ -117,7 +84,7 @@ constexpr bool inb_ones_in_pad(int KW, int in_w, int KT, int in_t, int KV, int i
 }
 constexpr int inb_chunks_of(int KW, int in_w, int KT, int in_t, int KV, int in_v) {
   const int mx = inb_max_cols(KW, KT, KV);
-  return (kFoldBias && !inb_ones_in_pad(KW, in_w, KT, in_t, KV, in_v)) ? mx / 8 + 2 : mx / 8;
+  return !inb_ones_in_pad(KW, in_w, KT, in_t, KV, in_v) ? mx / 8 + 2 : mx / 8;
 }
 
 // Derived channel counts for a model descriptor.
@@ -132,7 +99,7 @@ struct Dims {
   int n_rgb0a;                     // rgb layer 0 merged with the alpha head (pad16(128 + 1))
   bool t_in_act;                   // trunk input vector lives in ACT (see kMaxTrunkInInb)
   int inb_chunks;                  // chunks of the shared input buffer (+2 when the ones columns do not fit in padding)
-  int ones_col;                    // first column of the chunk pair whose last two columns are 1.0 (kFoldBias)
+  int ones_col;                    // first column of the chunk pair whose last two columns are 1.0 (bias folding)
 };
 inline Dims make_dims(const hn_model_desc& d) {
   Dims m{};
@@ -239,7 +206,7 @@ struct MmaOp {
   uint8_t src;
   uint8_t acc_init;            // 1: accumulate onto what TMEM already holds
   uint8_t cps;                 // 8-col chunks of K per ring stage (even)
-  uint8_t pad;                 // 1: bias K step (HN_FOLD_BIAS), dropped from ModelPlan::fwd_train
+  uint8_t pad;                 // 1: bias K step (bias folding), dropped from ModelPlan::fwd_train
   uint16_t kc0, kc_total;      // first chunk of this op inside its logical weight matrix / that matrix's chunk count
 };
 // A weight matrix as the packer sees it: one [n x k] operand image; a skip layer's matrix is consumed by two
@@ -353,7 +320,7 @@ struct ModelPlan {
   SlabMap slabs;
   PlanInfo info;
   Program fwd, bwd;
-  Program fwd_train;  // fwd without the bias K steps (kFoldBias): the stash-writing forward adds biases in its epilogue
+  Program fwd_train;  // fwd without the bias K steps: the stash-writing forward adds biases in its epilogue
   // Trunk-only programs (hyper model): the template NeRF (trunk, bottleneck, rgb / alpha heads) for rows whose warped
   // point and hyper coordinates are already known — the fine level inherits the coarse depths, and the warp / sheet nets
   // are shared between the levels, so those rows' warp / sheet evaluations are the coarse pass's (hn_mlp_fwd_trunk).

@@ -74,54 +74,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
                ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
 }
-// the same with an L2 cache policy (createpolicy): evict_last for data every SM keeps re-reading (weights), evict_first
-// for data that streams through once (stash slabs)
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-__device__ __forceinline__ void bulk_g2s_hint(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar, uint64_t policy) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-               ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
-               : "memory");
-}
-// shared -> global bulk copy (the copy engine reads shared memory; no per-thread store instructions), bulk-group completion
-__device__ __forceinline__ void bulk_s2g_hint(void* gmem_dst, const void* smem_src, uint32_t bytes, uint64_t policy) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;"
-               ::"l"(gmem_dst), "r"(smem_u32(smem_src)), "r"(bytes), "l"(policy)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// all bulk groups of this thread have finished READING their shared-memory source (the global writes may still be in flight)
-__device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-// ... and have completed entirely (before the kernel's shared memory goes away)
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-// Tensor-map TMA load of a contiguous run of 128-byte blocks (3-D view [block][8 rows][8 bf16], box = 2^i blocks) into this CTA's shared memory whose completion (complete_tx) is signalled
-// on the LEADER CTA's mbarrier: the cta_group::2 form accepts the barrier of the pair's other CTA (bit 24 of the
-// shared::cluster address selects the CTA; cute/arch/copy_sm100_tma.hpp, SM100_TMA_2SM_LOAD_2D).  The plain
-// cp.async.bulk form faults when given a remote barrier (tried), hence the tensor map.
-__device__ __forceinline__ void tma_g2s_3d_pair(void* smem_dst, const void* tensor_map, int32_t block, uint64_t* bar_same_offset) {
-  asm volatile("cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-               ::"r"(smem_u32(smem_dst)), "l"(tensor_map), "r"(smem_u32(bar_same_offset) & 0xFEFFFFFFu), "r"(0), "r"(0), "r"(block)
-               : "memory");
-}
-// The same over a 2-D view [128-byte row = 64 bf16][rows]: the inner box dimension is a full 128-byte line instead of the
-// 16-byte rows of the 3-D view (which make the TMA engine issue one request per 16 bytes).
-__device__ __forceinline__ void tma_g2s_2d_pair(void* smem_dst, const void* tensor_map, int32_t block, uint64_t* bar_same_offset) {
-  asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-               ::"r"(smem_u32(smem_dst)), "l"(tensor_map), "r"(smem_u32(bar_same_offset) & 0xFEFFFFFFu), "r"(0), "r"(block)
-               : "memory");
-}
-// bulk L2 prefetch of a contiguous global range (bytes: multiple of 16)
-__device__ __forceinline__ void bulk_prefetch_l2(const void* gmem_src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gmem_src), "r"(bytes) : "memory");
-}
 // bulk async copy shared -> global (bulk group completion)
 __device__ __forceinline__ void bulk_s2g(void* gmem_dst, const void* smem_src, uint32_t bytes) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gmem_dst),
@@ -132,10 +84,6 @@ __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.comm
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() {
   asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
-}
-template <int N>
-__device__ __forceinline__ void bulk_wait() {
-  asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
 }
 
 // ----------------------------------------------------------------------------------------------
@@ -195,28 +143,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// Weight-stationary form (tcgen05.mma.ws, cta_group::1 only): the B operand is parked in collector buffer 0 by a `fill`
-// instruction and re-used by the following `lastuse` instruction instead of being read from shared memory again.  The two
-// sub-tiles of a CTA multiply DIFFERENT A rows with the SAME weight K-slice back to back in the lock-step schedule, so the
-// second read of every weight byte (the dominant shared-memory traffic of a UMMA: N x 32 B against M x 32 B for A) goes away.
-__device__ __forceinline__ void umma_ws_fill_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                                  uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.ws.cta_group::1.kind::f16.collector::b0::fill [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_ws_lastuse_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                                     uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.ws.cta_group::1.kind::f16.collector::b0::lastuse [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // arrive on an mbarrier when all previously issued UMMAs of this thread have completed
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -257,37 +183,6 @@ __device__ __forceinline__ void umma2_commit_mc(uint64_t* bar, uint16_t cta_mask
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
 }
-// address of `p` (own shared memory) as seen in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_u32(const void* p, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// wait with cluster-scope acquire (pairs with remote release arrivals)
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.b32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait_cluster(bar, parity)) {
-    if (++spins > (1u << 26)) {
-      printf("hn: cluster mbarrier watchdog block %d thread %d bar %u parity %u\n", blockIdx.x, threadIdx.x, smem_u32(bar), parity);
-      __trap();
-    }
-  }
-}
-
 // TMEM -> registers: 32 lanes x 32 bit, N consecutive columns per thread (thread t <- lane base+t)
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* r) {
   asm volatile(
@@ -307,15 +202,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* r) {
         "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
       : "r"(taddr));
 }
-// registers -> TMEM, same addressing (thread t -> lane base+t, 16 consecutive columns)
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* r) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // One elected lane of a CONVERGED warp.  The UMMA issuer must run its loop with all 32 lanes (warp-uniform control

@@ -4,7 +4,6 @@
 //
 // Reference semantics (cited per kernel): hypernerf/model_utils.py of songrise/HyperNeRF-torch.
 #include <stdint.h>
-#include <stdlib.h>
 #include "hn_api_internal.h"
 
 namespace hn {
@@ -1111,12 +1110,6 @@ extern "C" int hn_sample_coarse(const float* origins, const float* dirs, const f
   return set_cuda_error(cudaGetLastError(), "hn_sample_coarse");
 }
 
-// HN_SAMPLE_PDF_GENERIC=1 in the environment forces the generic kernel (A/B measurements, tests of both paths)
-static bool sample_pdf_fast_enabled() {
-  static const bool on = [] { const char* e = getenv("HN_SAMPLE_PDF_GENERIC"); return !(e && e[0] == '1'); }();
-  return on;
-}
-
 static int sample_pdf_impl(const float* z_coarse, const float* bins, const float* weights, int64_t w_stride,
                            const float* u, const float* origins, const float* dirs, int64_t B, int Nc, int nb, int Nf,
                            float* z_fine, float* points, int32_t* bin_idx, int32_t* pos_coarse, int32_t* pos_new,
@@ -1129,7 +1122,7 @@ static int sample_pdf_impl(const float* z_coarse, const float* bins, const float
   if (B == 0) return 0;
   // the model's shapes (in-kernel bins, 64 / 128 coarse depths, 64 / 128 new samples) take the fast kernel
   const bool aligned = (reinterpret_cast<uintptr_t>(z_fine) & 15) == 0 && (!points || (reinterpret_cast<uintptr_t>(points) & 15) == 0);
-  if (bins == nullptr && aligned && (Nc == 64 || Nc == 128) && (Nf == 64 || Nf == 128) && sample_pdf_fast_enabled()) {
+  if (bins == nullptr && aligned && (Nc == 64 || Nc == 128) && (Nf == 64 || Nf == 128)) {
     const unsigned blocks4 = (unsigned)((B + 3) / 4);
 #define HN_PDF_FAST(CP, FP)                                                                                                 \
     sample_pdf_fast_kernel<CP, FP><<<blocks4, 128, 0, (cudaStream_t)stream>>>(z_coarse, weights, w_stride, u, origins, dirs, B, \

@@ -12,12 +12,6 @@
 extern "C" {
 #endif
 
-/* scheduling experiment (profiles/overlap_wgrad.py; exported by both libraries, the state is per library): cap the
- * persistent grids of hn_mlp_fwd* / hn_mlp_bwd*_data at mlp_ctas CTAs and of hn_mlp_bwd*_weights at wgrad_ctas CTAs (0 = one
- * CTA per SM), so that a weight-gradient launch on a second stream can run beside forward / data-gradient launches on the SMs
- * they leave free.  Results do not depend on it.  Measured: no partition beats running the kernels back to back. */
-int hn_set_sm_partition(int mlp_ctas, int wgrad_ctas);
-
 /* test hook: one UMMA tile D[128,N] = A * B^T through the shared-memory layouts the MLP kernels use.
  * a_mn / b_mn = 0: operand given row-major [rows][K]; 1: given as [K][rows] (MN-major). */
 int hn_umma_probe(const void* A_bf16, const void* B_bf16, float* D, int N, int K, int a_mn, int b_mn, void* stream);

@@ -9,7 +9,7 @@ EXTRA = dict(nerf_alpha=None, warp_alpha=None, hyper_alpha=None, hyper_sheet_alp
 EMB = {'warp': list(range(100)), 'camera': [0], 'appearance': list(range(100)), 'time': list(range(100))}
 
 # saved-activation slab map (hn_mlp_program.h make_slabs, cfg-1 shape), in 8-column chunks
-TILE_ROWS = 256   # stash granularity: CTA tiles of 256 rows (512 with HN_PAIR=1: tile count rounded up to even)
+TILE_ROWS = 256   # stash granularity: CTA tiles of 256 rows
 X_IN_WS, X_HWS, X_IN_T, X_T, X_BOTT, X_IN_V, X_R, X_TOTAL = 0, 10, 154, 166, 454, 470, 476, 540
 
 
