@@ -26,6 +26,7 @@ HN_COMP_ACC_ALL = 2
 EXPORTS = [
     "hn_abi_version", "hn_last_error", "hn_query", "hn_pack_weights", "hn_sample_coarse", "hn_sample_pdf", "hn_sample_pdf_ranks",
     "hn_composite_fwd", "hn_composite_bwd", "hn_filter_sigma", "hn_mse_loss", "hn_make_ndc_rays", "hn_adam_step", "hn_mlp_fwd", "hn_mlp_bwd", "hn_mlp_bwd_data", "hn_mlp_bwd_weights", "hn_mlp_fwd_trunk", "hn_mlp_bwd_trunk", "hn_mlp_bwd_trunk_data", "hn_mlp_bwd_trunk_weights",
+    "hn_pack_weights_windowed", "hn_mlp_bwd_weights_windowed", "hn_mlp_bwd_trunk_weights_windowed",
 ]
 # microbenchmarks / descriptor probes: their own library and header (include/hypernerf_b200_probe.h), not the product ABI
 PROBE_LIB_PATH = os.path.join(_HERE, "libhypernerf_b200_probe.so")
@@ -96,6 +97,9 @@ def lib():
                                    C.POINTER(C.c_int64), vp, vp, vp, vp]
     L.hn_mlp_bwd_trunk_data.argtypes = L.hn_mlp_bwd_trunk.argtypes
     L.hn_mlp_bwd_trunk_weights.argtypes = L.hn_mlp_bwd_weights.argtypes
+    L.hn_pack_weights_windowed.argtypes = [C.POINTER(ModelDesc), vp, C.POINTER(C.c_int64), i32, vp, vp, vp]
+    L.hn_mlp_bwd_weights_windowed.argtypes = [C.POINTER(ModelDesc), vp, i64, i32, i32, C.POINTER(C.c_int64), vp, vp, vp, vp]
+    L.hn_mlp_bwd_trunk_weights_windowed.argtypes = L.hn_mlp_bwd_weights_windowed.argtypes
     if hasattr(L, "hn_debug_set_timing_buffer"):   # role-timing builds only (make timing; HN_LIB selects them)
         L.hn_debug_set_timing_buffer.argtypes = [vp]
         L.hn_debug_set_timing_buffer.restype = C.c_int

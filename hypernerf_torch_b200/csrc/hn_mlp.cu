@@ -1345,9 +1345,22 @@ static void assign_wgrad_groups(WgradTable& t, int groups, int grid, int16_t* gr
   for (int g = 0; g < groups; ++g) group_start[g + 1] = (int16_t)(group_start[g] + ctas[g]);
 }
 
+// Positional-encoding window w_k(alpha) = 0.5 (1 - cos(pi clamp(alpha - k, 0, 1))) of encoded column e (PackBlock::win_c):
+// exactly 1 for alpha >= k + 1 (cospif(1) = -1), exactly 0 for alpha <= k.
+__device__ __forceinline__ float pe_window(float alpha, uint8_t win_c, int e) {
+  const int C = win_c & ~kWinIdentity;
+  if (win_c & kWinIdentity) {
+    if (e < C) return 1.f;
+    e -= C;
+  }
+  const float x = fminf(fmaxf(alpha - (float)(e / (2 * C)), 0.f), 1.f);
+  return 0.5f * (1.f - cospif(x));
+}
+
 struct WgradParams {
   WgradTable tab;
   const uint8_t* saved; const uint8_t* dsaved;
+  const float* pe_alpha;   // windowed tables (mlp_wgrad_kernel<true>): device {warp, sheet, nerf, hyper} alphas
   float* flat_grad;
   int64_t n_half;
   int x_total, d_total;
@@ -1355,6 +1368,9 @@ struct WgradParams {
   int16_t group_start[17];   // CTAs [group_start[g], group_start[g + 1]) serve group g (share of the grid ~ the group's bytes)
 };
 
+// WIN: the X stash holds the unwindowed encodings, so the accumulator holds dY^T pe; a flush segment with a window
+// scales it by w on its way out (dW of W diag(w) = (dY^T pe) diag(w)).
+template <bool WIN>
 __global__ void __launch_bounds__(192, 1) mlp_wgrad_kernel(const __grid_constant__ WgradParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + WgSmem::BARS);
@@ -1523,15 +1539,24 @@ __global__ void __launch_bounds__(192, 1) mlp_wgrad_kernel(const __grid_constant
               // reductions when the row is 16-byte aligned (ld % 4 == 0, the wide layers), scalar ones otherwise
               float* dst = p.flat_grad + F.dst + (int64_t)(drow - F.row0) * F.ld + (c0 - (int)F.col0);
               const bool vec = (reinterpret_cast<uintptr_t>(dst) & 15) == 0;
+              uint32_t v[16];
+#pragma unroll
+              for (int j = 0; j < 16; ++j) v[j] = r[j];
+              if (WIN && F.win != kNoWin) {   // columns outside [col0, col0 + ncols) get a weight too but are not written
+                const float a = p.pe_alpha[F.win - 1];
+#pragma unroll
+                for (int j = 0; j < 16; ++j)
+                  v[j] = __float_as_uint(__uint_as_float(r[j]) * pe_window(a, F.win_c, (int)F.win_e0 + c0 + j - (int)F.col0));
+              }
 #pragma unroll
               for (int j = 0; j < 16; j += 4) {
                 const int col = c0 + j;
                 if (vec && col >= F.col0 && col + 4 <= F.col0 + F.ncols) {
-                  red_add_v4(dst + j, r[j], r[j + 1], r[j + 2], r[j + 3]);
+                  red_add_v4(dst + j, v[j], v[j + 1], v[j + 2], v[j + 3]);
                 } else {
 #pragma unroll
                   for (int jj = j; jj < j + 4; ++jj)
-                    if (c0 + jj >= F.col0 && c0 + jj < F.col0 + F.ncols) atomicAdd(dst + jj, __uint_as_float(r[jj]));
+                    if (c0 + jj >= F.col0 && c0 + jj < F.col0 + F.ncols) atomicAdd(dst + jj, __uint_as_float(v[jj]));
                 }
               }
             }
@@ -1553,6 +1578,7 @@ __global__ void __launch_bounds__(192, 1) mlp_wgrad_kernel(const __grid_constant
 struct PackParams {
   PackTable tab;
   const float* flat;
+  const float* pe_alpha;   // device {warp, sheet, nerf, hyper} alphas of the windowed tables; NULL: no window
   uint8_t* blob;
   int64_t bias_off, glo_off;
   int64_t glo_src;
@@ -1572,6 +1598,10 @@ __global__ void pack_kernel(const __grid_constant__ PackParams p) {
       for (int b = op.blk0; b < op.blk0 + op.nblk; ++b) {
         const PackBlock& B = p.tab.blocks[b];
         if (n < B.n0 || n >= B.n0 + B.nn) continue;
+        // windowed block: W diag(w) in fp32, rounded to bf16 below; the source column runs along k in the forward
+        // images (sk == 1) and along n in the transposed ones
+        const float a = p.pe_alpha != nullptr && B.win != kNoWin ? __ldg(p.pe_alpha + B.win - 1) : 0.f;
+        const bool win = p.pe_alpha != nullptr && B.win != kNoWin;
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           int k = chunk * 8 + j;
@@ -1582,6 +1612,7 @@ __global__ void pack_kernel(const __grid_constant__ PackParams p) {
               v[j] = k == B.k0 ? hi : bv - hi;
             } else {
               v[j] = __ldg(p.flat + B.src + (int64_t)(n - B.n0) * B.sn + (int64_t)(k - B.k0) * B.sk);
+              if (win) v[j] *= pe_window(a, B.win_c, (int)B.win_e0 + (B.sk == 1 ? k - B.k0 : n - B.n0));
             }
           }
         }
@@ -1637,13 +1668,14 @@ static int set_smem(K kernel, int bytes, const char* what) {
 // The layer programs / slab maps depend on the descriptor only, the pack and weight-gradient tables additionally on
 // (level, parameter offsets): both are cached per thread, so a launch does not rebuild several KB of tables.
 struct PlanCache {
-  bool have_plan = false, have_tables = false;
+  bool have_plan = false, have_tables = false, windowed = false;
   hn_model_desc desc;
   int level = -1;
   int64_t offs[HN_NUM_PARAM_TENSORS];
   ModelPlan plan;
 };
-static ModelPlan& cached_plan(const hn_model_desc& d, int level = -1, const int64_t* offsets = nullptr) {
+static ModelPlan& cached_plan(const hn_model_desc& d, int level = -1, const int64_t* offsets = nullptr,
+                              bool windowed = false) {
   static thread_local PlanCache c;
   if (!c.have_plan || memcmp(&c.desc, &d, sizeof(d)) != 0) {
     build_plan(d, &c.plan);
@@ -1651,10 +1683,10 @@ static ModelPlan& cached_plan(const hn_model_desc& d, int level = -1, const int6
   }
   if (offsets != nullptr) {
     const size_t nb = sizeof(int64_t) * c.plan.info.n_params;
-    if (!c.have_tables || c.level != level || memcmp(c.offs, offsets, nb) != 0) {
-      build_tables(d, level, offsets, &c.plan);
+    if (!c.have_tables || c.level != level || c.windowed != windowed || memcmp(c.offs, offsets, nb) != 0) {
+      build_tables(d, level, offsets, windowed, &c.plan);
       memcpy(c.offs, offsets, nb);
-      c.level = level; c.have_tables = true;
+      c.level = level; c.windowed = windowed; c.have_tables = true;
     }
   }
   return c.plan;
@@ -1699,15 +1731,16 @@ extern "C" int hn_query(const hn_model_desc* desc, int64_t n_samples, hn_sizes* 
   return 0;
 }
 
-extern "C" int hn_pack_weights(const hn_model_desc* desc, const float* flat_params, const int64_t* param_offsets, int level,
-                               void* packed, void* stream) {
+static int pack_impl(const hn_model_desc* desc, const float* flat_params, const int64_t* param_offsets, int level,
+                     void* packed, const float* pe_alpha, void* stream) {
   if (!desc || !flat_params || !param_offsets || !packed) return set_error(-2, "hn_pack_weights: null pointer");
   if (level < 0 || level > 1) return set_error(-1, "hn_pack_weights: level must be 0 or 1");
   if (int rc = validate_desc(*desc)) return rc;
-  const ModelPlan& plan = cached_plan(*desc, level, param_offsets);
+  const ModelPlan& plan = cached_plan(*desc, level, param_offsets, pe_alpha != nullptr);
   PackParams pp;
   pp.tab = plan.pack;
   pp.flat = flat_params;
+  pp.pe_alpha = pe_alpha;
   pp.blob = (uint8_t*)packed;
   pp.bias_off = plan.layout.bias_off;
   pp.glo_off = plan.layout.glo_off;
@@ -1717,6 +1750,18 @@ extern "C" int hn_pack_weights(const hn_model_desc* desc, const float* flat_para
   dim3 grid(16, plan.pack.nops + 1);
   pack_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(pp);
   return set_cuda_error(cudaGetLastError(), "hn_pack_weights");
+}
+
+extern "C" int hn_pack_weights(const hn_model_desc* desc, const float* flat_params, const int64_t* param_offsets, int level,
+                               void* packed, void* stream) {
+  return pack_impl(desc, flat_params, param_offsets, level, packed, nullptr, stream);
+}
+
+extern "C" int hn_pack_weights_windowed(const hn_model_desc* desc, const float* flat_params, const int64_t* param_offsets,
+                                        int level, void* packed, const float* pe_alpha, void* stream) {
+  if (!pe_alpha) return set_error(-2, "hn_pack_weights_windowed: null pe_alpha");
+  if (desc && is_static(*desc)) return set_error(-13, "hn_pack_weights_windowed: the static NeRF has no encoding window");
+  return pack_impl(desc, flat_params, param_offsets, level, packed, pe_alpha, stream);
 }
 
 #endif  // !HN_MLP_FWD_VARIANT
@@ -1841,7 +1886,8 @@ static int mlp_bwd_impl(const hn_model_desc* desc, const void* packed, const int
                         const int64_t* param_offsets, float* flat_grad, void* workspace, void* stream, bool do_data,
                         bool do_weights, bool trunk = false,
                         float* g_warped_out = nullptr,     // trunk: trunk-only programs (hn_mlp_bwd_trunk*)
-                        const float* points = nullptr, const float* aux = nullptr) {   // SE3 warp, full program only
+                        const float* points = nullptr, const float* aux = nullptr,     // SE3 warp, full program only
+                        const float* pe_alpha = nullptr) {   // windowed weight gradient (hn_mlp_bwd_*weights_windowed)
   if (!desc || !saved || !param_offsets || !flat_grad || !workspace) return set_error(-2, "hn_mlp_bwd: null pointer");
   const bool stat = desc && is_static(*desc);
   const bool nowarp = !stat && !has_warp(*desc);
@@ -1858,7 +1904,8 @@ static int mlp_bwd_impl(const hn_model_desc* desc, const void* packed, const int
   if (level < 0 || level > 1) return set_error(-1, "hn_mlp_bwd: level must be 0 or 1");
   if (int rc = validate_desc(*desc)) return rc;
   if (B == 0) return 0;
-  const ModelPlan& plan = cached_plan(*desc, level, param_offsets);
+  // the data gradient reads no offset-dependent table: only the weight gradient (re)builds them
+  const ModelPlan& plan = cached_plan(*desc, level, do_weights ? param_offsets : nullptr, pe_alpha != nullptr);
   const int64_t n = B * S;
   const int64_t nt = tiles_of(n);
   if (nt > 0x7fffffff) return set_error(-1, "hn_mlp_bwd: too many samples");
@@ -1899,14 +1946,16 @@ static int mlp_bwd_impl(const hn_model_desc* desc, const void* packed, const int
     WgradParams wp;
     wp.tab = trunk ? plan.wgrad_trunk : plan.wgrad;
     wp.saved = (const uint8_t*)saved; wp.dsaved = (const uint8_t*)workspace;
+    wp.pe_alpha = pe_alpha;
     wp.flat_grad = flat_grad;
     wp.n_half = 2 * kSubTiles * nt;
     wp.x_total = plan.info.x_total; wp.d_total = plan.info.d_total;
-    if (int rc = set_smem(mlp_wgrad_kernel, WgSmem::TOTAL, "hn_mlp_bwd: wgrad smem attr")) return rc;
+    const auto wgrad_kernel = pe_alpha != nullptr ? mlp_wgrad_kernel<true> : mlp_wgrad_kernel<false>;
+    if (int rc = set_smem(wgrad_kernel, WgSmem::TOTAL, "hn_mlp_bwd: wgrad smem attr")) return rc;
     const int wgrid = (int)std::min<int64_t>(wp.n_half, num_sms());
     wp.groups = wp.n_half >= 8 * (int64_t)wgrid ? std::min(wgrad_groups(wp.tab.njobs), wgrid) : 1;
     assign_wgrad_groups(wp.tab, wp.groups, wgrid, wp.group_start);
-    mlp_wgrad_kernel<<<wgrid, 192, WgSmem::TOTAL, (cudaStream_t)stream>>>(wp);
+    wgrad_kernel<<<wgrid, 192, WgSmem::TOTAL, (cudaStream_t)stream>>>(wp);
     if (int rc = set_cuda_error(cudaGetLastError(), "hn_mlp_bwd: wgrad launch")) return rc;
   }
   return 0;
@@ -1958,6 +2007,27 @@ extern "C" int hn_mlp_bwd_trunk_weights(const hn_model_desc* desc, const void* s
                                         const int64_t* param_offsets, float* flat_grad, const void* workspace, void* stream) {
   return mlp_bwd_impl(desc, nullptr, nullptr, nullptr, nullptr, nullptr, saved, nullptr, nullptr, nullptr, B, S, nullptr, 0,
                       level, param_offsets, flat_grad, (void*)workspace, stream, false, true, true, nullptr);
+}
+
+extern "C" int hn_mlp_bwd_weights_windowed(const hn_model_desc* desc, const void* saved, int64_t B, int S, int level,
+                                           const int64_t* param_offsets, float* flat_grad, const void* workspace,
+                                           const float* pe_alpha, void* stream) {
+  if (!pe_alpha) return set_error(-2, "hn_mlp_bwd_weights_windowed: null pe_alpha");
+  if (desc && is_static(*desc)) return set_error(-13, "hn_mlp_bwd_weights_windowed: the static NeRF has no encoding window");
+  return mlp_bwd_impl(desc, nullptr, nullptr, nullptr, nullptr, nullptr, saved, nullptr, nullptr, nullptr, B, S, nullptr, 0,
+                      level, param_offsets, flat_grad, (void*)workspace, stream, false, true, false, nullptr, nullptr, nullptr,
+                      pe_alpha);
+}
+
+extern "C" int hn_mlp_bwd_trunk_weights_windowed(const hn_model_desc* desc, const void* saved, int64_t B, int S, int level,
+                                                 const int64_t* param_offsets, float* flat_grad, const void* workspace,
+                                                 const float* pe_alpha, void* stream) {
+  if (!pe_alpha) return set_error(-2, "hn_mlp_bwd_trunk_weights_windowed: null pe_alpha");
+  if (desc && is_static(*desc))
+    return set_error(-13, "hn_mlp_bwd_trunk_weights_windowed: the static NeRF has no encoding window");
+  return mlp_bwd_impl(desc, nullptr, nullptr, nullptr, nullptr, nullptr, saved, nullptr, nullptr, nullptr, B, S, nullptr, 0,
+                      level, param_offsets, flat_grad, (void*)workspace, stream, false, true, true, nullptr, nullptr, nullptr,
+                      pe_alpha);
 }
 
 #if HN_ROLE_TIMING

@@ -1,6 +1,7 @@
 // Host-side construction of the layer programs, pack tables and weight-gradient job tables
 // (see hn_mlp_program.h).  Pure host code.
 #include <string.h>
+#include <algorithm>
 #include "hn_api_internal.h"
 #include "hn_mlp_program.h"
 
@@ -125,23 +126,65 @@ void slice_program(const Program& src, int l0, int l1, Program* dst) {
   }
 }
 
+// Positional-encoding windows by weight tensor: the source columns [c0, c1) of a tensor that read one encoder's output.
+struct WinSeg { int c0, c1; uint8_t win, win_c; };
+struct WinLayout {
+  uint8_t nseg[HN_NUM_PARAM_TENSORS] = {};
+  WinSeg seg[HN_NUM_PARAM_TENSORS][2];
+  void add(int param, int c0, int n, PeAlpha a, int C, bool identity) {
+    if (n > 0) seg[param][nseg[param]++] = WinSeg{c0, c0 + n, (uint8_t)(1 + a), (uint8_t)(C | (identity ? kWinIdentity : 0))};
+  }
+  // Splits the source columns [c, c + n) of `param` at its encoder boundaries: piece(offset, count, win, win_c, win_e0).
+  template <class F>
+  void split(int param, int c, int n, F piece) const {
+    int at = 0;
+    while (at < n) {
+      int end = n;
+      uint8_t win = kNoWin, win_c = 0; int e0 = 0;
+      for (int i = 0; i < nseg[param]; ++i) {
+        const WinSeg& s = seg[param][i];
+        if (c + at >= s.c0 && c + at < s.c1) { win = s.win; win_c = s.win_c; e0 = c + at - s.c0; end = std::min(end, s.c1 - c); }
+        else if (s.c0 > c + at) end = std::min(end, s.c0 - c);
+      }
+      piece(at, end - at, win, win_c, e0);
+      at = end;
+    }
+  }
+};
+
 // A tensor the configuration does not have carries a negative offset (include/hypernerf_b200.h): its pack blocks are left
 // out (the operand image stays zero), its gradient segments are dropped.
 struct Packer {
   PackTable* t;
   const int64_t* off;
+  const WinLayout* wl = nullptr;   // windowed tables: blocks are split at the encoder boundaries
   int cur = -1;
   void op(const LogicalOp& o) {
     cur = t->nops++;
     PackOp& po = t->ops[cur];
     po.w_off16 = o.w_off16; po.n = o.n; po.k = o.k; po.blk0 = (uint8_t)t->nblocks; po.nblk = 0; po.pad = 0;
   }
-  void block(int param, int64_t src_extra, int sn, int sk, int n0, int nn, int k0, int kk) {
-    if (off[param] < 0 || nn <= 0 || kk <= 0) return;
+  void raw_block(int param, int64_t src_extra, int sn, int sk, int n0, int nn, int k0, int kk, uint8_t win = kNoWin,
+                 uint8_t win_c = 0, int win_e0 = 0) {
     PackBlock& b = t->blocks[t->nblocks++];
     b.src = off[param] + src_extra; b.sn = sn; b.sk = sk;
     b.n0 = (uint16_t)n0; b.nn = (uint16_t)nn; b.k0 = (uint16_t)k0; b.kk = (uint16_t)kk;
+    b.win = win; b.win_c = win_c; b.win_e0 = (uint16_t)win_e0;
     t->ops[cur].nblk++;
+  }
+  // src_extra is the block's first source column (row 0): the forward images walk the columns along k (sk == 1), the
+  // transposed ones along n (sn == 1)
+  void block(int param, int64_t src_extra, int sn, int sk, int n0, int nn, int k0, int kk) {
+    if (off[param] < 0 || nn <= 0 || kk <= 0) return;
+    if (wl == nullptr || wl->nseg[param] == 0 || sk == kBiasPairStride || (sk != 1 && sn != 1)) {
+      raw_block(param, src_extra, sn, sk, n0, nn, k0, kk);
+      return;
+    }
+    const bool along_k = sk == 1;
+    wl->split(param, (int)src_extra, along_k ? kk : nn, [&](int o, int cnt, uint8_t win, uint8_t win_c, int e0) {
+      if (along_k) raw_block(param, src_extra + o, sn, sk, n0, nn, k0 + o, cnt, win, win_c, e0);
+      else raw_block(param, src_extra + o, sn, sk, n0 + o, cnt, k0, kk, win, win_c, e0);
+    });
   }
   // bias of output rows [n0, n0 + nn) of the current op into its last two K rows (folded-bias programs)
   void bias_rows(int param, int n0, int nn) {
@@ -334,15 +377,32 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
   I.n_params = HN_NUM_PARAM_TENSORS;
 }
 
-void build_tables(const hn_model_desc& d, int level, const int64_t* off, ModelPlan* plan) {
+void build_tables(const hn_model_desc& d, int level, const int64_t* off, bool windowed, ModelPlan* plan) {
   if (is_static(d)) { build_tables_static(off, plan); return; }
   const Dims& m = plan->dims;
   const SlabMap& s = plan->slabs;
   const bool cond = m.cond_a || m.cond_r;
+  // ------------------------------------------------------------------ positional-encoding windows
+  // (reference column space; the skip layers read [hidden | input vector])
+  WinLayout wl;
+  if (m.se3) {
+    wl.add(P_WARP_W(0), 0, m.pe_w, PE_WARP, 3, false);                 // posenc(points, 0, 8): bands of 6, no identity
+    wl.add(P_WARP_W(kSkip + 1), kSe3W, m.pe_w, PE_WARP, 3, false);
+  } else if (!m.nowarp) {
+    wl.add(P_WARP_W(0), 0, m.pe_w, PE_WARP, 3, true);                  // posenc_orig(points, 10)
+    wl.add(P_WARP_W(kSkip + 1), kWarpW, m.pe_w, PE_WARP, 3, true);
+    wl.add(P_SHEET_W(0), 0, m.pe_s, PE_SHEET, 3, true);                // posenc_orig(points, 7)
+    wl.add(P_SHEET_W(kSkip + 1), kSheetW, m.pe_s, PE_SHEET, 3, true);
+  }
+  for (int l : {0, kSkip + 1}) {                                       // posenc_orig(xyz) | posenc_orig(hyper point)
+    const int c = l == 0 ? 0 : kTrunkW;
+    wl.add(P_TRUNK_W(level, l), c, m.pe_x, PE_NERF, 3, true);
+    wl.add(P_TRUNK_W(level, l), c + m.pe_x, m.pe_h, PE_HYPER, m.H, true);
+  }
   // ------------------------------------------------------------------ pack table
   PackTable& t = plan->pack;
   memset(&t, 0, sizeof(t));
-  Packer pk{&t, off};
+  Packer pk{&t, off, windowed ? &wl : nullptr};
   const LogicalOps& F = plan->fwd_logical;
   int oi = 0;
   const int ldw5 = kWarpW + m.in_w, lds5 = kSheetW + m.in_s;
@@ -532,11 +592,17 @@ void build_tables(const hn_model_desc& d, int level, const int64_t* off, ModelPl
     j.mblocks = (uint8_t)((dy_cols + 127) / 128);
     return j;
   };
+  // `extra` is the segment's first source column; windowed tables split it at the encoder boundaries (<= 3 pieces)
   auto flush = [&](WgradJob& j, int param, int64_t extra, int ld, int row0, int nrows, int col0, int ncols) {
     if (off[param] < 0 || nrows <= 0 || ncols <= 0) return;
-    FlushSeg& f = j.flush[j.nflush++];
-    f.dst = off[param] + extra; f.ld = ld; f.row0 = (uint16_t)row0; f.nrows = (uint16_t)nrows;
-    f.col0 = (uint16_t)col0; f.ncols = (uint16_t)ncols;
+    auto piece = [&](int o, int cnt, uint8_t win, uint8_t win_c, int e0) {
+      FlushSeg& f = j.flush[j.nflush++];
+      f.dst = off[param] + extra + o; f.ld = ld; f.row0 = (uint16_t)row0; f.nrows = (uint16_t)nrows;
+      f.col0 = (uint16_t)(col0 + o); f.ncols = (uint16_t)cnt;
+      f.win = win; f.win_c = win_c; f.win_e0 = (uint16_t)e0;
+    };
+    if (windowed) wl.split(param, (int)extra, ncols, piece);
+    else piece(0, ncols, kNoWin, 0, 0);
   };
   auto bseg = [&](WgradJob& j, int param, int col0, int ncols) {
     if (off[param] < 0 || ncols <= 0) return;

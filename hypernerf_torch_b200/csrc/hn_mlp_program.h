@@ -248,10 +248,20 @@ struct LogicalOps {
 // dest(n, k) of an op's [N x K] bf16 matrix (interleave layout: ((k/8) * N + n) * 8 + k%8) is gathered from
 // flat_params[src + (n - n0) * sn + (k - k0) * sk] for the (n, k) inside a block; everything else is zero.
 constexpr int32_t kBiasPairStride = INT32_MIN;   // PackBlock::sk marker: rows k0, k0 + 1 = bf16(b[n]), bf16(b[n] - bf16(b[n]))
+// Positional-encoding window (include/hypernerf_b200.h, hn_pack_weights_windowed): a block / flush segment whose source
+// columns are encoded columns of one encoder carries the encoder's window spec.  The source column runs along k for the
+// forward images (sk == 1) and along n for the transposed ones (sn == 1); for a weight-gradient segment along its columns.
+// Encoded column e = win_e0 + (offset along that axis); with identity columns first (kWinIdentity), e < C is identity.
+// win = 1 + the index of the encoder's alpha in pe_alpha, 0 (kNoWin, what a zeroed table holds) for none.
+enum PeAlpha : uint8_t { PE_WARP = 0, PE_SHEET = 1, PE_NERF = 2, PE_HYPER = 3, kNumPeAlphas = 4 };
+constexpr uint8_t kNoWin = 0;
+constexpr uint8_t kWinIdentity = 0x80;  // win_c flag: C identity columns precede the bands; low 7 bits = C
 struct PackBlock {
   int64_t src;         // element offset in the flat fp32 parameter buffer
   int32_t sn, sk;      // source strides (elements)
   uint16_t n0, nn, k0, kk;
+  uint8_t win, win_c;  // window: 1 + pe_alpha index (kNoWin: none), channels | kWinIdentity
+  uint16_t win_e0;     // encoded column of the block's first source column
 };
 struct PackOp {
   uint32_t w_off16;
@@ -276,6 +286,8 @@ struct FlushSeg {
   int32_t ld;            // destination leading dimension
   uint16_t row0, nrows;  // rows in dY-column space of the job (row = mblock * 128 + lane row)
   uint16_t col0, ncols;
+  uint8_t win, win_c;    // window of the columns (PackBlock): the flush scales dY^T pe by w
+  uint16_t win_e0;
 };
 struct BiasSeg { int64_t dst; uint16_t col0, ncols; uint32_t pad; };
 struct WgradJob {
@@ -337,7 +349,8 @@ inline bool is_static(const hn_model_desc& d) { return (d.flags & HN_FLAG_STATIC
 int validate_desc(const hn_model_desc& d);
 // Static part (programs, slabs, blob layout).
 void build_plan(const hn_model_desc& d, ModelPlan* plan);
-// Offset-dependent part for one level.
-void build_tables(const hn_model_desc& d, int level, const int64_t* param_offsets, ModelPlan* plan);
+// Offset-dependent part for one level.  windowed: blocks / flush segments are split at the encoder boundaries and carry
+// window specs (the unwindowed tables are the same as without the feature).
+void build_tables(const hn_model_desc& d, int level, const int64_t* param_offsets, bool windowed, ModelPlan* plan);
 
 }  // namespace hn

@@ -21,7 +21,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib, model_utils, modules
-from ._packing import PackedWeights
+from ._packing import PackedWeights, pe_alphas
 from ._lib import check, lib, ptr, stream
 
 
@@ -79,6 +79,24 @@ def _param_grads(ctx, model, level, flat_grad, offs, first):
     return grads
 
 
+def _level_window(level):
+    """The `level` argument of the fused autograd functions: the level (0 coarse, 1 fine), or (level, encoding window of
+    _packing.pe_alphas) to run on a blob packed with that window."""
+    return (level, None) if isinstance(level, int) else level
+
+
+def _bwd_weights(model, trunk, saved, B, S, level, offs, flat_grad, work, pe_alpha):
+    """hn_mlp_bwd[_trunk]_weights, or their windowed forms for a blob packed with an encoding window."""
+    d, L = C.byref(model._desc), lib()
+    if pe_alpha is None:
+        fn, name, extra = (L.hn_mlp_bwd_trunk_weights, "hn_mlp_bwd_trunk_weights", ()) if trunk else \
+            (L.hn_mlp_bwd_weights, "hn_mlp_bwd_weights", ())
+    else:
+        fn, name, extra = (L.hn_mlp_bwd_trunk_weights_windowed, "hn_mlp_bwd_trunk_weights_windowed", (ptr(pe_alpha),)) \
+            if trunk else (L.hn_mlp_bwd_weights_windowed, "hn_mlp_bwd_weights_windowed", (ptr(pe_alpha),))
+    check(fn(d, ptr(saved), B, S, level, offs, ptr(flat_grad), ptr(work), *extra, stream()), name)
+
+
 class _FusedMlp(torch.autograd.Function):
     """hn_mlp_fwd / hn_mlp_bwd as one autograd node per level.  Inputs after the fixed arguments are the parameter
     tensors of the canonical slots this configuration has (include/hypernerf_b200.h); gradients come back as views of
@@ -90,7 +108,8 @@ class _FusedMlp(torch.autograd.Function):
         B, S = points.shape[0], points.shape[1]
         dev = points.device
         desc = model._desc
-        packed = model._packed_weights(level)
+        level, window = _level_window(level)
+        packed, pe_alpha = model._packed_window(level, window)
         pts = points.detach().to(torch.float32).contiguous()
         vd = viewdirs.detach().to(torch.float32).contiguous()
         ids = ids.reshape(-1).to(torch.int64).contiguous()
@@ -113,14 +132,14 @@ class _FusedMlp(torch.autograd.Function):
         _lib.count(1)
         ctx.model, ctx.level, ctx.shape = model, level, (B, S)
         ctx.param_meta = [(slot, p.shape, p.numel()) for slot, p in zip(model._slots_present(), params)]
-        ctx.save_for_backward(ids, sigma, rgb, warped, saved, packed, pts if aux is not None else None, aux)
+        ctx.save_for_backward(ids, sigma, rgb, warped, saved, packed, pts if aux is not None else None, aux, pe_alpha)
         ctx.set_materialize_grads(False)
         return sigma, rgb, warped
 
     @staticmethod
     @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, g_sigma, g_rgb, g_warped):
-        ids, sigma, rgb, warped, saved, packed, pts, aux = ctx.saved_tensors
+        ids, sigma, rgb, warped, saved, packed, pts, aux, pe_alpha = ctx.saved_tensors
         model, level = ctx.model, ctx.level
         B, S = ctx.shape
         if saved is None:
@@ -143,8 +162,7 @@ class _FusedMlp(torch.autograd.Function):
                                         ptr(saved), ptr(g_sigma), ptr(g_rgb), ptr(g_warped), B, S, None, 0, level, offs,
                                         ptr(flat_grad), ptr(work), ptr(pts), ptr(aux), stream()), "hn_mlp_bwd_data")
         with _lib.timed("mlp_wgrad", B * S):
-            check(lib().hn_mlp_bwd_weights(C.byref(model._desc), ptr(saved), B, S, level, offs, ptr(flat_grad), ptr(work),
-                                           stream()), "hn_mlp_bwd_weights")
+            _bwd_weights(model, False, saved, B, S, level, offs, flat_grad, work, pe_alpha)
         _lib.count(2)
         if direct:
             return (None,) * (7 + len(ctx.param_meta))
@@ -162,7 +180,8 @@ class _FusedTrunk(torch.autograd.Function):
         B, S = warped_in.shape[0], warped_in.shape[1]
         dev = warped_in.device
         desc = model._desc
-        packed = model._packed_weights(level)
+        level, window = _level_window(level)
+        packed, pe_alpha = model._packed_window(level, window)
         wi = warped_in.detach().to(torch.float32).contiguous()
         vd = viewdirs.detach().to(torch.float32).contiguous()
         sigma = torch.empty(B, S, device=dev, dtype=torch.float32)
@@ -181,14 +200,14 @@ class _FusedTrunk(torch.autograd.Function):
         _lib.count(1)
         ctx.model, ctx.level, ctx.shape = model, level, (B, S)
         ctx.param_meta = [(slot, p.shape, p.numel()) for slot, p in zip(model._slots_present(), params)]
-        ctx.save_for_backward(sigma, rgb, wi, saved, packed, ids)
+        ctx.save_for_backward(sigma, rgb, wi, saved, packed, ids, pe_alpha)
         ctx.set_materialize_grads(False)
         return sigma, rgb
 
     @staticmethod
     @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, g_sigma, g_rgb):
-        sigma, rgb, wi, saved, packed, ids = ctx.saved_tensors
+        sigma, rgb, wi, saved, packed, ids, pe_alpha = ctx.saved_tensors
         model, level = ctx.model, ctx.level
         B, S = ctx.shape
         if saved is None:
@@ -210,8 +229,7 @@ class _FusedTrunk(torch.autograd.Function):
                                               ptr(saved), ptr(g_sigma), ptr(g_rgb), None, B, S, None, 0, level, offs,
                                               ptr(flat_grad), ptr(g_wi), ptr(work), stream()), "hn_mlp_bwd_trunk_data")
         with _lib.timed("mlp_wgrad_trunk", B * S):
-            check(lib().hn_mlp_bwd_trunk_weights(C.byref(model._desc), ptr(saved), B, S, level, offs, ptr(flat_grad),
-                                                 ptr(work), stream()), "hn_mlp_bwd_trunk_weights")
+            _bwd_weights(model, True, saved, B, S, level, offs, flat_grad, work, pe_alpha)
         _lib.count(2)
         head = (None, None, g_wi if ctx.needs_input_grad[2] else None, None, None, None, None)
         if direct:
@@ -232,7 +250,8 @@ class _FusedFineLevel(torch.autograd.Function):
         Sk, Sn = pos_known.shape[1], pos_new.shape[1]
         dev = points.device
         desc = model._desc
-        packed = model._packed_weights(level)
+        level, window = _level_window(level)
+        packed, pe_alpha = model._packed_window(level, window)
         pts = points.detach().to(torch.float32).contiguous()
         vd = viewdirs.detach().to(torch.float32).contiguous()
         kw = known_warped.detach().to(torch.float32).contiguous()
@@ -263,14 +282,14 @@ class _FusedFineLevel(torch.autograd.Function):
         ctx.model, ctx.level, ctx.shape = model, level, (B, S, Sk, Sn)
         ctx.param_meta = [(slot, p.shape, p.numel()) for slot, p in zip(model._slots_present(), params)]
         ctx.save_for_backward(ids, sigma, rgb, warped, kw, saved_n, saved_k, packed, pos_known, pos_new,
-                              pts if aux is not None else None, aux)
+                              pts if aux is not None else None, aux, pe_alpha)
         ctx.set_materialize_grads(False)
         return sigma, rgb, warped
 
     @staticmethod
     @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, g_sigma, g_rgb, g_warped):
-        ids, sigma, rgb, warped, kw, saved_n, saved_k, packed, pos_known, pos_new, pts, aux = ctx.saved_tensors
+        ids, sigma, rgb, warped, kw, saved_n, saved_k, packed, pos_known, pos_new, pts, aux, pe_alpha = ctx.saved_tensors
         model, level = ctx.model, ctx.level
         B, S, Sk, Sn = ctx.shape
         if saved_n is None:
@@ -293,15 +312,13 @@ class _FusedFineLevel(torch.autograd.Function):
                                         ptr(g_rgb), ptr(g_warped), B, Sn, ptr(pos_new), S, level, offs, ptr(flat_grad),
                                         ptr(work), ptr(pts), ptr(aux), stream()), "hn_mlp_bwd_data")
         with _lib.timed("mlp_wgrad", B * Sn):
-            check(lib().hn_mlp_bwd_weights(d, ptr(saved_n), B, Sn, level, offs, ptr(flat_grad), ptr(work), stream()),
-                  "hn_mlp_bwd_weights")
+            _bwd_weights(model, False, saved_n, B, Sn, level, offs, flat_grad, work, pe_alpha)
         with _lib.timed("mlp_dgrad_trunk", B * Sk):
             check(lib().hn_mlp_bwd_trunk_data(d, ptr(packed), ptr(ids), ptr(sigma), ptr(rgb), ptr(kw), ptr(saved_k), ptr(g_sigma),
                                               ptr(g_rgb), ptr(g_warped), B, Sk, ptr(pos_known), S, level, offs, ptr(flat_grad),
                                               ptr(g_kw), ptr(work), stream()), "hn_mlp_bwd_trunk_data")
         with _lib.timed("mlp_wgrad_trunk", B * Sk):
-            check(lib().hn_mlp_bwd_trunk_weights(d, ptr(saved_k), B, Sk, level, offs, ptr(flat_grad), ptr(work), stream()),
-                  "hn_mlp_bwd_trunk_weights")
+            _bwd_weights(model, True, saved_k, B, Sk, level, offs, flat_grad, work, pe_alpha)
         _lib.count(4)
         head = (None,) * 7 + (g_kw if ctx.needs_input_grad[7] else None, None, None)
         if direct:
@@ -693,7 +710,8 @@ class NerfModel(PackedWeights, nn.Module):
         if not self.use_warp:
             raise AttributeError("'NerfModel' object has no attribute 'warp_field'")   # as in the reference
         params = self._canonical_params() if torch.is_grad_enabled() else [q.detach() for q in self._canonical_params()]
-        _, _, warped = _FusedMlp.apply(self, 0, points, self._zero_dirs(points), warp_embed, None, 0.0, *params)
+        _, _, warped = _FusedMlp.apply(self, (0, pe_alphas(extra_params)), points, self._zero_dirs(points), warp_embed,
+                                       None, 0.0, *params)
         return {'warped_points': warped[..., :3]}
 
     def map_points(self, points, warp_embed, hyper_embed, extra_params, use_warp=True, return_warp_jacobian=False,
@@ -713,7 +731,8 @@ class NerfModel(PackedWeights, nn.Module):
         view = self._embed_view(warp_embed)
         ids = torch.arange(points.shape[0], device=points.device, dtype=torch.int64)
         params = view._canonical_params() if torch.is_grad_enabled() else [q.detach() for q in view._canonical_params()]
-        _, _, warped = _FusedMlp.apply(view, 0, points, self._zero_dirs(points), ids, None, 0.0, *params)
+        _, _, warped = _FusedMlp.apply(view, (0, pe_alphas(extra_params)), points, self._zero_dirs(points), ids, None,
+                                       0.0, *params)
         return warped, None
 
     def map_spatial_points(self, points, warp_embed, extra_params, use_warp=True, return_warp_jacobian=False):
@@ -749,8 +768,9 @@ class NerfModel(PackedWeights, nn.Module):
             noise = torch.randn((B, S, 1), device=points.device, dtype=torch.float32)
             noise_std = float(self.noise_std)
         params = owner._canonical_params() if torch.is_grad_enabled() else [q.detach() for q in owner._canonical_params()]
-        with owner.packed_frozen():
-            sigma, rgb = _FusedTrunk.apply(owner, 1 if level == 'fine' else 0, points, viewdirs, ids, noise, noise_std, *params)
+        with owner.packed_frozen(extra_params):
+            sigma, rgb = _FusedTrunk.apply(owner, (1 if level == 'fine' else 0, pe_alphas(extra_params)), points, viewdirs,
+                                           ids, noise, noise_std, *params)
         return rgb, sigma
 
     def render_samples(self, level, points, z_vals, directions, viewdirs, metadata, extra_params, use_warp=True,
@@ -787,7 +807,7 @@ class NerfModel(PackedWeights, nn.Module):
             # autograd.Function reports needs_input_grad for parameters even under no_grad; detached parameters make
             # the eval path (eval.py:77 @torch.no_grad) take the inference kernel, which writes no activation stash
             params = [q.detach() for q in params]
-        lvl = 1 if level == 'fine' else 0
+        lvl = (1 if level == 'fine' else 0, pe_alphas(extra_params))
         if not self.use_warp:
             # map_points returns the raw points (models.py:568-569): the template alone
             sigma, rgb = _FusedTrunk.apply(owner, lvl, points, viewdirs, ids, noise, noise_std, *params)
@@ -817,7 +837,8 @@ class NerfModel(PackedWeights, nn.Module):
             raise RuntimeError(self._forward_error)
         if rays_dict['origins'].shape[0] == 0:
             raise ValueError("NerfModel.forward: empty ray batch (the reference fails on it too: model_utils.py:389, models.py:668)")
-        with self.packed_frozen():   # re-packs the bf16 weight blobs unless an enclosing block froze them (_packing.py)
+        # re-packs the bf16 weight blobs (with the encoding window of extra_params) unless an enclosing block froze them
+        with self.packed_frozen(extra_params):
             return self._forward(rays_dict, extra_params, metadata_encoded, use_warp, return_points, return_weights,
                                  return_warp_jacobian, near, far, use_sample_at_infinity, render_opts, deterministic)
 

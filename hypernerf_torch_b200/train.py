@@ -11,7 +11,7 @@ ShardedDDP gradient reduction (train.py:224-229) do, without Lightning.
 import torch
 import torch.distributed as dist
 
-from . import _lib, losses, model_utils
+from . import _lib, _packing, losses, model_utils
 
 EXTRA_PARAMS = {'nerf_alpha': None, 'warp_alpha': None, 'hyper_alpha': None, 'hyper_sheet_alpha': None}
 
@@ -115,22 +115,30 @@ def shard_bounds(n, rank, world):
     return lo, min(lo + per, n)
 
 
+def _extra(extra_params):
+    """EXTRA_PARAMS with the caller's entries on top."""
+    return {**EXTRA_PARAMS, **(extra_params or {})}
+
+
 def train_step(model, rays, rgbs, flat_grads, global_rays=None, chunk=8192, optimizer=None, return_stats=False,
-               _exchange=True):
+               _exchange=True, extra_params=None, _window=None):
     """One data-parallel training step on this rank's ray rows (B,9) / target colours (B,3).
     Returns the local contribution to the global-mean loss (sum over ranks = the reference's loss); with
     return_stats, training_step's log entries {'train/loss', 'train/psnr'} (train.py:147-163; psnr of the fine level
-    over this rank's rays, metrics.py:4-13) as device tensors."""
+    over this rank's rays, metrics.py:4-13) as device tensors.  extra_params: the forward's `extra_params`
+    ({'nerf_alpha', 'warp_alpha', 'hyper_alpha', 'hyper_sheet_alpha'}: the coarse-to-fine encoding windows; unset = none)."""
     B = rays.shape[0]
     global_rays = B if global_rays is None else global_rays
+    extra = _extra(extra_params)
     flat_grads.zero()
     total = torch.zeros((), device=rays.device, dtype=torch.float32)
     fine_sq = None
-    with model.packed_frozen():   # the weights do not change between the chunks of one step: pack the bf16 blobs once
+    # the weights do not change between the chunks of one step: pack the bf16 blobs once
+    with model.packed_frozen(extra, _window=_window):
         for i in range(0, B, chunk):
             rows = rays[i:i + chunk]
             tgt = rgbs[i:i + chunk]
-            out = model(model_utils.prepare_ray_dict(rows), dict(EXTRA_PARAMS))
+            out = model(model_utils.prepare_ray_dict(rows), dict(extra))
             # mean over the global batch: (sum_sq(coarse) + sum_sq(fine)) / (3 * global_rays), one fused kernel that
             # also seeds both levels' gradients (losses.py:9-14)
             loss, sums = losses.mse_coarse_fine(out, tgt, global_count=3.0 * global_rays)
@@ -157,20 +165,27 @@ class GraphedTrainStep:
 
         step = GraphedTrainStep(model, flat_grads, n_rays, global_rays, chunk)
         loss = step(rays, rgbs, optimizer)          # first call captures; the result lives in a static buffer that the
-                                                    # next call overwrites (a dict of such with return_stats=True)"""
+                                                    # next call overwrites (a dict of such with return_stats=True)
 
-    def __init__(self, model, flat_grads, n_rays, global_rays=None, chunk=8192, return_stats=False):
+    windowed=True captures the windowed weight packing / weight gradient (coarse-to-fine encoding windows) over a persistent
+    4-float device buffer of alphas; `step(rays, rgbs, optimizer, extra_params)` writes it before the replay (no host
+    synchronisation, no new capture), so a schedule changes the alphas every step.  Unset alphas mean no window."""
+
+    def __init__(self, model, flat_grads, n_rays, global_rays=None, chunk=8192, return_stats=False, windowed=False):
         dev = flat_grads.flat.device
         self.model, self.fg = model, flat_grads
         self.global_rays = n_rays if global_rays is None else global_rays
         self.chunk, self.return_stats = chunk, return_stats
         self.rays = torch.zeros(n_rays, 9, device=dev, dtype=torch.float32)
         self.rgbs = torch.zeros(n_rays, 3, device=dev, dtype=torch.float32)
+        self.windowed = windowed
+        self.alphas = torch.full((4,), float('inf'), device=dev, dtype=torch.float32) if windowed else None
         self.graph, self.loss, self.launches = None, None, 0
 
     def _local(self):
+        window = _packing._DeviceWindow(self.alphas) if self.windowed else None
         return train_step(self.model, self.rays, self.rgbs, self.fg, global_rays=self.global_rays, chunk=self.chunk,
-                          return_stats=self.return_stats, _exchange=False)
+                          return_stats=self.return_stats, _exchange=False, _window=window)
 
     def _capture(self):
         side = torch.cuda.Stream()
@@ -186,7 +201,16 @@ class GraphedTrainStep:
             self.loss = self._local()
         self.graph, self.launches = graph, _lib.launches - before
 
-    def __call__(self, rays, rgbs, optimizer=None):
+    def __call__(self, rays, rgbs, optimizer=None, extra_params=None):
+        window = _packing.pe_alphas(extra_params)
+        if self.windowed:
+            # from pinned memory: an asynchronous copy ordered before the replay (the caching host allocator keeps the
+            # staging block alive until the copy has run)
+            vals = window if window is not None else (float('inf'),) * 4
+            self.alphas.copy_(torch.tensor(vals, dtype=torch.float32).pin_memory(), non_blocking=True)
+        elif window is not None:
+            raise ValueError("this GraphedTrainStep was captured without encoding windows: build it with windowed=True "
+                             "to pass extra_params alphas")
         self.rays.copy_(rays, non_blocking=True)
         self.rgbs.copy_(rgbs, non_blocking=True)
         if self.graph is None:
@@ -279,7 +303,7 @@ def save_ckpt(model, path, epoch=0, global_step=0, optimizer=None, module_name='
 
 
 def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=0.0, decay_step=(20,), decay_gamma=0.1,
-        chunk=8192, seed=0, ckpt_path=None, log_every=0, cuda_graph=False):
+        chunk=8192, seed=0, ckpt_path=None, log_every=0, cuda_graph=False, extra_params=None):
     """Minimal stand-in for `Trainer.fit(NeRFSystem)` (train.py:35-233) on a ray pool that is already on the device:
     per epoch one shuffled pass over (rays (P,9), rgbs (P,3)) in batches of `batch_size` (train_dataloader,
     train.py:133-138: shuffle=True; the last short batch is kept, as DataLoader's drop_last=False does), each batch
@@ -287,7 +311,9 @@ def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=
     (get_scheduler 'steplr', utils/__init__.py:43-47; opt.py:62-75 defaults).  Under torch.distributed every rank
     passes its own shard of the pool (SURVEY.md §8(e)); gradients are all-reduced inside train_step.
     cuda_graph: replay the full-size batches from one CUDA graph (GraphedTrainStep); the last short batch of an epoch runs
-    eagerly.  Returns a list of per-step dicts {'epoch', 'step', 'lr', 'train/loss', 'train/psnr'} (training_step's log)."""
+    eagerly.  extra_params: the forward's encoding-window alphas (train_step), a dict or a callable step -> dict (a
+    coarse-to-fine schedule; `step` counts from 0).  Returns a list of per-step dicts {'epoch', 'step', 'lr', 'train/loss',
+    'train/psnr'} (training_step's log)."""
     distributed = dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
     fg = FlatGrads(model.parameters())
     model.attach_flat_grads(fg)
@@ -313,13 +339,15 @@ def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=
             r, t = rays[idx], rgbs[idx]
             # every rank holds P rows and the same batch boundaries, so the global batch is world * local
             world = dist.get_world_size() if distributed else 1
+            extra = extra_params(step) if callable(extra_params) else extra_params
             if cuda_graph and r.shape[0] == batch_size:
                 if graphed is None:
-                    graphed = GraphedTrainStep(model, fg, batch_size, world * batch_size, chunk, return_stats=True)
-                stats = {k: v.clone() for k, v in graphed(r, t, opt).items()}
+                    graphed = GraphedTrainStep(model, fg, batch_size, world * batch_size, chunk, return_stats=True,
+                                               windowed=extra_params is not None)
+                stats = {k: v.clone() for k, v in graphed(r, t, opt, extra).items()}
             else:
                 stats = train_step(model, r, t, fg, global_rays=world * r.shape[0], chunk=chunk, optimizer=opt,
-                                   return_stats=True)
+                                   return_stats=True, extra_params=extra)
             step += 1
             log.append({'epoch': epoch, 'step': step, 'lr': opt.param_groups[0]['lr'], **stats})
             if log_every and step % log_every == 0:
@@ -330,13 +358,15 @@ def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=
 
 
 @torch.no_grad()
-def render_rays(model, rays, chunk=32768, keys=('rgb', 'depth')):
+def render_rays(model, rays, chunk=32768, keys=('rgb', 'depth'), extra_params=None):
     """Chunked inference (eval.py:77-103 `batched_inference`), keeping only the per-ray outputs in `keys` of the
-    fine level instead of concatenating every per-sample tensor (SURVEY.md §8(f) row 3)."""
+    fine level instead of concatenating every per-sample tensor (SURVEY.md §8(f) row 3).  extra_params: as in
+    train_step."""
     outs = {k: [] for k in keys}
-    with model.packed_frozen():
+    extra = _extra(extra_params)
+    with model.packed_frozen(extra):
         for i in range(0, rays.shape[0], chunk):
-            out = model(model_utils.prepare_ray_dict(rays[i:i + chunk]), dict(EXTRA_PARAMS))
+            out = model(model_utils.prepare_ray_dict(rays[i:i + chunk]), dict(extra))
             for k in keys:
                 outs[k].append(out['fine'][k])
     return {k: torch.cat(v, 0) for k, v in outs.items()}

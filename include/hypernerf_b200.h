@@ -208,6 +208,31 @@ int hn_mlp_bwd_trunk_data(const hn_model_desc* desc, const void* packed, const i
 int hn_mlp_bwd_trunk_weights(const hn_model_desc* desc, const void* saved, int64_t B, int S, int level,
                              const int64_t* grad_offsets /* host */, float* flat_grad, const void* workspace, void* stream);
 
+/* Annealed positional encodings (the Nerfies / HyperNeRF coarse-to-fine window).  Band k of an encoder with bands
+ * 0..F-1 is scaled by w_k(alpha) = 0.5 (1 - cos(pi clamp(alpha - k, 0, 1))); identity, GLO, view-direction columns, biases
+ * and padding never are.  A window on an encoded input is a per-column scale of the weights that read it,
+ * W (w . pe) = (W diag(w)) pe, so:
+ *   hn_pack_weights_windowed           packs W diag(w) into the forward AND the transposed (data-gradient) images;
+ *   hn_mlp_bwd_weights_windowed /      the weight gradient of such a blob: the stash holds the unwindowed encoding, so the
+ *   hn_mlp_bwd_trunk_weights_windowed  accumulated dY^T pe is scaled by w on its way to flat_grad (bias sums unchanged).
+ * A windowed blob must be paired with the windowed weight-gradient entries, with the same pe_alpha values.
+ * pe_alpha: DEVICE array of 4 floats {warp_alpha, hyper_sheet_alpha, nerf_alpha, hyper_alpha}, read by the kernels (a CUDA
+ * graph replays with new values without a new capture); +inf (or any alpha >= F) = no window.  Encoders:
+ *   warp_alpha         posenc_orig(points, 10) of the TranslationField (bands of 6 columns after the 3 identity columns),
+ *                      posenc(points, 0, 8) of the SE3Field (48 columns, bands of 6)
+ *   hyper_sheet_alpha  posenc_orig(points, 7) of the HyperSheetMLP
+ *   nerf_alpha         posenc_orig(warped xyz, xyz_freqs) of both levels' trunks
+ *   hyper_alpha        posenc_orig(hyper point, hyper_freqs) of both levels' trunks (bands of 2H columns after H identity)
+ * An alpha whose encoder the configuration does not have is not read.  The static NeRF has no window (-13). */
+int hn_pack_weights_windowed(const hn_model_desc* desc, const float* flat_params, const int64_t* param_offsets /* host */,
+                             int level, void* packed, const float* pe_alpha, void* stream);
+int hn_mlp_bwd_weights_windowed(const hn_model_desc* desc, const void* saved, int64_t B, int S, int level,
+                                const int64_t* grad_offsets /* host */, float* flat_grad, const void* workspace,
+                                const float* pe_alpha, void* stream);
+int hn_mlp_bwd_trunk_weights_windowed(const hn_model_desc* desc, const void* saved, int64_t B, int S, int level,
+                                      const int64_t* grad_offsets /* host */, float* flat_grad, const void* workspace,
+                                      const float* pe_alpha, void* stream);
+
 /* losses.py:9-14 (MSELoss: mean-MSE of coarse.rgb + fine.rgb against the target colours) fused with its gradient seed and
  * with the fine-level MSE of metrics.py:4-13 (psnr = -10 log10(mse)).  sums[0] += sum (coarse - t)^2, sums[1] += sum
  * (fine - t)^2 (caller zeroes `sums`); g_level (B,3) = 2 (pred - t) * grad_scale, grad_scale = upstream / (3 B_global).
