@@ -27,6 +27,7 @@ EXPORTS = [
     "hn_abi_version", "hn_last_error", "hn_query", "hn_pack_weights", "hn_sample_coarse", "hn_sample_pdf", "hn_sample_pdf_ranks",
     "hn_composite_fwd", "hn_composite_bwd", "hn_filter_sigma", "hn_mse_loss", "hn_make_ndc_rays", "hn_adam_step", "hn_mlp_fwd", "hn_mlp_bwd", "hn_mlp_bwd_data", "hn_mlp_bwd_weights", "hn_mlp_fwd_trunk", "hn_mlp_bwd_trunk", "hn_mlp_bwd_trunk_data", "hn_mlp_bwd_trunk_weights",
     "hn_pack_weights_windowed", "hn_mlp_bwd_weights_windowed", "hn_mlp_bwd_trunk_weights_windowed",
+    "hn_mlp_fwd_warp", "hn_mlp_bwd_warp_data", "hn_mlp_bwd_warp_weights", "hn_background_loss",
 ]
 # microbenchmarks / descriptor probes: their own library and header (include/hypernerf_b200_probe.h), not the product ABI
 PROBE_LIB_PATH = os.path.join(_HERE, "libhypernerf_b200_probe.so")
@@ -42,7 +43,8 @@ class ModelDesc(C.Structure):
 
 class Sizes(C.Structure):
     _fields_ = [("packed_bytes", C.c_int64), ("saved_bytes", C.c_int64), ("workspace_bytes", C.c_int64),
-                ("flat_param_floats", C.c_int64), ("reserved", C.c_int64 * 4)]
+                ("flat_param_floats", C.c_int64), ("warp_saved_bytes", C.c_int64), ("warp_workspace_bytes", C.c_int64),
+                ("reserved", C.c_int64 * 2)]
 
 
 class NativeLibraryError(RuntimeError):
@@ -100,6 +102,11 @@ def lib():
     L.hn_pack_weights_windowed.argtypes = [C.POINTER(ModelDesc), vp, C.POINTER(C.c_int64), i32, vp, vp, vp]
     L.hn_mlp_bwd_weights_windowed.argtypes = [C.POINTER(ModelDesc), vp, i64, i32, i32, C.POINTER(C.c_int64), vp, vp, vp, vp]
     L.hn_mlp_bwd_trunk_weights_windowed.argtypes = L.hn_mlp_bwd_weights_windowed.argtypes
+    L.hn_mlp_fwd_warp.argtypes = [C.POINTER(ModelDesc), vp, vp, vp, i64, i32, vp, vp, vp, vp]
+    L.hn_mlp_bwd_warp_data.argtypes = [C.POINTER(ModelDesc), vp, vp, vp, vp, i64, i32, C.POINTER(C.c_int64), vp, vp, vp, vp,
+                                       vp]
+    L.hn_mlp_bwd_warp_weights.argtypes = [C.POINTER(ModelDesc), vp, i64, i32, C.POINTER(C.c_int64), vp, vp, vp, vp]
+    L.hn_background_loss.argtypes = [vp, vp, i64, i32, f32, f32, f32, vp, vp, vp]
     if hasattr(L, "hn_debug_set_timing_buffer"):   # role-timing builds only (make timing; HN_LIB selects them)
         L.hn_debug_set_timing_buffer.argtypes = [vp]
         L.hn_debug_set_timing_buffer.restype = C.c_int

@@ -19,6 +19,7 @@
 #include <math.h>
 #include <algorithm>
 #include <string.h>
+#include <string>
 #include <type_traits>
 #include <unordered_map>
 #include "hn_api_internal.h"
@@ -27,9 +28,9 @@
 
 // This file is compiled twice into libhypernerf_b200.so (Makefile).  The second compilation (hn_mlp_fv.o:
 // -DHN_MLP_FWD_VARIANT=1) holds the INFERENCE forward kernels with two epilogue warpgroups per sub-tile (hn_mlp_program.h:
-// kEpiSplit), in their own namespace, and exports only hn_mlp_fwd_fv / hn_mlp_fwd_trunk_fv, which the first compilation's
-// hn_mlp_fwd / hn_mlp_fwd_trunk call for every launch without a stash.  Measured per 1 M samples in isolation: inference
-// forward 2.03 -> 1.93 ms, training forward 2.50 -> 2.42 ms, data gradient +2 %; a full-frame render goes from 2.27 to
+// kEpiSplit), in their own namespace, and exports only hn_mlp_fwd_fv / hn_mlp_fwd_trunk_fv / hn_mlp_fwd_warp_fv, which the
+// first compilation's hn_mlp_fwd / hn_mlp_fwd_trunk / hn_mlp_fwd_warp call for every launch without a stash.  Measured
+// per 1 M samples in isolation: inference forward 2.03 -> 1.93 ms, training forward 2.50 -> 2.42 ms, data gradient +2 %; a full-frame render goes from 2.27 to
 // 2.40 Mrays/s, while inside the power-capped training step the split training forward is a wash (690 k against 691 k
 // rays/s over three alternating runs, the trunk-only launch 3 % slower), so training keeps the single-warpgroup kernels.
 // The stash / gate-word layout does not depend on the epilogue split.
@@ -38,6 +39,7 @@ namespace hn_fv { using namespace hn; }
 #define hn hn_fv
 #define hn_mlp_fwd hn_mlp_fwd_fv
 #define hn_mlp_fwd_trunk hn_mlp_fwd_trunk_fv
+#define hn_mlp_fwd_warp hn_mlp_fwd_warp_fv
 #define HN_FV_HIDDEN __attribute__((visibility("hidden")))
 #else
 #define HN_FV_HIDDEN
@@ -900,10 +902,13 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
 #pragma unroll
             for (int i = 0; i < C::NWARPED; ++i) p.warped[gq * C::NWARPED + i] = wp[i];
           }
-          store_trunk_input<C>(wp, act_row, inb_row, save_row, L.save_chunk);
-          if constexpr (C::TIN_ACT) {
+          // a warp-stage-only program ends here: no trunk input (its stash has no slab for it)
+          if (!(prog.flags & PF_WARP_ONLY)) {
+            store_trunk_input<C>(wp, act_row, inb_row, save_row, L.save_chunk);
+            if constexpr (C::TIN_ACT) {
 #pragma unroll
-            for (int i = 0; i < C::NWARPED; ++i) wp_keep[i] = wp[i];
+              for (int i = 0; i < C::NWARPED; ++i) wp_keep[i] = wp[i];
+            }
           }
           }
         } else if (L.epi == FE_SKIPFEED) {
@@ -1045,6 +1050,30 @@ __device__ __forceinline__ void trunk_in_bwd(uint32_t tlane, const float* wp, fl
   }
 }
 
+// d(warped point, hyper coordinates) of one row in f[0, 3 + H) -> the warp / sheet head's pre-activation gradient in f[0, 16)
+template <class C>
+__device__ __forceinline__ void wshead_dy(const BwdParams& p, float* f, bool valid, int64_t ray, int64_t gq, int64_t gc, int lane) {
+  if constexpr (C::H == C::G) {
+    if (p.mflags & MF_AXIS) {
+      // axis-aligned slicing: the hyper coordinates ARE the GLO vector (models.py:533-534), their gradient
+      // goes to the table; the (absent) sheet head receives nothing
+      const int64_t id = __ldg(p.ids + ray);
+      glo_grad_add<C::G>(f + 3, valid, id, p.glo_grad, lane);
+#pragma unroll
+      for (int i = 0; i < C::G; ++i) f[3 + i] = 0.f;
+    }
+  }
+  if constexpr (C::SE3) {
+    // d(warped xyz) -> d(w, v) through the exp map; columns 0..2 / 3..5 of the head's pre-activation gradient
+    float x[3], wv[6], gy[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) { x[i] = __ldg(p.points + gq * 3 + i); gy[i] = f[i]; }
+#pragma unroll
+    for (int i = 0; i < 6; ++i) wv[i] = __ldg(p.aux + gc * 6 + i);
+    se3_apply_bwd(x, wv, wv + 3, gy, f, f + 3);
+  }
+}
+
 // ======================================================================================================
 // backward-data
 // ======================================================================================================
@@ -1136,8 +1165,22 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_dgrad_kernel(const __grid_
       const uint32_t* gate_row = p.gates + half * (size_t)p.g_total * kHalfRows + (row & 63);
       uint4* save_row = reinterpret_cast<uint4*>(p.dsaved + half * (size_t)p.d_total * kHalfChunkBytes) + (row & 63);
 
+      if constexpr (PRIMARY && !C::STATIC && !C::NOWARP) {
+        if (prog.flags & PF_WARP_ONLY) {
+          // warp-stage-only program: dY of the warp / sheet head from the upstream gradient of `warped` (launch rows)
+          float f[16];
+#pragma unroll
+          for (int i = 0; i < 16; ++i) f[i] = 0.f;
+          if (valid) {
+#pragma unroll
+            for (int i = 0; i < C::NWARPED; ++i) f[i] = __ldg(p.g_warped + gc * C::NWARPED + i);
+          }
+          wshead_dy<C>(p, f, valid, ray, gq, gc, lane);
+          store_features<16>(f, act_row, save_row, p.d_rgbhead);
+        }
+      }
       // prologue: dY of the rgb head = g_rgb * y (1 - y) (Sigmoid, models.py:164)
-      if constexpr (PRIMARY) {
+      if (PRIMARY && !(prog.flags & PF_WARP_ONLY)) {
         float f[16];
 #pragma unroll
         for (int i = 0; i < 16; ++i) f[i] = 0.f;
@@ -1243,25 +1286,7 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_dgrad_kernel(const __grid_
               if (p.g_warped != nullptr) f[i] += __ldg(p.g_warped + gq * C::NWARPED + i);
             }
           }
-          if constexpr (C::H == C::G) {
-            if (p.mflags & MF_AXIS) {
-              // axis-aligned slicing: the hyper coordinates ARE the GLO vector (models.py:533-534), their gradient
-              // goes to the table; the (absent) sheet head receives nothing
-              const int64_t id = __ldg(p.ids + ray);
-              glo_grad_add<C::G>(f + 3, valid, id, p.glo_grad, lane);
-#pragma unroll
-              for (int i = 0; i < C::G; ++i) f[3 + i] = 0.f;
-            }
-          }
-          if constexpr (C::SE3) {
-            // d(warped xyz) -> d(w, v) through the exp map; columns 0..2 / 3..5 of the head's pre-activation gradient
-            float x[3], wv[6], gy[3];
-#pragma unroll
-            for (int i = 0; i < 3; ++i) { x[i] = __ldg(p.points + gq * 3 + i); gy[i] = f[i]; }
-#pragma unroll
-            for (int i = 0; i < 6; ++i) wv[i] = __ldg(p.aux + gc * 6 + i);
-            se3_apply_bwd(x, wv, wv + 3, gy, f, f + 3);
-          }
+          wshead_dy<C>(p, f, valid, ray, gq, gc, lane);
           store_features<16>(f, act_row, save_row, L.save_chunk);
           }
         } else if constexpr (!C::NOWARP) {  // BE_GLO: d(GLO embedding) of this sample -> per-ray reduction -> atomics on the table gradient
@@ -1708,6 +1733,9 @@ extern "C" int hn_query(const hn_model_desc* desc, int64_t n_samples, hn_sizes* 
   // X slabs, then the ReLU gate words ([half tile][g_total][64 rows] uint32)
   out->saved_bytes = halves * plan.info.x_total * kHalfChunkBytes + halves * plan.info.g_total * kHalfRows * 4;
   out->workspace_bytes = halves * plan.info.d_total * kHalfChunkBytes;
+  // the warp-stage-only launches (hn_mlp_fwd_warp / hn_mlp_bwd_warp_*) stash the slab-map prefixes alone
+  out->warp_saved_bytes = halves * plan.info.x_warp * kHalfChunkBytes + halves * plan.info.g_warp * kHalfRows * 4;
+  out->warp_workspace_bytes = halves * plan.info.d_warp * kHalfChunkBytes;
   const Dims& m = plan.dims;
   auto lin = [](int64_t out_f, int64_t in_f) { return out_f * in_f + out_f; };
   if (is_static(*desc)) {   // NeRF(D=8, W=256): 595 844 parameters at the default 63 / 27 input channels
@@ -1879,6 +1907,59 @@ extern "C" HN_FV_HIDDEN int hn_mlp_fwd_trunk(const hn_model_desc* desc, const vo
                       saved, nullptr, stream);
 }
 
+#if defined(HN_MLP_FV_LINKED) && !defined(HN_MLP_FWD_VARIANT)
+extern "C" int hn_mlp_fwd_warp_fv(const hn_model_desc*, const void*, const float*, const int64_t*, int64_t, int, float*, void*,
+                                  float*, void*);
+#endif
+
+// checks shared by the warp-stage-only entry points: a hyper model with a warp stage, a positive sample count
+static int check_warp_only(const hn_model_desc* desc, int64_t B, int S, const char* what) {
+  if (is_static(*desc)) return set_error(-13, (std::string(what) + ": the static NeRF has no warp stage").c_str());
+  if (!has_warp(*desc)) return set_error(-13, (std::string(what) + ": this model has no warp field (use_warp=False)").c_str());
+  if (B <= 0 || S <= 0) return set_error(-1, (std::string(what) + ": B and S must be positive").c_str());
+  return validate_desc(*desc);
+}
+
+extern "C" HN_FV_HIDDEN int hn_mlp_fwd_warp(const hn_model_desc* desc, const void* packed, const float* points, const int64_t* ids,
+                                            int64_t B, int S, float* warped, void* saved, float* aux, void* stream) {
+  HN_MLP_FV_CALL(hn_mlp_fwd_warp_fv, desc, packed, points, ids, B, S, warped, saved, aux, stream);
+  if (!desc || !packed || !points || !ids || !warped) return set_error(-2, "hn_mlp_fwd_warp: null pointer");
+  if (int rc = check_warp_only(desc, B, S, "hn_mlp_fwd_warp")) return rc;
+  if ((desc->flags & HN_FLAG_WARP_SE3) && saved != nullptr && !aux)
+    return set_error(-2, "hn_mlp_fwd_warp: the SE3 warp needs the aux buffer when the stash is written");
+  const ModelPlan& plan = cached_plan(*desc);
+  const bool train = saved != nullptr;
+  FwdParams fp;
+  memset(&fp, 0, sizeof(fp));
+  fp.prog = train ? plan.fwd_warp_train : plan.fwd_warp;
+  fp.weights = (const uint8_t*)packed + plan.layout.fwd_off;
+  fp.bias = (const float*)((const uint8_t*)packed + plan.layout.bias_off);
+  fp.glo = (const float*)((const uint8_t*)packed + plan.layout.glo_off);
+  fp.points = points; fp.ids = ids;
+  fp.n = B * S; fp.S = S; fp.n_embed = desc->num_embeddings;
+  fp.view_freqs = desc->view_freqs; fp.mflags = model_flags(*desc);
+  fp.S_full = S;
+  const int64_t nt = tiles_of(fp.n);
+  if (nt > 0x7fffffff) return set_error(-1, "hn_mlp_fwd_warp: too many samples");
+  fp.n_tiles = (int)nt;
+  // the warp-only stash: slab-map prefixes as the per-half-tile strides (PlanInfo::x_warp / g_warp)
+  fp.x_total = plan.info.x_warp;
+  fp.x_in_ws = plan.info.x_in0; fp.x_in_t = kNone; fp.x_in_v = kNone;
+  fp.warped = warped; fp.saved = (uint8_t*)saved; fp.aux = aux;
+  fp.g_total = plan.info.g_warp;
+  fp.gates = train ? (uint32_t*)((uint8_t*)saved + (size_t)(2 * kSubTiles) * nt * plan.info.x_warp * kHalfChunkBytes) : nullptr;
+  fp.dbg = g_dbg;
+  const int grid = (int)std::min<int64_t>(nt, num_sms());
+#ifdef HN_MLP_FWD_VARIANT
+#define HN_LAUNCH_FWD(CFG) return launch_fwd<CFG, false>(fp, grid, stream)
+#else
+#define HN_LAUNCH_FWD(CFG) return train ? launch_fwd<CFG, true>(fp, grid, stream) : launch_fwd<CFG, false>(fp, grid, stream)
+#endif
+  HN_DISPATCH_SHAPE(shape_of(*desc), HN_LAUNCH_FWD)
+#undef HN_LAUNCH_FWD
+  return set_error(-1, "hn_mlp_fwd_warp: unreachable");
+}
+
 #ifndef HN_MLP_FWD_VARIANT
 static int mlp_bwd_impl(const hn_model_desc* desc, const void* packed, const int64_t* ids, const float* sigma,
                         const float* rgb, const float* warped, const void* saved, const float* g_sigma, const float* g_rgb,
@@ -2028,6 +2109,84 @@ extern "C" int hn_mlp_bwd_trunk_weights_windowed(const hn_model_desc* desc, cons
   return mlp_bwd_impl(desc, nullptr, nullptr, nullptr, nullptr, nullptr, saved, nullptr, nullptr, nullptr, B, S, nullptr, 0,
                       level, param_offsets, flat_grad, (void*)workspace, stream, false, true, true, nullptr, nullptr, nullptr,
                       pe_alpha);
+}
+
+// Warp-stage-only backward (level-0 blob, hn_mlp_fwd_warp's stash): data gradient from g_warped, then / or the weight
+// gradient of the warp / sheet jobs.
+static int mlp_bwd_warp_impl(const hn_model_desc* desc, const void* packed, const int64_t* ids, const void* saved,
+                             const float* g_warped, int64_t B, int S, const int64_t* param_offsets, float* flat_grad,
+                             void* workspace, const float* points, const float* aux, const float* pe_alpha, bool do_data,
+                             bool do_weights, void* stream, const char* what) {
+  if (!desc || !saved || !param_offsets || !flat_grad || !workspace) return set_error(-2, (std::string(what) + ": null pointer").c_str());
+  if (do_data && (!packed || !ids || !g_warped)) return set_error(-2, (std::string(what) + ": null pointer").c_str());
+  if (int rc = check_warp_only(desc, B, S, what)) return rc;
+  if (do_data && (desc->flags & HN_FLAG_WARP_SE3) && (!points || !aux))
+    return set_error(-2, (std::string(what) + ": the SE3 warp needs the sample points and the forward's aux buffer").c_str());
+  const ModelPlan& plan = cached_plan(*desc, 0, do_weights ? param_offsets : nullptr, pe_alpha != nullptr);
+  const int64_t n = B * S;
+  const int64_t nt = tiles_of(n);
+  if (nt > 0x7fffffff) return set_error(-1, (std::string(what) + ": too many samples").c_str());
+  if (do_data) {
+    BwdParams bp;
+    memset(&bp, 0, sizeof(bp));
+    bp.prog = plan.bwd_warp;
+    bp.weights = (const uint8_t*)packed + plan.layout.bwd_off;
+    bp.ids = ids; bp.g_warped = g_warped;
+    bp.points = points; bp.aux = aux;
+    bp.saved = (const uint8_t*)saved; bp.dsaved = (uint8_t*)workspace;
+    bp.g_total = plan.info.g_warp;
+    bp.gates = (const uint32_t*)((const uint8_t*)saved + (size_t)(2 * kSubTiles) * nt * plan.info.x_warp * kHalfChunkBytes);
+    if (param_offsets[plan.info.glo_param] < 0) return set_error(-2, (std::string(what) + ": the GLO table has no gradient offset").c_str());
+    bp.glo_grad = flat_grad + param_offsets[plan.info.glo_param];
+    bp.mflags = model_flags(*desc);
+    bp.S_full = S;
+    bp.n = n; bp.S = S; bp.n_embed = desc->num_embeddings;
+    bp.n_tiles = (int)nt;
+    bp.x_total = plan.info.x_warp; bp.d_total = plan.info.d_warp;
+    bp.d_rgbhead = plan.slabs.d_wshead;   // the dY slab the PF_WARP_ONLY prologue writes
+    bp.d_sigma = kNone;
+    bp.dbg = g_dbg;
+    const int grid = (int)std::min<int64_t>(nt, num_sms());
+#define HN_LAUNCH_BWD(CFG)                                                                                                  \
+  do {                                                                                                                      \
+    if (int rc = set_smem(mlp_dgrad_kernel<CFG>, SmemBwd<CFG>::TOTAL, what)) return rc;                                     \
+    if (int rc = set_cuda_error(launch_mlp(mlp_dgrad_kernel<CFG>, grid, SmemBwd<CFG>::TOTAL, (cudaStream_t)stream, bp), what)) \
+      return rc;                                                                                                            \
+  } while (0)
+    HN_DISPATCH_SHAPE(shape_of(*desc), HN_LAUNCH_BWD)
+#undef HN_LAUNCH_BWD
+  }
+  if (do_weights) {
+    WgradParams wp;
+    wp.tab = plan.wgrad_warp;
+    wp.saved = (const uint8_t*)saved; wp.dsaved = (const uint8_t*)workspace;
+    wp.pe_alpha = pe_alpha;
+    wp.flat_grad = flat_grad;
+    wp.n_half = 2 * kSubTiles * nt;
+    wp.x_total = plan.info.x_warp; wp.d_total = plan.info.d_warp;
+    const auto wgrad_kernel = pe_alpha != nullptr ? mlp_wgrad_kernel<true> : mlp_wgrad_kernel<false>;
+    if (int rc = set_smem(wgrad_kernel, WgSmem::TOTAL, what)) return rc;
+    const int wgrid = (int)std::min<int64_t>(wp.n_half, num_sms());
+    wp.groups = wp.n_half >= 8 * (int64_t)wgrid ? std::min(wgrad_groups(wp.tab.njobs), wgrid) : 1;
+    assign_wgrad_groups(wp.tab, wp.groups, wgrid, wp.group_start);
+    wgrad_kernel<<<wgrid, 192, WgSmem::TOTAL, (cudaStream_t)stream>>>(wp);
+    if (int rc = set_cuda_error(cudaGetLastError(), what)) return rc;
+  }
+  return 0;
+}
+
+extern "C" int hn_mlp_bwd_warp_data(const hn_model_desc* desc, const void* packed, const int64_t* ids, const void* saved,
+                                    const float* g_warped, int64_t B, int S, const int64_t* grad_offsets, float* flat_grad,
+                                    void* workspace, const float* points, const float* aux, void* stream) {
+  return mlp_bwd_warp_impl(desc, packed, ids, saved, g_warped, B, S, grad_offsets, flat_grad, workspace, points, aux, nullptr,
+                           true, false, stream, "hn_mlp_bwd_warp_data");
+}
+
+extern "C" int hn_mlp_bwd_warp_weights(const hn_model_desc* desc, const void* saved, int64_t B, int S,
+                                       const int64_t* grad_offsets, float* flat_grad, const void* workspace,
+                                       const float* pe_alpha, void* stream) {
+  return mlp_bwd_warp_impl(desc, nullptr, nullptr, saved, nullptr, B, S, grad_offsets, flat_grad, (void*)workspace, nullptr,
+                           nullptr, pe_alpha, false, true, stream, "hn_mlp_bwd_warp_weights");
 }
 
 #if HN_ROLE_TIMING

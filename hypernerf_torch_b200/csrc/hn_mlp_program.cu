@@ -298,6 +298,13 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
     // trunk-only: everything after the warp / sheet head (without warp that is the whole program)
     slice_program(plan->fwd, n_ws_layers, plan->fwd.nlayers, &plan->fwd_trunk);
     slice_program(plan->fwd_train, n_ws_layers, plan->fwd_train.nlayers, &plan->fwd_trunk_train);
+    // warp-stage-only: the complementary slice, up to and including the warp / sheet head
+    if (!m.nowarp) {
+      slice_program(plan->fwd, 0, n_ws_layers, &plan->fwd_warp);
+      slice_program(plan->fwd_train, 0, n_ws_layers, &plan->fwd_warp_train);
+      plan->fwd_warp.flags |= PF_WARP_ONLY;
+      plan->fwd_warp_train.flags |= PF_WARP_ONLY;
+    }
   }
   // ------------------------------------------------------------------ backward-data program
   {
@@ -363,6 +370,11 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
     plan->layout.bias_off = plan->layout.bwd_off + (int64_t)b.w16 * 16;
     // trunk-only: up to and including the trunk-input layer (BE_TRUNKIN), whose epilogue then emits d(warped point)
     slice_program(plan->bwd, 0, n_trunk_layers, &plan->bwd_trunk);
+    // warp-stage-only: from the head^T layer on (the prologue seeds its A operand from g_warped)
+    if (!m.nowarp) {
+      slice_program(plan->bwd, n_trunk_layers, plan->bwd.nlayers, &plan->bwd_warp);
+      plan->bwd_warp.flags |= PF_WARP_ONLY;
+    }
   }
   PlanInfo& I = plan->info;
   I.glo_param = m.nowarp ? (cond ? P_COND_GLO : -1) : P_GLO;
@@ -374,6 +386,7 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
   I.x_total = s.x_total; I.d_total = s.d_total; I.g_total = s.g_total;
   I.x_in0 = s.x_in_ws; I.x_in_t = s.x_in_t; I.x_in_v = s.x_in_v;
   I.d_rgbhead = s.d_rgbhead; I.d_sigma = kNone;
+  if (!m.nowarp) { I.x_warp = s.x_in_t; I.d_warp = (uint16_t)(s.d_wshead + 2); I.g_warp = s.g_t[0]; }
   I.n_params = HN_NUM_PARAM_TENSORS;
 }
 
@@ -726,6 +739,10 @@ void build_tables(const hn_model_desc& d, int level, const int64_t* off, bool wi
   WgradTable& wt = plan->wgrad_trunk;
   memset(&wt, 0, sizeof(wt));
   for (int i = first_trunk_job; i < w.njobs; ++i) wt.jobs[wt.njobs++] = w.jobs[i];
+  // warp-stage-only job table: the warp / sheet jobs (their slabs lie inside the warp-only stash prefixes)
+  WgradTable& ww = plan->wgrad_warp;
+  memset(&ww, 0, sizeof(ww));
+  for (int i = 0; i < first_trunk_job; ++i) ww.jobs[ww.njobs++] = w.jobs[i];
   (void)d;
 }
 

@@ -221,7 +221,10 @@ struct LogicalOp {
 // FE_LINEAR: plain linear layer (bias, no activation, stashed): the SE3 trunk's logit layer.
 enum FwdEpi : uint8_t { FE_RELU = 0, FE_WSHEAD, FE_BOTT, FE_RGB0A, FE_RGBHEAD, FE_SIGMA, FE_SKIPFEED, FE_LINEAR };
 enum BwdEpi : uint8_t { BE_MASK = 0, BE_LINEAR, BE_RGB1, BE_SKIPSTORE, BE_TRUNKIN, BE_GLO, BE_LINCOND };
-enum ProgFlags : int32_t { PF_TIN_ACT = 1 };   // Program::flags
+// PF_WARP_ONLY: a warp-stage-only program (ModelPlan::fwd_warp*, bwd_warp).  Its forward ends at the FE_WSHEAD epilogue,
+// which then writes `warped` (and the SE3 screw) but no trunk input; its data gradient starts at the head^T layer, whose
+// A operand the prologue builds from the upstream g_warped instead of from the rgb head.
+enum ProgFlags : int32_t { PF_TIN_ACT = 1, PF_WARP_ONLY = 2 };   // Program::flags
 
 struct Layer {
   uint8_t op0, nops, epi, pad;
@@ -315,6 +318,9 @@ struct PlanInfo {
   uint16_t x_total, d_total, g_total;   // chunks per half tile of the X / dY stashes, gate words per row
   uint16_t x_in0, x_in_t, x_in_v;       // X slabs written by the prologue / trunk-input / view-direction PE
   uint16_t d_rgbhead, d_sigma;          // dY slabs written by the data-gradient prologue
+  // Warp-stage-only stash (ModelPlan::fwd_warp*): the X slabs, dY slabs and gate words of the warp / sheet stage are
+  // prefixes of their maps (make_slabs), so their prefix lengths serve as the per-half-tile strides; 0 without warp
+  uint16_t x_warp, d_warp, g_warp;
   int32_t n_params;                     // canonical parameter tensors
   int32_t glo_floats;
   int32_t glo_param;                    // canonical index of the GLO table the kernels read (copied into the blob); -1: none
@@ -338,6 +344,11 @@ struct ModelPlan {
   // are shared between the levels, so those rows' warp / sheet evaluations are the coarse pass's (hn_mlp_fwd_trunk).
   Program fwd_trunk, fwd_trunk_train, bwd_trunk;
   WgradTable wgrad_trunk;   // built per call next to `wgrad`
+  // Warp-stage-only programs (models with warp): the layers from the input encoding up to and including the FE_WSHEAD
+  // head, and their transposes, flagged PF_WARP_ONLY (hn_mlp_fwd_warp / hn_mlp_bwd_warp_*): `apply_warp` and the
+  // background loss need `warped` alone, not the template behind it.
+  Program fwd_warp, fwd_warp_train, bwd_warp;
+  WgradTable wgrad_warp;    // built per call next to `wgrad`
   LogicalOps fwd_logical, bwd_logical;
   PackTable pack;     // needs param_offsets -> built per call
   WgradTable wgrad;   // needs param_offsets -> built per call

@@ -1,3 +1,4 @@
+#include <float.h>
 // HBM-bound per-ray stages of the HyperNeRF hot path: stratified sampling, inverse-CDF resampling and
 // alpha compositing (forward + reverse).  One warp owns one ray; every lane owns C consecutive samples so
 // global loads are contiguous across the warp and scans are lane-local + one shuffle scan.
@@ -1273,6 +1274,57 @@ extern "C" int hn_mse_loss(const float* rgb_coarse, const float* rgb_fine, const
   const int blocks = (int)std::min<int64_t>((n + 255) / 256, 4 * (int64_t)hn::num_sms());
   hn::mse_loss_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(rgb_coarse, rgb_fine, targets, n, grad_scale, sums, g_coarse, g_fine);
   return hn::set_cuda_error(cudaGetLastError(), "hn_mse_loss");
+}
+
+
+// ------------------------------------------------------------------------------------------------------
+// hn_background_loss — compute_background_loss + general_loss_with_squared_residual of the JAX HyperNeRF
+// (hypernerf/training.py, utils.py; the torch port has no background loss): Barron's robust loss of the squared
+// displacement r^2 = |warped[:3] - points|^2 of known-static points, with its gradient seed.  One thread per point,
+// the loss warp-reduced into one atomic per warp.
+// ------------------------------------------------------------------------------------------------------
+namespace hn {
+__global__ void __launch_bounds__(256) background_loss_kernel(const float* __restrict__ y, const float* __restrict__ pts,
+                                                              int64_t n, int cols, float alpha, float inv_s2,
+                                                              float grad_scale, float* __restrict__ sums,
+                                                              float* __restrict__ g) {
+  const float eps = FLT_EPSILON;
+  const float b = fmaxf(eps, fabsf(alpha - 2.f));
+  const float a = (alpha >= 0.f ? 1.f : -1.f) * fmaxf(eps, fabsf(alpha));
+  float acc = 0.f;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    float d[3], r2 = 0.f;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      d[c] = __ldg(y + i * cols + c) - __ldg(pts + i * 3 + c);
+      r2 += d[c] * d[c];
+    }
+    // rho = (b / a) ((x + 1)^(a/2) - 1), x = r^2 / s^2 / b, through expm1 / log1p: no cancellation at small x
+    const float l = log1pf(r2 * inv_s2 / b);
+    acc += (b / a) * expm1f(0.5f * a * l);
+    if (g != nullptr) {
+      const float drho = 0.5f * inv_s2 * expf((0.5f * a - 1.f) * l);   // d rho / d r^2
+#pragma unroll
+      for (int c = 0; c < 3; ++c) g[i * cols + c] = grad_scale * drho * 2.f * d[c];
+      for (int c = 3; c < cols; ++c) g[i * cols + c] = 0.f;
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o);
+  if ((threadIdx.x & 31) == 0) atomicAdd(sums, acc);
+}
+}  // namespace hn
+
+extern "C" int hn_background_loss(const float* warped, const float* points, int64_t n, int warped_cols, float alpha, float scale,
+                                  float grad_scale, float* sums, float* g_warped, void* stream) {
+  if (!warped || !points || !sums) return hn::set_error(-2, "hn_background_loss: null pointer");
+  if (n <= 0) return hn::set_error(-1, "hn_background_loss: n must be positive");
+  if (warped_cols < 3) return hn::set_error(-1, "hn_background_loss: warped_cols must be >= 3");
+  if (!(scale > 0.f)) return hn::set_error(-1, "hn_background_loss: scale must be positive");
+  const int blocks = (int)std::min<int64_t>((n + 255) / 256, 4 * (int64_t)hn::num_sms());
+  hn::background_loss_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(warped, points, n, warped_cols, alpha,
+                                                                      1.f / (scale * scale), grad_scale, sums, g_warped);
+  return hn::set_cuda_error(cudaGetLastError(), "hn_background_loss");
 }
 
 

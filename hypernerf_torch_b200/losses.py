@@ -1,10 +1,13 @@
 """losses.py of the reference (MSELoss, loss_dict) on the B200 path: one fused kernel (hn_mse_loss) computes
-MSE(coarse.rgb) + MSE(fine.rgb), the gradient seed of both levels and the fine-level MSE that metrics.psnr needs."""
+MSE(coarse.rgb) + MSE(fine.rgb), the gradient seed of both levels and the fine-level MSE that metrics.psnr needs.
+`background_loss` adds HyperNeRF's robust background regularisation, which the torch port dropped."""
 import torch
 from torch import nn
 
 from . import _lib
 from ._lib import check, lib, ptr, stream
+from ._packing import pe_alphas
+from .models import NerfModel, _FusedWarp
 
 
 class _FusedMSE(torch.autograd.Function):
@@ -40,6 +43,57 @@ def mse_coarse_fine(inputs, targets, global_count=None):
     fine = inputs['fine']['rgb'] if 'fine' in inputs else None
     n = targets.numel() if global_count is None else global_count
     return _FusedMSE.apply(coarse, fine, targets, 1.0 / float(n))
+
+
+class _FusedBackground(torch.autograd.Function):
+    @staticmethod
+    @torch.amp.custom_fwd(device_type="cuda", cast_inputs=torch.float32)
+    def forward(ctx, warped, points, alpha, scale, grad_scale):
+        y = warped.contiguous()
+        p = points.contiguous()
+        sums = torch.zeros(1, device=y.device, dtype=torch.float32)
+        g = torch.empty_like(y) if ctx.needs_input_grad[0] else None
+        check(lib().hn_background_loss(ptr(y), ptr(p), p.shape[0], y.shape[-1], float(alpha), float(scale),
+                                       float(grad_scale), ptr(sums), ptr(g), stream()), "hn_background_loss")
+        _lib.count(1)
+        ctx.save_for_backward(g)
+        return sums[0] * grad_scale
+
+    @staticmethod
+    @torch.amp.custom_bwd(device_type="cuda")
+    def backward(ctx, g_loss):
+        g, = ctx.saved_tensors
+        return (None if g is None else g * g_loss), None, None, None, None
+
+
+def background_loss(model, points, extra_params=None, *, noise_std=1e-3, alpha=-2.0, scale=1e-3, weight=1.0,
+                    global_count=None):
+    """HyperNeRF's background regularisation (compute_background_loss of the JAX original, hypernerf/training.py; the
+    torch port has none): known-static points (P, 3), e.g. the scene's SfM points, are jittered with Gaussian noise, warped
+    with a random warp id each, and their squared displacement r^2 = |warped - jittered|^2 is penalised with Barron's robust
+    loss rho(r^2, alpha, scale) (general_loss_with_squared_residual; alpha = -2 is Geman-McClure).  Returns
+    weight * sum(rho) / (global_count or P); autograd reaches the warp field, the hyper sheet's GLO rows and the GLO table.
+    The warp stage runs alone (hn_mlp_fwd_warp) on the level-0 blob, with the encoding window of `extra_params`.
+
+    Random draws, in this order, on the points' device with the default generator (a test replays them):
+      1. ids = model.warp_embeds.to(dev)[torch.randint(len(model.warp_embeds), (P,), device=dev)]
+      2. noise = torch.randn(P, 3, device=dev) * noise_std
+    Raises ValueError for a model without warp (and for the static NeRF) and for points that are not (P, 3), P > 0."""
+    if not isinstance(model, NerfModel):
+        raise ValueError(f"background_loss needs a NerfModel with a warp field, got {type(model).__name__}")
+    if not model.use_warp:
+        raise ValueError("background_loss needs a model with a warp field (use_warp=True)")
+    if model._forward_error is not None:
+        raise RuntimeError(model._forward_error)
+    if points.dim() != 2 or points.shape[1] != 3 or points.shape[0] == 0:
+        raise ValueError(f"background points must be (P, 3) with P > 0, got {tuple(points.shape)}")
+    dev, P = points.device, points.shape[0]
+    ids = model.warp_embeds.to(dev)[torch.randint(len(model.warp_embeds), (P,), device=dev)]
+    noise = torch.randn(P, 3, device=dev) * noise_std
+    jittered = (points.detach().to(torch.float32) + noise).contiguous()
+    warped = _FusedWarp.apply(model, pe_alphas(extra_params), jittered[:, None, :], ids, *model._warp_params())
+    count = P if global_count is None else global_count
+    return _FusedBackground.apply(warped[:, 0, :], jittered, alpha, scale, float(weight) / float(count))
 
 
 class MSELoss(nn.Module):

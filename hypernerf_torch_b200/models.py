@@ -169,6 +169,73 @@ class _FusedMlp(torch.autograd.Function):
         return (None,) * 7 + tuple(_param_grads(ctx, model, level, flat_grad, offs, 7))
 
 
+class _FusedWarp(torch.autograd.Function):
+    """hn_mlp_fwd_warp / hn_mlp_bwd_warp_*: the warp stage alone (TranslationField + HyperSheetMLP, or the SE3Field) on
+    the level-0 blob, -> warped (B, S, 3 + H), bit-identical to _FusedMlp's `warped`.  Inputs after the fixed arguments are
+    the parameter tensors of the warp-stage slots (NerfModel._warp_slots); gradients come back as views of one flat fp32
+    buffer, or go straight into the attached train.FlatGrads.  The sample points take no gradient."""
+
+    @staticmethod
+    @torch.amp.custom_fwd(device_type="cuda", cast_inputs=torch.float32)
+    def forward(ctx, model, window, points, ids, *params):
+        B, S = points.shape[0], points.shape[1]
+        dev = points.device
+        desc = model._desc
+        packed, pe_alpha = model._packed_window(0, window)
+        pts = points.detach().to(torch.float32).contiguous()
+        ids = ids.reshape(-1).to(torch.int64).contiguous()
+        if ids.numel() != B:
+            raise ValueError(f"metadata ids must have one entry per ray, got {tuple(ids.shape)} for {B} rays")
+        warped = torch.empty(B, S, 3 + desc.hyper_dim, device=dev, dtype=torch.float32)
+        need_grad = any(ctx.needs_input_grad[4:])
+        saved = aux = None
+        if need_grad:
+            saved = torch.empty(model._sizes(B * S).warp_saved_bytes, device=dev, dtype=torch.uint8)
+            if model._se3:   # the screw parameters (w, v) of every sample, for the exp map's chain rule
+                aux = torch.empty(B, S, 6, device=dev, dtype=torch.float32)
+        with _lib.timed("mlp_fwd_warp", B * S):
+            check(lib().hn_mlp_fwd_warp(C.byref(desc), ptr(packed), ptr(pts), ptr(ids), B, S, ptr(warped), ptr(saved),
+                                        ptr(aux), stream()), "hn_mlp_fwd_warp")
+        _lib.count(1)
+        ctx.model, ctx.shape = model, (B, S)
+        ctx.param_meta = [(slot, p.shape, p.numel()) for slot, p in zip(model._warp_slots(), params)]
+        ctx.save_for_backward(ids, saved, packed, pts if aux is not None else None, aux, pe_alpha)
+        ctx.set_materialize_grads(False)
+        return warped
+
+    @staticmethod
+    @torch.amp.custom_bwd(device_type="cuda")
+    def backward(ctx, g_warped):
+        ids, saved, packed, pts, aux, pe_alpha = ctx.saved_tensors
+        model = ctx.model
+        B, S = ctx.shape
+        if g_warped is None:
+            return (None,) * (4 + len(ctx.param_meta))
+        if saved is None:
+            raise RuntimeError("hn_mlp_bwd_warp needs the activation stash; forward ran without grad enabled")
+        dev = g_warped.device
+        g_warped = g_warped.to(torch.float32).contiguous()
+        direct = model._flat_grads is not None and model._flat_grads.flat.device == dev
+        if direct:
+            offs, flat_grad = model._flat_offsets(), model._flat_grads.flat
+        else:
+            offs, total = model._grad_offsets()
+            flat_grad = torch.zeros(total, device=dev, dtype=torch.float32)
+        work = torch.empty(model._sizes(B * S).warp_workspace_bytes, device=dev, dtype=torch.uint8)
+        d = C.byref(model._desc)
+        with _lib.timed("mlp_dgrad_warp", B * S):
+            check(lib().hn_mlp_bwd_warp_data(d, ptr(packed), ptr(ids), ptr(saved), ptr(g_warped), B, S, offs, ptr(flat_grad),
+                                             ptr(work), ptr(pts), ptr(aux), stream()), "hn_mlp_bwd_warp_data")
+        with _lib.timed("mlp_wgrad_warp", B * S):
+            check(lib().hn_mlp_bwd_warp_weights(d, ptr(saved), B, S, offs, ptr(flat_grad), ptr(work), ptr(pe_alpha),
+                                                stream()), "hn_mlp_bwd_warp_weights")
+        _lib.count(2)
+        if direct:
+            return (None,) * (4 + len(ctx.param_meta))
+        return (None,) * 4 + tuple(flat_grad[offs[slot]:offs[slot] + n].view(shape) if ctx.needs_input_grad[4 + i] else None
+                                   for i, (slot, shape, n) in enumerate(ctx.param_meta))
+
+
 class _FusedTrunk(torch.autograd.Function):
     """hn_mlp_fwd_trunk / hn_mlp_bwd_trunk: the template NeRF of one level on rows whose warped point / hyper coordinates
     are given (differentiable input).  Used for the coarse depths the fine level inherits: the warp / sheet nets are
@@ -545,6 +612,17 @@ class NerfModel(PackedWeights, nn.Module):
         """The kernel-visible parameter tensors in slot order (the `*params` of the autograd functions)."""
         return [p for p in self._slot_params() if p is not None]
 
+    def _warp_slots(self):
+        """The slots of the warp stage (GLO table, warp field, hyper sheet): everything but the two template levels."""
+        lo, hi = self._level_param_range(0)[0], self._level_param_range(1)[1]
+        return [i for i in self._slots_present() if not lo <= i < hi]
+
+    def _warp_params(self):
+        """The `*params` of _FusedWarp, detached when grad mode is off (the inference kernel then writes no stash)."""
+        slots = self._slot_params()
+        params = [slots[i] for i in self._warp_slots()]
+        return params if torch.is_grad_enabled() else [q.detach() for q in params]
+
     @staticmethod
     def _level_param_range(level):
         return 29 + 32 * level, 29 + 32 * (level + 1)
@@ -701,23 +779,18 @@ class NerfModel(PackedWeights, nn.Module):
                                           "kernels share one embedding per ray between warp, slicing and conditioning")
         return self._embed_view(first)
 
-    def _zero_dirs(self, points):
-        return torch.zeros(points.shape[0], 3, device=points.device, dtype=torch.float32)
-
     def apply_warp(self, points, warp_embed, extra_params):
         """models.py:583-585: `warp_embed` holds metadata IDS here (the method embeds them itself); returns
-        {'warped_points': (B, S, 3)}.  Runs the fused level-0 network and keeps the warp stage's output."""
+        {'warped_points': (B, S, 3)}.  Runs the warp stage alone (hn_mlp_fwd_warp) on the level-0 blob."""
         if not self.use_warp:
             raise AttributeError("'NerfModel' object has no attribute 'warp_field'")   # as in the reference
-        params = self._canonical_params() if torch.is_grad_enabled() else [q.detach() for q in self._canonical_params()]
-        _, _, warped = _FusedMlp.apply(self, (0, pe_alphas(extra_params)), points, self._zero_dirs(points), warp_embed,
-                                       None, 0.0, *params)
+        warped = _FusedWarp.apply(self, pe_alphas(extra_params), points, warp_embed, *self._warp_params())
         return {'warped_points': warped[..., :3]}
 
     def map_points(self, points, warp_embed, hyper_embed, extra_params, use_warp=True, return_warp_jacobian=False,
                    hyper_point_override=None):
         """models.py:545-581: embedding VECTORS in ((B, S, G) broadcasts of per-ray rows), (warped points (B, S, 3 + H),
-        None) out.  One launch of the fused network on a view whose table is the given vectors."""
+        None) out.  One launch of the warp stage (hn_mlp_fwd_warp) on a view whose table is the given vectors."""
         if not (self.use_warp and use_warp):
             return points, None
         if return_warp_jacobian:
@@ -730,10 +803,7 @@ class NerfModel(PackedWeights, nn.Module):
             raise NotImplementedError("distinct warp / hyper embeddings are not built (one embedding per ray)")
         view = self._embed_view(warp_embed)
         ids = torch.arange(points.shape[0], device=points.device, dtype=torch.int64)
-        params = view._canonical_params() if torch.is_grad_enabled() else [q.detach() for q in view._canonical_params()]
-        _, _, warped = _FusedMlp.apply(view, (0, pe_alphas(extra_params)), points, self._zero_dirs(points), ids, None,
-                                       0.0, *params)
-        return warped, None
+        return _FusedWarp.apply(view, pe_alphas(extra_params), points, ids, *view._warp_params()), None
 
     def map_spatial_points(self, points, warp_embed, extra_params, use_warp=True, return_warp_jacobian=False):
         """models.py:495-512."""

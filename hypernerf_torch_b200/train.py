@@ -121,12 +121,17 @@ def _extra(extra_params):
 
 
 def train_step(model, rays, rgbs, flat_grads, global_rays=None, chunk=8192, optimizer=None, return_stats=False,
-               _exchange=True, extra_params=None, _window=None):
+               _exchange=True, extra_params=None, _window=None, background_points=None, background_weight=1.0,
+               background_noise_std=1e-3, global_background=None):
     """One data-parallel training step on this rank's ray rows (B,9) / target colours (B,3).
     Returns the local contribution to the global-mean loss (sum over ranks = the reference's loss); with
     return_stats, training_step's log entries {'train/loss', 'train/psnr'} (train.py:147-163; psnr of the fine level
     over this rank's rays, metrics.py:4-13) as device tensors.  extra_params: the forward's `extra_params`
-    ({'nerf_alpha', 'warp_alpha', 'hyper_alpha', 'hyper_sheet_alpha'}: the coarse-to-fine encoding windows; unset = none)."""
+    ({'nerf_alpha', 'warp_alpha', 'hyper_alpha', 'hyper_sheet_alpha'}: the coarse-to-fine encoding windows; unset = none).
+    background_points: this rank's (P, 3) known-static points: adds HyperNeRF's background loss
+    (losses.background_loss with background_weight / background_noise_std) once per step, on the step's packed weights
+    and windows, scaled by 1 / global_background (default P) so that the all-reduced gradient is that of the global mean;
+    it is part of the returned loss and reported as 'train/background'."""
     B = rays.shape[0]
     global_rays = B if global_rays is None else global_rays
     extra = _extra(extra_params)
@@ -146,12 +151,22 @@ def train_step(model, rays, rgbs, flat_grads, global_rays=None, chunk=8192, opti
             total += loss.detach()
             if return_stats:
                 fine_sq = sums[1] if fine_sq is None else fine_sq + sums[1]
+        background = None
+        if background_points is not None:
+            background = losses.background_loss(model, background_points, dict(extra), noise_std=background_noise_std,
+                                                weight=background_weight, global_count=global_background)
+            background.backward()
+            background = background.detach()
+            total += background
     if _exchange:
         flat_grads.all_reduce()
     if optimizer is not None:
         optimizer.step()
     if return_stats:
-        return {'train/loss': total, 'train/psnr': -10.0 * torch.log10(fine_sq / (3.0 * B))}
+        stats = {'train/loss': total, 'train/psnr': -10.0 * torch.log10(fine_sq / (3.0 * B))}
+        if background is not None:
+            stats['train/background'] = background
+        return stats
     return total
 
 
@@ -303,7 +318,8 @@ def save_ckpt(model, path, epoch=0, global_step=0, optimizer=None, module_name='
 
 
 def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=0.0, decay_step=(20,), decay_gamma=0.1,
-        chunk=8192, seed=0, ckpt_path=None, log_every=0, cuda_graph=False, extra_params=None):
+        chunk=8192, seed=0, ckpt_path=None, log_every=0, cuda_graph=False, extra_params=None, background_points=None,
+        background_batch_size=16384, background_weight=1.0):
     """Minimal stand-in for `Trainer.fit(NeRFSystem)` (train.py:35-233) on a ray pool that is already on the device:
     per epoch one shuffled pass over (rays (P,9), rgbs (P,3)) in batches of `batch_size` (train_dataloader,
     train.py:133-138: shuffle=True; the last short batch is kept, as DataLoader's drop_last=False does), each batch
@@ -312,9 +328,14 @@ def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=
     passes its own shard of the pool (SURVEY.md §8(e)); gradients are all-reduced inside train_step.
     cuda_graph: replay the full-size batches from one CUDA graph (GraphedTrainStep); the last short batch of an epoch runs
     eagerly.  extra_params: the forward's encoding-window alphas (train_step), a dict or a callable step -> dict (a
-    coarse-to-fine schedule; `step` counts from 0).  Returns a list of per-step dicts {'epoch', 'step', 'lr', 'train/loss',
-    'train/psnr'} (training_step's log)."""
+    coarse-to-fine schedule; `step` counts from 0).  background_points: this rank's shard (Q, 3) of the known-static
+    points; every step draws background_batch_size of them (with replacement, from a generator seeded with seed + 1) for
+    train_step's background loss (not with cuda_graph).  Returns a list of per-step dicts {'epoch', 'step', 'lr',
+    'train/loss', 'train/psnr'[, 'train/background']} (training_step's log)."""
     distributed = dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
+    if background_points is not None and cuda_graph:
+        raise ValueError("fit: the background loss does not run in the CUDA-graph step (GraphedTrainStep); pass "
+                         "cuda_graph=False")
     fg = FlatGrads(model.parameters())
     model.attach_flat_grads(fg)
     opt = FusedAdam(fg, lr=lr, eps=1e-8, weight_decay=weight_decay)
@@ -329,6 +350,7 @@ def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=
         dist.all_reduce(n, op=dist.ReduceOp.MIN)
         P = int(n.item())
     gen = torch.Generator(device=rays.device).manual_seed(seed)
+    bg_gen = torch.Generator(device=rays.device).manual_seed(seed + 1) if background_points is not None else None
     step, log = 0, []
     graphed = None
     for epoch in range(num_epochs):
@@ -346,8 +368,13 @@ def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=
                                                windowed=extra_params is not None)
                 stats = {k: v.clone() for k, v in graphed(r, t, opt, extra).items()}
             else:
+                bg = None
+                if background_points is not None:
+                    bg = background_points[torch.randint(background_points.shape[0], (background_batch_size,),
+                                                         device=rays.device, generator=bg_gen)]
                 stats = train_step(model, r, t, fg, global_rays=world * r.shape[0], chunk=chunk, optimizer=opt,
-                                   return_stats=True, extra_params=extra)
+                                   return_stats=True, extra_params=extra, background_points=bg,
+                                   background_weight=background_weight, global_background=world * background_batch_size)
             step += 1
             log.append({'epoch': epoch, 'step': step, 'lr': opt.param_groups[0]['lr'], **stats})
             if log_every and step % log_every == 0:

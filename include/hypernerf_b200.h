@@ -80,7 +80,9 @@ typedef struct hn_sizes {
   int64_t saved_bytes;        /* activations saved by hn_mlp_fwd for n_samples (training)           */
   int64_t workspace_bytes;    /* hn_mlp_bwd scratch (pre-activation gradients) for n_samples        */
   int64_t flat_param_floats;  /* total parameter count                                              */
-  int64_t reserved[4];
+  int64_t warp_saved_bytes;   /* activations saved by hn_mlp_fwd_warp for n_samples (0 without warp) */
+  int64_t warp_workspace_bytes; /* hn_mlp_bwd_warp_* scratch for n_samples (0 without warp)          */
+  int64_t reserved[2];
 } hn_sizes;
 
 int hn_abi_version(void);
@@ -232,6 +234,37 @@ int hn_mlp_bwd_weights_windowed(const hn_model_desc* desc, const void* saved, in
 int hn_mlp_bwd_trunk_weights_windowed(const hn_model_desc* desc, const void* saved, int64_t B, int S, int level,
                                       const int64_t* grad_offsets /* host */, float* flat_grad, const void* workspace,
                                       const float* pe_alpha, void* stream);
+
+/* Warp-stage-only evaluation (level-0 blob as hn_pack_weights[_windowed] packed it): the TranslationField + HyperSheetMLP
+ * (warping.py:28-125, modules.py:302-337; or the axis-aligned hyper point, models.py:533-534) or the SE3Field
+ * (warping.py:128-272) that hn_mlp_fwd runs ahead of the template, without the template behind it.  `warped` is
+ * bit-identical to hn_mlp_fwd's `warped` output for the same points, ids, blob and mode (inference / training).
+ *   hn_mlp_fwd_warp          points (B,S,3), ids (B,) -> warped (B,S,3+H); saved (hn_sizes.warp_saved_bytes; NULL =
+ *                            inference); aux: SE3 only, (B,S,6) screw parameters (w, v), required with a stash
+ *   hn_mlp_bwd_warp_data     g_warped (B,S,3+H) -> pre-activation gradients in `workspace` (hn_sizes.warp_workspace_bytes)
+ *                            and the GLO-table gradient; points / aux: SE3 only, as the forward saw / wrote them.  The
+ *                            sample points take no gradient.
+ *   hn_mlp_bwd_warp_weights  dW / db of the warp / sheet tensors into flat_grad; pe_alpha: NULL for an unwindowed blob, else
+ *                            the device alphas the blob was packed with (hn_pack_weights_windowed).
+ * A static descriptor or one without warp is rejected (-13); B and S must be positive. */
+int hn_mlp_fwd_warp(const hn_model_desc* desc, const void* packed, const float* points, const int64_t* ids, int64_t B, int S,
+                    float* warped, void* saved, float* aux, void* stream);
+int hn_mlp_bwd_warp_data(const hn_model_desc* desc, const void* packed, const int64_t* ids, const void* saved,
+                         const float* g_warped, int64_t B, int S, const int64_t* grad_offsets /* host */, float* flat_grad,
+                         void* workspace, const float* points, const float* aux, void* stream);
+int hn_mlp_bwd_warp_weights(const hn_model_desc* desc, const void* saved, int64_t B, int S,
+                            const int64_t* grad_offsets /* host */, float* flat_grad, const void* workspace,
+                            const float* pe_alpha, void* stream);
+
+/* compute_background_loss + utils.general_loss_with_squared_residual of the JAX HyperNeRF (hypernerf/training.py): the
+ * torch port has no counterpart (its losses.py has the MSE only), so the formula is restated (DESIGN.md §2c).  For n
+ * points with warped outputs (n, warped_cols) and the jittered inputs points (n, 3):
+ *   r^2 = sum_{c<3} (warped_c - points_c)^2,  rho = (b / a) ((r^2 / scale^2 / b + 1)^(a/2) - 1),
+ *   b = max(eps, |alpha - 2|), a = sign(alpha) max(eps, |alpha|) (sign(0) = +1), eps = FLT_EPSILON;
+ *   sums[0] += sum rho (caller zeroes it);  g_warped[:, :3] = grad_scale d rho / d r^2 2 (warped - points),
+ *   g_warped[:, 3:] = 0 (g_warped may be NULL).  n must be positive, scale positive. */
+int hn_background_loss(const float* warped, const float* points, int64_t n, int warped_cols, float alpha, float scale,
+                       float grad_scale, float* sums, float* g_warped, void* stream);
 
 /* losses.py:9-14 (MSELoss: mean-MSE of coarse.rgb + fine.rgb against the target colours) fused with its gradient seed and
  * with the fine-level MSE of metrics.py:4-13 (psnr = -10 log10(mse)).  sums[0] += sum (coarse - t)^2, sums[1] += sum
