@@ -65,15 +65,22 @@ struct Shape {
   static constexpr bool STATIC = STATIC_;   // static baseline models/nerf.py: no GLO / warp / sheet / hyper coordinates
   static constexpr bool NOWARP = !STATIC_ && H_ == 0;   // NerfModel(use_warp=False): the template alone on the raw points
   static constexpr bool SE3 = SE3_;         // warp stage = SE3Field (warping.py:128-240): input posenc(points, 0, WF) alone
+  // SE3Field + HyperSheetMLP (bendy sheet, SF > 0): the 192-wide merged warp stage reads the vector
+  // [posenc(points, 0, WF) | posenc_orig(points, SF) | GLO], held in ACT (hn_mlp_program.h: kSe3W)
+  static constexpr bool WS_ACT = SE3_ && SF_ > 0;
   static constexpr int G = G_, H = H_, WF = WF_, SF = SF_, XF = XF_, HF = HF_;
   static constexpr int VF = VF_;            // hyper model: the MAXIMUM view frequency count (run time: FwdParams::view_freqs)
-  static constexpr int PE_W = SE3 ? 6 * WF : 3 + 6 * WF, IN_W = SE3 ? PE_W : PE_W + G, KW = NOWARP ? 0 : pad16(IN_W);
+  static constexpr int PE_S = 3 + 6 * SF;
+  static constexpr int PE_W = SE3 ? 6 * WF : 3 + 6 * WF, IN_W = WS_ACT ? PE_W + PE_S + G : SE3 ? PE_W : PE_W + G,
+                       KW = NOWARP ? 0 : pad16(IN_W);
   static constexpr int PE_X = 3 + 6 * XF, PE_H = H * (1 + 2 * HF), IN_T = PE_X + PE_H, KT = pad16(IN_T);
   static constexpr int PE_V = 3 + 6 * VF, KV = STATIC ? pad16(PE_V) : kKV;
   static constexpr bool TIN_ACT = !STATIC && trunk_in_act(KT);   // trunk input vector in ACT (hn_mlp_program.h: kMaxTrunkInInb)
   // bias folding (hn_mlp_program.h): the last two columns of INB's last chunk pair hold 1.0; they sit in
   // the zero padding of the widest input vector when every vector that reaches the last chunk has >= 2 pad columns
-  static constexpr int INB_CHUNKS = STATIC ? inb_chunks_of(KW, IN_W, 0, 0, KV, PE_V) : inb_chunks_of(KW, IN_W, KT, IN_T, KV, PE_V);
+  static constexpr int INB_CHUNKS = STATIC ? inb_chunks_of(KW, IN_W, 0, 0, KV, PE_V)
+                                           : inb_chunks_of(WS_ACT ? 0 : KW, IN_W, KT, IN_T, KV, PE_V);
+  static_assert(!(WS_ACT && TIN_ACT), "one input vector in ACT per model: FE_SKIPFEED serves either the warp stage or the trunk");
   static constexpr int N_RGB0A = pad16(kRgbW + 1);
   static constexpr int NWARPED = 3 + H;     // columns of a warped point + hyper coordinates
 };
@@ -83,6 +90,7 @@ using CfgH8 = Shape<8, 8, 10, 7, 10, 6, 6>;   // bendy sheet with 8 outputs, or 
 using CfgT = Shape<8, 0, 10, 7, 10, 6, 6>;    // no warp: template NeRF on the raw points
 using CfgStatic = Shape<0, 0, 10, 0, 10, 0, 4, true>;   // NeRF(): xyz PE 63 (-> K 64), dir PE 27 (-> K 32)
 using CfgSE3 = Shape<8, 8, kSe3Freqs, 0, 10, 6, 6, false, true>;   // config 5: SE3 warp + axis-aligned slicing (hyper point = GLO vector)
+using CfgSE3S = Shape<8, 2, kSe3Freqs, 7, 10, 6, 6, false, true>;  // SE3 warp + bendy sheet with 2 outputs (HyperNeRF's "DS" model)
 
 // ------------------------------------------------------------------------------------------------------
 // shared memory plan of the fused kernels
@@ -495,6 +503,26 @@ __device__ __forceinline__ void store_trunk_input(const float* wp, uint8_t* act_
   }
 }
 
+// Warp-stage input vector of SE3 + sheet (Shape::WS_ACT): [posenc(points, 0, WF) | posenc_orig(points, SF) | GLO | 0],
+// written as bf16 into ACT[0, KW) (and the stash) by the prologue, and again by the FE_SKIPFEED epilogue
+template <class C>
+__device__ __forceinline__ void store_ws_input(const FwdParams& p, int64_t gq, int64_t ray, uint8_t* act_row, uint4* save_row,
+                                               int save_chunk) {
+  float f[C::KW], pt[3];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) pt[i] = __ldg(p.points + gq * 3 + i);
+  posenc_se3(pt, f);
+  posenc<3, C::SF>(pt, f + C::PE_W);
+  const int64_t id = __ldg(p.ids + ray);
+  HN_CHECK_ID(id, p.n_embed);
+  const float* e = p.glo + id * C::G;
+#pragma unroll
+  for (int i = 0; i < C::G; ++i) f[C::PE_W + C::PE_S + i] = __ldg(e + i);
+#pragma unroll
+  for (int i = C::IN_W; i < C::KW; ++i) f[i] = 0.f;
+  store_features<C::KW>(f, act_row, save_row, save_chunk);
+}
+
 // d(GLO embedding) of one sample (G values in r[0..G)) -> per-ray reduction -> atomics on the table gradient
 template <int G>
 __device__ __forceinline__ void glo_grad_add(const float* v_in, bool valid, int64_t id, float* __restrict__ glo_grad, int lane) {
@@ -797,6 +825,7 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
       // (the sample point and view direction are re-loaded where they are needed — FE_WSHEAD, FE_BOTT — instead of being
       // kept in registers across the drain loops; only the wide trunk inputs keep the warped point for FE_SKIPFEED)
       float wp_keep[C::TIN_ACT ? C::NWARPED : 1];
+      float hy_keep[C::WS_ACT ? C::H : 1];   // SE3 + sheet: the sheet's hyper coordinates, from FE_LINSHEET to FE_WSHEAD
       const bool trunk_only = !C::STATIC && p.warped_in != nullptr;
       if constexpr (PRIMARY) {
       if (trunk_only) {
@@ -820,6 +849,11 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
             store_ones_pair<C, C::KT>(inb_row);
           }
         }
+      } else if constexpr (C::WS_ACT) {
+        // prologue: the warp-stage vector -> ACT; INB only gets the ones pair of the folded biases (the trunk input follows
+        // from FE_WSHEAD)
+        store_ws_input<C>(p, gq, ray, act_row, save_row, p.x_in_ws);
+        store_ones_only<C>(inb_row);
       } else if constexpr (!C::NOWARP) {
       // prologue: [posenc(points, WF) | GLO | 0] -> INB   (static baseline: [Embedding(xyz) | 0], nerf.py:21-38)
         float f[C::KW];
@@ -879,6 +913,10 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
 #pragma unroll
             for (int i = 0; i < 3; ++i) x[i] = wp[i];
             se3_apply(x, wv, wv + 3, wp);
+            if constexpr (C::WS_ACT) {
+#pragma unroll
+              for (int i = 0; i < C::H; ++i) wp[3 + i] = hy_keep[i];
+            }
             if (valid && p.aux != nullptr) {
 #pragma unroll
               for (int i = 0; i < 6; ++i) p.aux[g * 6 + i] = wv[i];
@@ -914,9 +952,21 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
         } else if (L.epi == FE_SKIPFEED) {
           // hidden part of the skip layer is in the accumulator and stays there; ACT[0, KT) <- the trunk input vector,
           // recomputed from the warped point this thread still holds, for the input part that accumulates on top
+          // (SE3 + sheet: the warp stage's skip layer, ACT[0, KW) <- the warp-stage vector)
           if constexpr (PRIMARY && C::TIN_ACT) store_trunk_input<C>(wp_keep, act_row, inb_row, nullptr, 0);
+          if constexpr (PRIMARY && C::WS_ACT) store_ws_input<C>(p, gq, ray, act_row, nullptr, 0);
         } else if (L.epi == FE_LINEAR) {
           fwd_cols_share<false, STASH, FOLD>(share, tlane, bias, act_row, save_row, L.save_chunk, L.n_out, nullptr);
+        } else if (C::WS_ACT && L.epi == FE_LINSHEET) {
+          // SE3 logit columns [0, 128) as FE_LINEAR; the sheet's H outputs in [128, 144) are kept for FE_WSHEAD
+          fwd_cols_share<false, STASH, FOLD>(share, tlane, bias, act_row, save_row, L.save_chunk, kSe3W, nullptr);
+          if constexpr (PRIMARY && C::WS_ACT) {
+            uint32_t r[16];
+            tmem_ld16(tlane + kSe3W, r);
+            tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < C::H; ++i) hy_keep[i] = __uint_as_float(r[i]) + head_bias<FOLD>(bias, kSe3W + i);
+          }
         } else if (L.epi == FE_SIGMA) {
           // static baseline: raw sigma = Linear(W, 1)(h8) (nerf.py:109); rendering.py:150 uses relu(sigma + noise)
           if constexpr (PRIMARY) {
@@ -1051,8 +1101,10 @@ __device__ __forceinline__ void trunk_in_bwd(uint32_t tlane, const float* wp, fl
 }
 
 // d(warped point, hyper coordinates) of one row in f[0, 3 + H) -> the warp / sheet head's pre-activation gradient in f[0, 16)
+// (SE3 + sheet: the exp map's in f[0, 16), the sheet head's = d(hyper coordinates) in gh[0, H))
 template <class C>
-__device__ __forceinline__ void wshead_dy(const BwdParams& p, float* f, bool valid, int64_t ray, int64_t gq, int64_t gc, int lane) {
+__device__ __forceinline__ void wshead_dy(const BwdParams& p, float* f, float* gh, bool valid, int64_t ray, int64_t gq, int64_t gc,
+                                          int lane) {
   if constexpr (C::H == C::G) {
     if (p.mflags & MF_AXIS) {
       // axis-aligned slicing: the hyper coordinates ARE the GLO vector (models.py:533-534), their gradient
@@ -1066,11 +1118,28 @@ __device__ __forceinline__ void wshead_dy(const BwdParams& p, float* f, bool val
   if constexpr (C::SE3) {
     // d(warped xyz) -> d(w, v) through the exp map; columns 0..2 / 3..5 of the head's pre-activation gradient
     float x[3], wv[6], gy[3];
+    if constexpr (C::WS_ACT) {
+#pragma unroll
+      for (int i = 0; i < C::H; ++i) gh[i] = f[3 + i];
+    }
 #pragma unroll
     for (int i = 0; i < 3; ++i) { x[i] = __ldg(p.points + gq * 3 + i); gy[i] = f[i]; }
 #pragma unroll
     for (int i = 0; i < 6; ++i) wv[i] = __ldg(p.aux + gc * 6 + i);
     se3_apply_bwd(x, wv, wv + 3, gy, f, f + 3);
+  }
+}
+
+// the head's dY (f, 16 columns) -> ACT[0, 16) and the dY stash at `chunk`; SE3 + sheet: the sheet head's dY (gh) -> the stash
+// at chunk + 2 (SlabMap::d_sheethead) and ACT[16, 32), where the head^T layer leaves it unread (BE_LINSHEET re-writes it)
+template <class C>
+__device__ __forceinline__ void store_head_dy(const float* f, const float* gh, uint8_t* act_row, uint4* save_row, int chunk) {
+  store_features<16>(f, act_row, save_row, chunk);
+  if constexpr (C::WS_ACT) {
+    float fs[16];
+#pragma unroll
+    for (int i = 0; i < 16; ++i) fs[i] = i < C::H ? gh[i] : 0.f;
+    store_features<16>(fs, act_row + 2 * kChunkBytes, save_row, chunk + 2);
   }
 }
 
@@ -1164,6 +1233,7 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_dgrad_kernel(const __grid_
       const size_t half = (size_t)tile * (2 * kSubTiles) + sub * 2 + (row >> 6);
       const uint32_t* gate_row = p.gates + half * (size_t)p.g_total * kHalfRows + (row & 63);
       uint4* save_row = reinterpret_cast<uint4*>(p.dsaved + half * (size_t)p.d_total * kHalfChunkBytes) + (row & 63);
+      float gh_keep[C::WS_ACT ? C::H : 1] = {};   // SE3 + sheet: the sheet head's dY, from the head's dY to BE_LINSHEET
 
       if constexpr (PRIMARY && !C::STATIC && !C::NOWARP) {
         if (prog.flags & PF_WARP_ONLY) {
@@ -1175,8 +1245,8 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_dgrad_kernel(const __grid_
 #pragma unroll
             for (int i = 0; i < C::NWARPED; ++i) f[i] = __ldg(p.g_warped + gc * C::NWARPED + i);
           }
-          wshead_dy<C>(p, f, valid, ray, gq, gc, lane);
-          store_features<16>(f, act_row, save_row, p.d_rgbhead);
+          wshead_dy<C>(p, f, gh_keep, valid, ray, gq, gc, lane);
+          store_head_dy<C>(f, gh_keep, act_row, save_row, p.d_rgbhead);
         }
       }
       // prologue: dY of the rgb head = g_rgb * y (1 - y) (Sigmoid, models.py:164)
@@ -1232,9 +1302,17 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_dgrad_kernel(const __grid_
         }
         { long long t0 = HN_T0(); mbar_wait(my_acc, ph_acc); ph_acc ^= 1; t_acc += HN_T0() - t0; }
         tc_fence_after();
-        if (L.epi == BE_LINEAR || L.epi == BE_LINCOND) {
+        if (L.epi == BE_LINEAR || L.epi == BE_LINCOND || (C::WS_ACT && L.epi == BE_LINSHEET)) {
           if (L.n_out == kTrunkW) bwd_linear_share<kTrunkW>(share, tlane, act_row, save_row, L.save_chunk);
           else bwd_linear_share<kRgbW>(share, tlane, act_row, save_row, L.save_chunk);
+          if constexpr (PRIMARY && C::WS_ACT) {
+            if (L.epi == BE_LINSHEET) {   // A operand of the sheet logit^T op of the next layer (kSe3W == kRgbW columns above)
+              float fs[16];
+#pragma unroll
+              for (int i = 0; i < 16; ++i) fs[i] = i < C::H ? gh_keep[i] : 0.f;
+              store_features<16>(fs, act_row + (kSe3W / 8) * kChunkBytes, nullptr, 0);
+            }
+          }
           if constexpr (PRIMARY && !C::STATIC) {
             if (L.epi == BE_LINCOND) {
               // gradient of the GLO condition columns of the view vector (alpha / rgb conditioning, modules.py:283,292),
@@ -1286,8 +1364,8 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_dgrad_kernel(const __grid_
               if (p.g_warped != nullptr) f[i] += __ldg(p.g_warped + gq * C::NWARPED + i);
             }
           }
-          wshead_dy<C>(p, f, valid, ray, gq, gc, lane);
-          store_features<16>(f, act_row, save_row, L.save_chunk);
+          wshead_dy<C>(p, f, gh_keep, valid, ray, gq, gc, lane);
+          store_head_dy<C>(f, gh_keep, act_row, save_row, L.save_chunk);
           }
         } else if constexpr (!C::NOWARP) {  // BE_GLO: d(GLO embedding) of this sample -> per-ray reduction -> atomics on the table gradient
           uint32_t r[16];
@@ -1749,9 +1827,10 @@ extern "C" int hn_query(const hn_model_desc* desc, int64_t n_samples, hn_sizes* 
     cnt += lin(kSe3W, m.in_w) + 4 * lin(kSe3W, kSe3W) + lin(kSe3W, kSe3W + m.in_w) + lin(kSe3W, kSe3W) +
            2 * (lin(kSe3W, kSe3W) + lin(3, kSe3W));
   } else if (!m.nowarp) {
-    if (!m.axis) cnt += lin(kSheetW, m.in_s) + 4 * lin(kSheetW, kSheetW) + lin(kSheetW, kSheetW + m.in_s) + lin(m.H, kSheetW);
     cnt += lin(kWarpW, m.in_w) + 4 * lin(kWarpW, kWarpW) + lin(kWarpW, kWarpW + m.in_w) + lin(3, kWarpW);
   }
+  if (!m.nowarp && !m.axis)   // the HyperSheetMLP of bendy-sheet slicing, with either warp field
+    cnt += lin(kSheetW, m.in_s) + 4 * lin(kSheetW, kSheetW) + lin(kSheetW, kSheetW + m.in_s) + lin(m.H, kSheetW);
   int64_t lvl = lin(kTrunkW, m.in_t) + 7 * lin(kTrunkW, kTrunkW) + lin(kTrunkW, kTrunkW + m.in_t) + lin(kRgbW, kTrunkW) +
                 lin(kRgbW, kRgbW + m.pe_v + (m.cond_r ? m.G : 0)) + 3 * lin(kRgbW, kRgbW) + lin(3, kRgbW) +
                 lin(1, kRgbW + (m.cond_a ? m.G : 0));
@@ -1802,9 +1881,10 @@ static int model_flags(const hn_model_desc& d) {
   return f;
 }
 // which compile-time shape serves a descriptor: 0 static, 1 hyper_dim 2, 2 hyper_dim 4, 3 hyper_dim 8, 4 no warp, 5 SE3 warp
+// + axis-aligned slicing, 6 SE3 warp + bendy sheet
 static int shape_of(const hn_model_desc& d) {
   if (is_static(d)) return 0;
-  if (d.flags & HN_FLAG_WARP_SE3) return 5;
+  if (d.flags & HN_FLAG_WARP_SE3) return (d.flags & HN_FLAG_SLICE_AXIS) ? 5 : 6;
   if (!has_warp(d)) return 4;
   return d.hyper_dim == 2 ? 1 : d.hyper_dim == 4 ? 2 : 3;
 }
@@ -1815,6 +1895,7 @@ static int shape_of(const hn_model_desc& d) {
     case 2: MACRO(CfgH4); break;        \
     case 3: MACRO(CfgH8); break;        \
     case 5: MACRO(CfgSE3); break;       \
+    case 6: MACRO(CfgSE3S); break;      \
     default: MACRO(CfgT); break;        \
   }
 

@@ -26,10 +26,15 @@ int validate_desc(const hn_model_desc& d) {
     return set_error(-10, "hn_model_desc: without warp map_points returns the raw points (models.py:568-569): pass no slicing flag");
   if (d.xyz_freqs != 10 || d.view_freqs < 0 || d.view_freqs > kMaxViewFreqs)
     return set_error(-11, "hn_model_desc: kernels are instantiated for xyz freqs 10 and view freqs <= 6");
-  if (se3) {
-    if (!axis || d.glo_dim != 8 || d.hyper_dim != 8 || d.hyper_freqs != 6 || d.warp_freqs != kSe3Freqs)
+  if (se3 && axis) {
+    if (d.glo_dim != 8 || d.hyper_dim != 8 || d.hyper_freqs != 6 || d.warp_freqs != kSe3Freqs)
       return set_error(-11, "hn_model_desc: the SE3 warp is instantiated for axis_aligned_plane slicing with G = hyper_dim = 8, "
                             "hyper freqs 6 and posenc(points, 0, 8) (warp_freqs = 8; warping.py:150-151)");
+  } else if (se3) {
+    if (d.glo_dim != 8 || d.hyper_dim != 2 || d.hyper_freqs != 6 || d.warp_freqs != kSe3Freqs || d.sheet_freqs != 7)
+      return set_error(-11, "hn_model_desc: the SE3 warp with bendy_sheet slicing is instantiated for G = 8, hyper_dim 2, hyper "
+                            "freqs 6, sheet freqs 7 and posenc(points, 0, 8) (warp_freqs = 8); add an instantiation in hn_mlp.cu "
+                            "for other shapes");
   } else if (warp) {
     if (d.glo_dim != 8 || d.hyper_freqs != 6 || d.warp_freqs != 10 || d.sheet_freqs != 7)
       return set_error(-11, "hn_model_desc: kernels are instantiated for G=8, hyper freqs 6 (warp 10, sheet 7); add an "
@@ -74,8 +79,10 @@ struct Builder {
   }
   // One logical [n x k_total] weight matrix (+ 16 bias rows in the folded-bias forward programs), consumed by one or
   // more parts; the parts may sit in consecutive layers (split skip layer, see kMaxTrunkInInb).
-  void begin_logical(int n, int k_total) {
-    const int kb = ones_col >= 0 ? 16 : 0;   // bias rows (hn_mlp_program.h: bias folding)
+  // bias = false: a matrix without bias rows (the hidden parts of the warp stage's split skip layer, whose bias rides with
+  // the input part)
+  void begin_logical(int n, int k_total, bool bias = true) {
+    const int kb = ones_col >= 0 && bias ? 16 : 0;   // bias rows (hn_mlp_program.h: bias folding)
     LogicalOp& l = lg->ops[lg->n++];
     l.w_off16 = w16; l.n = (uint16_t)n; l.k = (uint16_t)(k_total + kb);
     lg_chunks = 0; lg_total = (k_total + kb) / 8;
@@ -219,7 +226,42 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
     b.ones_col = m.ones_col;
     plan->fwd.flags = m.t_in_act ? PF_TIN_ACT : 0;
     int bias = 0;
-    if (m.se3) {
+    if (m.ws_act) {
+      // SE3Field + HyperSheetMLP merged to one 192-wide net (SE3 trunk 128 | sheet 64) on the warp-stage vector in ACT
+      b.begin_layer(FE_RELU, kWsW, bias, s.x_hws[0], kNone, s.g_hws[0]);
+      b.add_op(kWsW, m.KW, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
+      bias += kWsW;
+      for (int l = 1; l < kWsDepth; ++l) {
+        if (l == kSkip + 1) {
+          // hidden parts; the FE_SKIPFEED epilogue re-fills ACT[0, KW) with the input vector; then the input part (one
+          // block-diagonal 192-row matrix, as layer 0) and the biases on top
+          b.begin_layer(FE_SKIPFEED, kWsW, bias, kNone, kNone);
+          b.begin_logical(kSe3W, kSe3W, false);
+          b.part(kSe3W, kSe3W, SRC_ACT, 0, 0, 0);
+          b.begin_logical(kSheetW, kSheetW, false);
+          b.part(kSheetW, kSheetW, SRC_ACT, kSe3W, kSe3W, 0);
+          b.begin_layer(FE_RELU, kWsW, bias, s.x_hws[l], kNone, s.g_hws[l]);
+          b.add_op(kWsW, m.KW, SRC_ACT, 0, 0, SRC_ACT, 0, 0, /*acc_init=*/1);
+        } else {
+          b.begin_layer(FE_RELU, kWsW, bias, s.x_hws[l], kNone, s.g_hws[l]);
+          b.add_op(kSe3W, kSe3W, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
+          b.add_op(kSheetW, kSheetW, SRC_ACT, kSe3W, 0, SRC_ACT, 0, kSe3W);
+        }
+        bias += kWsW;
+      }
+      // the SE3 trunk's logit layer and the sheet's (64 -> H, accumulator columns [128, 144)): the sheet's must run before
+      // the w / v hidden layer, whose 256-wide output overwrites all of ACT
+      b.begin_layer(FE_LINSHEET, kSe3W + 16, bias, s.x_se_logit, kNone);
+      b.add_op(kSe3W, kSe3W, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
+      b.add_op(16, kSheetW, SRC_ACT, kSe3W, 0, SRC_ACT, 0, kSe3W);
+      bias += kSe3W + 16;
+      b.begin_layer(FE_RELU, 2 * kSe3W, bias, s.x_se_wv, kNone, s.g_se_wv);
+      b.add_op(2 * kSe3W, kSe3W, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
+      bias += 2 * kSe3W;
+      b.begin_layer(FE_WSHEAD, 16, bias, s.x_in_t, kNone);
+      b.add_op(16, 2 * kSe3W, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
+      bias += 16;
+    } else if (m.se3) {
       // SE3Field.warp (warping.py:212-227): trunk on posenc(points) alone, logit layer, merged w / v hidden layer, 6-output head
       b.begin_layer(FE_RELU, kSe3W, bias, s.x_hws[0], kNone, s.g_hws[0]);
       b.add_op(kSe3W, m.KW, SRC_INB, 0, 0, SRC_ACT, 0, 0);
@@ -344,13 +386,31 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
       // head^T: A = d(w, v) (16 columns, written by BE_TRUNKIN's exp-map chain rule), gated by the w / v hidden ReLUs
       b.begin_layer(BE_MASK, 2 * kSe3W, 0, s.d_se_wv, s.x_se_wv, s.g_se_wv);
       b.add_op(2 * kSe3W, 16, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
-      // (w hidden | v hidden)^T -> gradient of the logit layer's output (no activation)
-      b.begin_layer(BE_LINEAR, kSe3W, 0, s.d_se_logit, kNone);
+      // (w hidden | v hidden)^T -> gradient of the logit layer's output (no activation); with the sheet, the epilogue also
+      // writes the sheet head's dY into ACT[128, 144)
+      b.begin_layer(m.ws_act ? BE_LINSHEET : BE_LINEAR, kSe3W, 0, s.d_se_logit, kNone);
       b.add_op(kSe3W, 2 * kSe3W, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
-      // logit^T, then trunk layers 5..1 (the skip layer's input part is posenc(points): no gradient wanted)
-      for (int l = kWsDepth; l >= 1; --l) {
-        b.begin_layer(BE_MASK, kSe3W, 0, s.d_ws[l - 1], s.x_hws[l - 1], s.g_hws[l - 1]);
+      if (m.ws_act) {
+        // (SE3 logit | sheet logit)^T, gated by layer 5's ReLUs, then layers 5..1 as in the translation configurations (the
+        // sample point takes no gradient, the GLO columns of the sheet's inputs go to the table)
+        b.begin_layer(BE_MASK, kWsW, 0, s.d_ws[kWsDepth - 1], s.x_hws[kWsDepth - 1], s.g_hws[kWsDepth - 1]);
         b.add_op(kSe3W, kSe3W, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
+        b.add_op(kSheetW, 16, SRC_ACT, kSe3W, 0, SRC_ACT, 0, kSe3W);
+        for (int l = kWsDepth - 1; l >= 1; --l) {
+          b.begin_layer(BE_MASK, kWsW, 0, s.d_ws[l - 1], s.x_hws[l - 1], s.g_hws[l - 1]);
+          if (l == kSkip + 1)  // GLO columns of the sheet's skip input, parked in TMEM cols [192, 208)
+            b.add_op(16, kWsW, SRC_ACT, 0, 0, SRC_ACT, 0, kWsW);
+          b.add_op(kSe3W, kSe3W, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
+          b.add_op(kSheetW, kSheetW, SRC_ACT, kSe3W, 0, SRC_ACT, 0, kSe3W);
+        }
+        b.begin_layer(BE_GLO, 16, 0, kNone, kNone);
+        b.add_op(16, kWsW, SRC_ACT, 0, 0, SRC_ACT, 0, kWsW, /*acc_init=*/1);
+      } else {
+        // logit^T, then trunk layers 5..1 (the skip layer's input part is posenc(points): no gradient wanted)
+        for (int l = kWsDepth; l >= 1; --l) {
+          b.begin_layer(BE_MASK, kSe3W, 0, s.d_ws[l - 1], s.x_hws[l - 1], s.g_hws[l - 1]);
+          b.add_op(kSe3W, kSe3W, SRC_ACT, 0, 0, SRC_ACT, 0, 0);
+        }
       }
     } else if (!m.nowarp) {
       // warp/sheet head^T
@@ -386,7 +446,7 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
   I.x_total = s.x_total; I.d_total = s.d_total; I.g_total = s.g_total;
   I.x_in0 = s.x_in_ws; I.x_in_t = s.x_in_t; I.x_in_v = s.x_in_v;
   I.d_rgbhead = s.d_rgbhead; I.d_sigma = kNone;
-  if (!m.nowarp) { I.x_warp = s.x_in_t; I.d_warp = (uint16_t)(s.d_wshead + 2); I.g_warp = s.g_t[0]; }
+  if (!m.nowarp) { I.x_warp = s.x_in_t; I.d_warp = s.d_t[0]; I.g_warp = s.g_t[0]; }
   I.n_params = HN_NUM_PARAM_TENSORS;
 }
 
@@ -401,6 +461,10 @@ void build_tables(const hn_model_desc& d, int level, const int64_t* off, bool wi
   if (m.se3) {
     wl.add(P_WARP_W(0), 0, m.pe_w, PE_WARP, 3, false);                 // posenc(points, 0, 8): bands of 6, no identity
     wl.add(P_WARP_W(kSkip + 1), kSe3W, m.pe_w, PE_WARP, 3, false);
+    if (m.ws_act) {
+      wl.add(P_SHEET_W(0), 0, m.pe_s, PE_SHEET, 3, true);              // posenc_orig(points, 7)
+      wl.add(P_SHEET_W(kSkip + 1), kSheetW, m.pe_s, PE_SHEET, 3, true);
+    }
   } else if (!m.nowarp) {
     wl.add(P_WARP_W(0), 0, m.pe_w, PE_WARP, 3, true);                  // posenc_orig(points, 10)
     wl.add(P_WARP_W(kSkip + 1), kWarpW, m.pe_w, PE_WARP, 3, true);
@@ -424,7 +488,40 @@ void build_tables(const hn_model_desc& d, int level, const int64_t* off, bool wi
   const int ld_rgb0 = kRgbW + m.pe_v + (m.cond_r ? m.G : 0), ld_alpha = kRgbW + (m.cond_a ? m.G : 0);
   const int k_cond = kRgbW + kViewCondCol;
   const int ld_se5 = kSe3W + m.in_w;
-  if (m.se3) {
+  if (m.ws_act) {
+    // warp-stage vector: [posenc(points, 0, 8) | posenc_orig(points, 7) | GLO]; the sheet reads it from column pe_w on
+    pk.op(F.ops[oi++]);  // layer 0: rows [0, 128) SE3 trunk, rows [128, 192) sheet
+    pk.block(P_WARP_W(0), 0, m.in_w, 1, 0, kSe3W, 0, m.in_w);
+    pk.block(P_SHEET_W(0), 0, m.in_s, 1, kSe3W, kSheetW, m.pe_w, m.in_s);
+    pk.bias_rows(P_WARP_B(0), 0, kSe3W);
+    pk.bias_rows(P_SHEET_B(0), kSe3W, kSheetW);
+    for (int l = 1; l < kWsDepth; ++l) {
+      if (l == kSkip + 1) {   // hidden parts, then the input part of both nets with their biases
+        pk.op(F.ops[oi++]);
+        pk.block(P_WARP_W(l), 0, ld_se5, 1, 0, kSe3W, 0, kSe3W);
+        pk.op(F.ops[oi++]);
+        pk.block(P_SHEET_W(l), 0, lds5, 1, 0, kSheetW, 0, kSheetW);
+        pk.op(F.ops[oi++]);
+        pk.block(P_WARP_W(l), kSe3W, ld_se5, 1, 0, kSe3W, 0, m.in_w);
+        pk.block(P_SHEET_W(l), kSheetW, lds5, 1, kSe3W, kSheetW, m.pe_w, m.in_s);
+        pk.bias_rows(P_WARP_B(l), 0, kSe3W);
+        pk.bias_rows(P_SHEET_B(l), kSe3W, kSheetW);
+      } else {
+        pk.op(F.ops[oi++]);
+        pk.block(P_WARP_W(l), 0, kSe3W, 1, 0, kSe3W, 0, kSe3W);
+        pk.bias_rows(P_WARP_B(l), 0, kSe3W);
+        pk.op(F.ops[oi++]);
+        pk.block(P_SHEET_W(l), 0, kSheetW, 1, 0, kSheetW, 0, kSheetW);
+        pk.bias_rows(P_SHEET_B(l), 0, kSheetW);
+      }
+    }
+    pk.op(F.ops[oi++]);  // SE3 logit layer
+    pk.block(P_WARP_W(kWsDepth), 0, kSe3W, 1, 0, kSe3W, 0, kSe3W);
+    pk.bias_rows(P_WARP_B(kWsDepth), 0, kSe3W);
+    pk.op(F.ops[oi++]);  // sheet logit layer: rows 0..H-1
+    pk.block(P_SHEET_W(kWsDepth), 0, kSheetW, 1, 0, m.H, 0, kSheetW);
+    pk.bias_rows(P_SHEET_B(kWsDepth), 0, m.H);
+  } else if (m.se3) {
     pk.op(F.ops[oi++]);
     pk.block(P_WARP_W(0), 0, m.in_w, 1, 0, kSe3W, 0, m.in_w);
     pk.bias_rows(P_WARP_B(0), 0, kSe3W);
@@ -434,6 +531,8 @@ void build_tables(const hn_model_desc& d, int level, const int64_t* off, bool wi
       pk.block(P_WARP_W(l), 0, ld, 1, 0, kSe3W, 0, ld);
       pk.bias_rows(P_WARP_B(l), 0, kSe3W);
     }
+  }
+  if (m.se3) {
     pk.op(F.ops[oi++]);  // rows [0, 128) w_net.linears.0, [128, 256) v_net.linears.0
     pk.block(P_SE3_W(SE3_W_HID), 0, kSe3W, 1, 0, kSe3W, 0, kSe3W);
     pk.block(P_SE3_W(SE3_V_HID), 0, kSe3W, 1, kSe3W, kSe3W, 0, kSe3W);
@@ -539,9 +638,29 @@ void build_tables(const hn_model_desc& d, int level, const int64_t* off, bool wi
     bop();  // (w hidden | v hidden)^T: dest(n, k < 128) = Wwh[k][n], dest(n, 128 + k) = Wvh[k][n]
     pk.block(P_SE3_W(SE3_W_HID), 0, 1, kSe3W, 0, kSe3W, 0, kSe3W);
     pk.block(P_SE3_W(SE3_V_HID), 0, 1, kSe3W, 0, kSe3W, kSe3W, kSe3W);
-    for (int l = kWsDepth; l >= 1; --l) {
-      bop();
-      pk.block(P_WARP_W(l), 0, 1, l == kSkip + 1 ? ld_se5 : kSe3W, 0, kSe3W, 0, kSe3W);
+    if (m.ws_act) {
+      bop();  // SE3 logit^T
+      pk.block(P_WARP_W(kWsDepth), 0, 1, kSe3W, 0, kSe3W, 0, kSe3W);
+      bop();  // sheet logit^T: dest(j < 64, h < H) = sheetW6[h][j]
+      pk.block(P_SHEET_W(kWsDepth), 0, 1, kSheetW, 0, kSheetW, 0, m.H);
+      for (int l = kWsDepth - 1; l >= 1; --l) {
+        const bool skip = (l == kSkip + 1);
+        if (skip) {  // GLO columns of the sheet's skip input: dest(g, 128 + j) = sheetW5[j][64 + pe_s + g]
+          bop();
+          pk.block(P_SHEET_W(l), kSheetW + m.pe_s, 1, lds5, 0, m.G, kSe3W, kSheetW);
+        }
+        bop();
+        pk.block(P_WARP_W(l), 0, 1, skip ? ld_se5 : kSe3W, 0, kSe3W, 0, kSe3W);
+        bop();
+        pk.block(P_SHEET_W(l), 0, 1, skip ? lds5 : kSheetW, 0, kSheetW, 0, kSheetW);
+      }
+      bop();  // GLO columns of the sheet's layer 0
+      pk.block(P_SHEET_W(0), m.pe_s, 1, m.in_s, 0, m.G, kSe3W, kSheetW);
+    } else {
+      for (int l = kWsDepth; l >= 1; --l) {
+        bop();
+        pk.block(P_WARP_W(l), 0, 1, l == kSkip + 1 ? ld_se5 : kSe3W, 0, kSe3W, 0, kSe3W);
+      }
     }
   } else if (!m.nowarp) {
     bop();  // ws head^T: n < 128 <- warp logit (k < 3); n = 128 + j <- sheet logit (k = 3 + h)
@@ -566,8 +685,19 @@ void build_tables(const hn_model_desc& d, int level, const int64_t* off, bool wi
 
   // biases, in forward layer order
   int bo = 0;
+  if (m.ws_act) {
+    for (int l = 0; l < kWsDepth; ++l) {
+      pk.bias(P_WARP_B(l), bo, kSe3W);
+      pk.bias(P_SHEET_B(l), bo + kSe3W, kSheetW);
+      bo += kWsW;
+    }
+    pk.bias(P_WARP_B(kWsDepth), bo, kSe3W);
+    pk.bias(P_SHEET_B(kWsDepth), bo + kSe3W, m.H);
+    bo += kSe3W + 16;
+  }
   if (m.se3) {
-    for (int l = 0; l <= kWsDepth; ++l) { pk.bias(P_WARP_B(l), bo, kSe3W); bo += kSe3W; }
+    if (!m.ws_act)
+      for (int l = 0; l <= kWsDepth; ++l) { pk.bias(P_WARP_B(l), bo, kSe3W); bo += kSe3W; }
     pk.bias(P_SE3_B(SE3_W_HID), bo, kSe3W);
     pk.bias(P_SE3_B(SE3_V_HID), bo + kSe3W, kSe3W);
     bo += 2 * kSe3W;
@@ -629,12 +759,28 @@ void build_tables(const hn_model_desc& d, int level, const int64_t* off, bool wi
       WgradJob& j = job(s.d_ws[0], kSe3W, s.x_in_ws, m.KW, 0, 0);
       flush(j, P_WARP_W(0), 0, m.in_w, 0, kSe3W, 0, m.in_w);
       bseg(j, P_WARP_B(0), 0, kSe3W);
+      if (m.ws_act) {   // the sheet reads the warp-stage vector from column pe_w on
+        WgradJob& k = job(s.d_ws[0] + kSe3W / 8, kSheetW, s.x_in_ws, m.KW, 0, 0);
+        flush(k, P_SHEET_W(0), 0, m.in_s, 0, kSheetW, m.pe_w, m.in_s);
+        bseg(k, P_SHEET_B(0), 0, kSheetW);
+      }
     }
     for (int l = 1; l < kWsDepth; ++l) {
       const bool skip = (l == kSkip + 1);
       WgradJob& j = job(s.d_ws[l], kSe3W, s.x_hws[l - 1], kSe3W, s.x_in_ws, skip ? m.KW : 0);
       flush(j, P_WARP_W(l), 0, skip ? ld_se5 : kSe3W, 0, kSe3W, 0, skip ? ld_se5 : kSe3W);
       bseg(j, P_WARP_B(l), 0, kSe3W);
+      if (m.ws_act) {
+        WgradJob& k = job(s.d_ws[l] + kSe3W / 8, kSheetW, s.x_hws[l - 1] + kSe3W / 8, kSheetW, s.x_in_ws, skip ? m.KW : 0);
+        flush(k, P_SHEET_W(l), 0, skip ? lds5 : kSheetW, 0, kSheetW, 0, kSheetW);
+        if (skip) flush(k, P_SHEET_W(l), kSheetW, lds5, 0, kSheetW, kSheetW + m.pe_w, m.in_s);
+        bseg(k, P_SHEET_B(l), 0, kSheetW);
+      }
+    }
+    if (m.ws_act) {
+      WgradJob& j = job(s.d_sheethead, 16, s.x_hws[kWsDepth - 1] + kSe3W / 8, kSheetW, 0, 0);
+      flush(j, P_SHEET_W(kWsDepth), 0, kSheetW, 0, m.H, 0, kSheetW);
+      bseg(j, P_SHEET_B(kWsDepth), 0, m.H);
     }
     {
       WgradJob& j = job(s.d_se_logit, kSe3W, s.x_hws[kWsDepth - 1], kSe3W, 0, 0);

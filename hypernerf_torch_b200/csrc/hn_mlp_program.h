@@ -61,6 +61,11 @@ constexpr int kWarpW = 128, kSheetW = 64, kWsDepth = 6, kWsW = kWarpW + kSheetW,
 // columns, no identity, no metadata), a 128 -> 128 logit layer without activation, then the w / v heads: one hidden 128 ReLU
 // layer each (run as one 256-wide layer) and 3 outputs each (one 16-row head: rows 0..2 = w, 3..5 = v).
 constexpr int kSe3W = 128, kSe3Freqs = 8;
+// SE3Field + HyperSheetMLP (HyperNeRF's "DS" model, bendy-sheet slicing, H = 2): the two nets share no input column
+// (posenc(points, 0, 8) has no identity columns and non-integer octaves), so their common input vector is
+// [posenc(points, 0, 8) 48 | posenc_orig(points, 7) 45 | GLO 8] = 101 -> 112 columns.  That is too wide for INB beside
+// the trunk input, so it lives in ACT like the wide trunk inputs (FE_SKIPFEED re-fills it for the skip layer); the merged
+// warp stage is 192 wide (SE3 trunk 128 | sheet 64) as in the translation configurations.
 
 // View-direction condition vector of the template (hyper model): [posenc_orig(viewdirs, view_freqs <= 6) zero-padded to 40
 // columns | GLO condition (8 columns, zero without template conditioning)] = 48 columns, whatever view_freqs is, so that
@@ -91,7 +96,8 @@ constexpr int inb_chunks_of(int KW, int in_w, int KT, int in_t, int KV, int in_v
 struct Dims {
   int G, H;
   bool nowarp, axis, cond_a, cond_r;   // no warp / sheet stage; hyper point = GLO vector; template GLO conditioning
-  bool se3;                            // the warp stage is an SE3Field (no sheet MLP, no GLO input) instead of warp + sheet
+  bool se3;                            // the warp stage is an SE3Field (no GLO input) instead of a TranslationField
+  bool ws_act;                         // SE3Field + HyperSheetMLP: the warp-stage input vector lives in ACT (see kSe3W)
   int ws_w;                            // width of the warp-stage hidden layers: 192 (warp 128 | sheet 64) or 128 (SE3 trunk)
   int pe_w, pe_s, in_w, in_s, KW;  // warp / sheet inputs, shared padded input width (KW = 0 without warp)
   int pe_x, pe_h, in_t, KT;        // trunk input
@@ -105,20 +111,21 @@ inline Dims make_dims(const hn_model_desc& d) {
   Dims m{};
   m.se3 = (d.flags & HN_FLAG_WARP_SE3) != 0;
   m.nowarp = (d.flags & (HN_FLAG_WARP_TRANSLATION | HN_FLAG_WARP_SE3)) == 0;
-  m.ws_w = m.se3 ? kSe3W : kWsW;
   m.axis = (d.flags & HN_FLAG_SLICE_AXIS) != 0;
+  m.ws_act = m.se3 && !m.axis;
+  m.ws_w = m.se3 && !m.ws_act ? kSe3W : kWsW;
   m.cond_a = (d.flags & HN_FLAG_ALPHA_COND) != 0; m.cond_r = (d.flags & HN_FLAG_RGB_COND) != 0;
   m.G = d.glo_dim; m.H = m.nowarp ? 0 : d.hyper_dim;
   m.pe_w = 3 + 6 * d.warp_freqs; m.pe_s = 3 + 6 * d.sheet_freqs;
   m.in_w = m.pe_w + m.G; m.in_s = m.pe_s + m.G;
-  if (m.se3) { m.pe_w = 6 * d.warp_freqs; m.in_w = m.pe_w; m.pe_s = 0; m.in_s = 0; }
-  m.KW = m.nowarp ? 0 : pad16(m.in_w);
+  if (m.se3) { m.pe_w = 6 * d.warp_freqs; m.in_w = m.pe_w; if (!m.ws_act) { m.pe_s = 0; m.in_s = 0; } }
+  m.KW = m.nowarp ? 0 : pad16(m.ws_act ? m.in_w + m.in_s : m.in_w);
   m.pe_x = 3 + 6 * d.xyz_freqs; m.pe_h = m.H * (1 + 2 * d.hyper_freqs);
   m.in_t = m.pe_x + m.pe_h; m.KT = pad16(m.in_t);
   m.pe_v = 3 + 6 * d.view_freqs; m.KV = kKV;
   m.n_rgb0a = pad16(kRgbW + 1);
   m.t_in_act = trunk_in_act(m.KT);
-  m.inb_chunks = inb_chunks_of(m.KW, m.in_w, m.KT, m.in_t, m.KV, m.pe_v);
+  m.inb_chunks = inb_chunks_of(m.ws_act ? 0 : m.KW, m.in_w, m.KT, m.in_t, m.KV, m.pe_v);
   m.ones_col = m.inb_chunks * 8 - 16;
   return m;
 }
@@ -153,6 +160,7 @@ struct SlabMap {
   // gradients w.r.t. every layer's pre-activation output
   uint16_t d_ws[kWsDepth], d_wshead, d_t[kTrunkDepth + 1], d_bott, d_rgb0a, d_r[kRgbDepth] /* [0] unused */, d_rgbhead;
   uint16_t d_se_logit, d_se_wv;
+  uint16_t d_sheethead;   // SE3 + sheet: the sheet logit layer's dY (16 columns), right after d_wshead
   uint16_t d_total;
   // ReLU gate words (one uint32 per row per 32 output columns of every ReLU layer), written by the forward epilogue
   // next to the X slabs and read by the data gradient instead of the activations themselves
@@ -177,6 +185,7 @@ inline SlabMap make_slabs(const Dims& m) {
     for (int l = 0; l < kWsDepth; ++l) { s.d_ws[l] = c; c += m.ws_w / 8; }
     if (m.se3) { s.d_se_logit = c; c += kSe3W / 8; s.d_se_wv = c; c += 2 * kSe3W / 8; }
     s.d_wshead = c; c += 2;
+    if (m.ws_act) { s.d_sheethead = c; c += 2; }
   }
   for (int l = 0; l <= kTrunkDepth; ++l) { s.d_t[l] = c; c += kTrunkW / 8; }
   s.d_bott = c; c += kRgbW / 8;
@@ -219,8 +228,12 @@ struct LogicalOp {
 // FE_SKIPFEED: no drain — the accumulator keeps the hidden part of the skip layer; the epilogue re-fills ACT with the trunk
 // input vector for the input part (see kMaxTrunkInInb).  BE_LINCOND: BE_LINEAR + the GLO-condition columns (-> table gradient).
 // FE_LINEAR: plain linear layer (bias, no activation, stashed): the SE3 trunk's logit layer.
-enum FwdEpi : uint8_t { FE_RELU = 0, FE_WSHEAD, FE_BOTT, FE_RGB0A, FE_RGBHEAD, FE_SIGMA, FE_SKIPFEED, FE_LINEAR };
-enum BwdEpi : uint8_t { BE_MASK = 0, BE_LINEAR, BE_RGB1, BE_SKIPSTORE, BE_TRUNKIN, BE_GLO, BE_LINCOND };
+// SE3 + sheet (Dims::ws_act): FE_SKIPFEED re-fills ACT[0, KW) with the warp-stage input vector instead; FE_LINSHEET is
+// FE_LINEAR on the SE3 logit columns [0, 128) plus the sheet's logit layer (64 -> H) in columns [128, 144), whose H hyper
+// coordinates the epilogue keeps for FE_WSHEAD (the next layer's 256-wide output overwrites all of ACT).  BE_LINSHEET is
+// BE_LINEAR plus the sheet head's dY (kept since BE_TRUNKIN) written to ACT[128, 144) for the (SE3 logit | sheet logit)^T layer.
+enum FwdEpi : uint8_t { FE_RELU = 0, FE_WSHEAD, FE_BOTT, FE_RGB0A, FE_RGBHEAD, FE_SIGMA, FE_SKIPFEED, FE_LINEAR, FE_LINSHEET };
+enum BwdEpi : uint8_t { BE_MASK = 0, BE_LINEAR, BE_RGB1, BE_SKIPSTORE, BE_TRUNKIN, BE_GLO, BE_LINCOND, BE_LINSHEET };
 // PF_WARP_ONLY: a warp-stage-only program (ModelPlan::fwd_warp*, bwd_warp).  Its forward ends at the FE_WSHEAD epilogue,
 // which then writes `warped` (and the SE3 screw) but no trunk input; its data gradient starts at the head^T layer, whose
 // A operand the prologue builds from the upstream g_warped instead of from the rgb head.

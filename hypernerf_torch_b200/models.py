@@ -401,6 +401,7 @@ class NerfModel(PackedWeights, nn.Module):
       use_warp + 'axis_aligned_plane'                      hyper point = the GLO vector, hyper_slice_out_dim == GLO_dim == 8
       use_warp=False (any slicing argument)                the template NeRF on the raw points (models.py:568-569)
       use_warp + 'axis_aligned_plane' + warp_field_type='se3'   SE3Field warp (restated; the reference never instantiates it)
+      use_warp + 'bendy_sheet' + warp_field_type='se3'          SE3Field + HyperSheetMLP (HyperNeRF's "DS" model), hyper_slice_out_dim 2
     each with or without template GLO conditioning (use_nerf_embed + use_alpha_cond [+ use_rgb_cond], models.py:404-445),
     view_fourier_dim <= 6, xyz / hyper fourier dims 10 / 6, GLO_dim 8.  Combinations that fail inside the reference's
     forward (use_warp with slicing 'none'; use_nerf_embed without use_alpha_cond; use_rgb_cond without use_nerf_embed:
@@ -526,9 +527,6 @@ class NerfModel(PackedWeights, nn.Module):
             self._forward_error = "use_rgb_cond without use_nerf_embed: rgb_mlp expects the GLO columns (models.py:269-272)"
         elif self.hyper_slice_method not in ('none', 'bendy_sheet', 'axis_aligned_plane'):
             self._forward_error = f'Unknown hyper slice method {self.hyper_slice_method}.'   # models.py:394-396
-        elif self._se3 and self.hyper_slice_method != 'axis_aligned_plane':
-            self._forward_error = ("warp_field_type 'se3' is built for hyper_slice_method 'axis_aligned_plane' "
-                                   "(BASELINE.json config 5)")
 
         # ---- the kernels' view of the model ---------------------------------------------------------------------------
         cond_a = self.use_nerf_embed and self.use_alpha_condition

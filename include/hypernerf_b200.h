@@ -49,7 +49,10 @@ typedef struct hn_model_desc {
 #define HN_FLAG_ALPHA_COND 16       /* use_nerf_embed + use_alpha_cond: alpha head input [bottleneck | GLO] (modules.py:283)   */
 #define HN_FLAG_RGB_COND 32         /* use_nerf_embed + use_rgb_cond: rgb branch input [bottleneck | view PE | GLO] (:292)     */
 #define HN_FLAG_WARP_SE3 64         /* SE3Field warp (warping.py:128-272, rigid_body.py:55-83) instead of TranslationField; set
-                                       together with HN_FLAG_WARP_TRANSLATION's place taken: flags = WARP_SE3 | SLICE_AXIS.  The
+                                       together with HN_FLAG_WARP_TRANSLATION's place taken: flags = WARP_SE3 | SLICE_AXIS
+                                       (config 5: glo_dim = hyper_dim = 8) or WARP_SE3 | SLICE_BENDY (SE3Field + HyperSheetMLP,
+                                       HyperNeRF's "DS" model: glo_dim 8, hyper_dim 2, sheet_freqs 7; other hyper_dim are
+                                       rejected by hn_query with a message); warp_freqs = 8 either way.  The
                                        reference never instantiates SE3Field and its exp map is not runnable batched
                                        (SURVEY.md App. B.1): parity for this flag is against the batched restatement in oracle/ */
 #define HN_FLAG_STATIC_NERF 4       /* static baseline models/nerf.py:41-123 (one NeRF per blob; xyz_freqs 10,
