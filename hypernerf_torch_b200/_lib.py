@@ -28,6 +28,7 @@ EXPORTS = [
     "hn_composite_fwd", "hn_composite_bwd", "hn_filter_sigma", "hn_mse_loss", "hn_make_ndc_rays", "hn_adam_step", "hn_mlp_fwd", "hn_mlp_bwd", "hn_mlp_bwd_data", "hn_mlp_bwd_weights", "hn_mlp_fwd_trunk", "hn_mlp_bwd_trunk", "hn_mlp_bwd_trunk_data", "hn_mlp_bwd_trunk_weights",
     "hn_pack_weights_windowed", "hn_mlp_bwd_weights_windowed", "hn_mlp_bwd_trunk_weights_windowed",
     "hn_mlp_fwd_warp", "hn_mlp_bwd_warp_data", "hn_mlp_bwd_warp_weights", "hn_background_loss",
+    "hn_mlp_fwd_warp_tangent", "hn_elastic_loss",
 ]
 # microbenchmarks / descriptor probes: their own library and header (include/hypernerf_b200_probe.h), not the product ABI
 PROBE_LIB_PATH = os.path.join(_HERE, "libhypernerf_b200_probe.so")
@@ -107,6 +108,8 @@ def lib():
                                        vp]
     L.hn_mlp_bwd_warp_weights.argtypes = [C.POINTER(ModelDesc), vp, i64, i32, C.POINTER(C.c_int64), vp, vp, vp, vp]
     L.hn_background_loss.argtypes = [vp, vp, i64, i32, f32, f32, f32, vp, vp, vp]
+    L.hn_mlp_fwd_warp_tangent.argtypes = [C.POINTER(ModelDesc), vp, vp, vp, i64, i32, vp, vp, vp]
+    L.hn_elastic_loss.argtypes = [vp, vp, i64, f32, f32, f32, f32, vp, vp, i32, vp]
     if hasattr(L, "hn_debug_set_timing_buffer"):   # role-timing builds only (make timing; HN_LIB selects them)
         L.hn_debug_set_timing_buffer.argtypes = [vp]
         L.hn_debug_set_timing_buffer.restype = C.c_int

@@ -178,6 +178,10 @@ struct FwdParams {
   uint32_t* gates;          // ReLU gate words: [half tile][g_total][64 rows] (inside `saved`, after the X slabs)
   int g_total;
   unsigned long long* dbg;  // optional per-CTA cycle counters (hn_debug_set_timing_buffer)
+  // tangent launch (mlp_fwd_kernel<C, true, true>): (n, 3, 3) Jacobian of the translation warp.  `gates` are then the PRIMAL
+  // stash's gate words, `saved` the nullable tangent stash of 3 planes of x_total X chunks + g_total (unwritten) gate words
+  // per half tile each, and n_tiles counts 3 x the primal tiles (plane = tile / primal tiles).
+  float* jac;
 };
 
 struct BwdParams {
@@ -334,6 +338,32 @@ __device__ __forceinline__ void posenc_bwd(const float* x, const float* g, float
       float c2 = 1.f - 2.f * s[i] * s[i];
       s[i] = s2; c[i] = c2;
     }
+    f *= 2.f;
+  }
+}
+
+// d posenc / d x[c] (the tangent of posenc along input direction c): identity column c -> 1, band k of coordinate c:
+// sin column -> 2^k cos(2^k x_c), cos column -> -2^k sin(2^k x_c); every other column 0.  The sines and cosines are the
+// primal's (sincosf of the base angle, double-angle recurrence), so the tangent matches the encoding it differentiates.
+template <int NC, int NF>
+__device__ __forceinline__ void posenc_tangent(const float* x, int c, float* out) {
+#pragma unroll
+  for (int i = 0; i < NC + 2 * NC * NF; ++i) out[i] = 0.f;
+  float xc = 0.f;
+#pragma unroll
+  for (int i = 0; i < NC; ++i) if (i == c) { xc = x[i]; out[i] = 1.f; }
+  float s, cs;
+  sincosf(xc, &s, &cs);
+  float f = 1.f;
+#pragma unroll
+  for (int k = 0; k < NF; ++k) {
+#pragma unroll
+    for (int i = 0; i < NC; ++i) {
+      if (i == c) { out[NC + 2 * NC * k + i] = f * cs; out[NC + 2 * NC * k + NC + i] = -f * s; }
+    }
+    float s2 = 2.f * s * cs;
+    float c2 = 1.f - 2.f * s * s;
+    s = s2; cs = c2;
     f *= 2.f;
   }
 }
@@ -724,9 +754,15 @@ __device__ __forceinline__ float sigmoid_f(float x) { return 1.f / (1.f + expf(-
 // ======================================================================================================
 // forward
 // ======================================================================================================
+// tangent launch (FwdParams::jac): tile -> (input direction, primal tile) over 3 x the primal's tiles; every direction
+// reads the primal tile's gate words
+__device__ __forceinline__ int tangent_plane(int tile, int n_tiles) { return tile / (n_tiles / 3); }
+
 // STASH = false (inference, hn_mlp_fwd with saved == NULL) compiles every stash store out: even predicated-off
 // st.global instructions in the drain loop cost 23 % of the kernel (2.67 -> 2.06 ms per 1 M samples, measured).
-template <class C, bool STASH>
+// TANGENT (with STASH, translation warp only): the program is ModelPlan::fwd_warp_tangent, one launch for the three input
+// directions (FwdParams::jac); its stash stores are skipped at run time when FwdParams::saved is NULL.
+template <class C, bool STASH, bool TANGENT = false>
 __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_constant__ FwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   using SM = Smem<C>;
@@ -809,7 +845,7 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
     const long long t_begin = HN_T0();
     for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
       const long long t_tile = HN_T0();
-      const int64_t g = (int64_t)tile * kCtaRows + sub * kTileRows + row;
+      const int64_t g = (int64_t)(TANGENT ? tile % (p.n_tiles / 3) : tile) * kCtaRows + sub * kTileRows + row;
       const bool valid = g < p.n;
       const int64_t gc = valid ? g : p.n - 1;
       const int64_t ray = gc / p.S;
@@ -817,7 +853,15 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
       const int64_t gq = p.pos != nullptr ? ray * p.S_full + __ldg(p.pos + gc) : gc;
       uint4* save_row = nullptr;
       uint32_t* gate_row = nullptr;   // this row's column of the half tile's gate words
-      if (p.saved != nullptr) {
+      if constexpr (TANGENT) {
+        const size_t half = (size_t)(tile % (p.n_tiles / 3)) * (2 * kSubTiles) + sub * 2 + (row >> 6);
+        gate_row = p.gates + half * (size_t)p.g_total * kHalfRows + (row & 63);
+        if (p.saved != nullptr) {   // plane c of the tangent stash: the warp-only stash layout of the primal's tiles
+          const size_t plane_bytes = (size_t)(p.n_tiles / 3) * (2 * kSubTiles) * ((size_t)p.x_total * kHalfChunkBytes + (size_t)p.g_total * kHalfRows * 4);
+          save_row = reinterpret_cast<uint4*>(p.saved + tangent_plane(tile, p.n_tiles) * plane_bytes +
+                                              half * (size_t)p.x_total * kHalfChunkBytes) + (row & 63);
+        }
+      } else if (p.saved != nullptr) {
         const size_t half = (size_t)tile * (2 * kSubTiles) + sub * 2 + (row >> 6);
         save_row = reinterpret_cast<uint4*>(p.saved + half * (size_t)p.x_total * kHalfChunkBytes) + (row & 63);
         gate_row = p.gates + half * (size_t)p.g_total * kHalfRows + (row & 63);
@@ -827,7 +871,16 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
       float wp_keep[C::TIN_ACT ? C::NWARPED : 1];
       float hy_keep[C::WS_ACT ? C::H : 1];   // SE3 + sheet: the sheet's hyper coordinates, from FE_LINSHEET to FE_WSHEAD
       const bool trunk_only = !C::STATIC && p.warped_in != nullptr;
-      if constexpr (PRIMARY) {
+      if constexpr (PRIMARY && TANGENT) {
+        // prologue: d posenc(points, WF) / d x[plane] | 0 (GLO columns and padding) -> INB and the tangent stash
+        float f[C::KW], pt[3];
+#pragma unroll
+        for (int i = 0; i < 3; ++i) pt[i] = __ldg(p.points + gq * 3 + i);
+        posenc_tangent<3, C::WF>(pt, tangent_plane(tile, p.n_tiles), f);
+#pragma unroll
+        for (int i = C::PE_W; i < C::KW; ++i) f[i] = 0.f;
+        store_features<C::KW>(f, inb_row, save_row, p.x_in_ws);
+      } else if constexpr (PRIMARY) {
       if (trunk_only) {
         // trunk-only program: the warped point / hyper coordinates of this row were computed by another launch (the
         // coarse level's, for the depths the fine level inherits) or are the raw sample point (model without warp); the
@@ -886,7 +939,7 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
         // a per-block __ldg would go to L2 every time); double-buffered by layer parity
         float* bias = PP ? sbias + chain * 256 : sbias + (li & 1) * 256;
         const long long t_layer = HN_T0();
-        if constexpr (!FOLD) {
+        if constexpr (!FOLD && !TANGENT) {
           if (PP) epi_named_barrier<PP>(chain);   // single buffer per chain: everyone is done with the previous layer's bias
           for (int i = et; i < L.n_out; i += 128 * Sched<PP>::SUBS * kEpiSplit) bias[i] = __ldg(p.bias + L.bias_off + i);
           epi_named_barrier<PP>(chain);
@@ -894,7 +947,23 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_fwd_kernel(const __grid_co
         { long long t0 = HN_T0(); mbar_wait(my_acc, ph_acc); ph_acc ^= 1; t_acc += HN_T0() - t0; }
         tc_fence_after();
         const long long t_drain = HN_T0();
-        if (L.epi == FE_RELU) {
+        if constexpr (TANGENT) {
+          if (L.epi == FE_TANGENT) {
+            // D_l W_l t_{l-1}: the bf16 tangent masked by the primal's ReLU gates, into ACT and the tangent stash
+            uint32_t gw[kWsW / 32];
+            load_gates<kWsW>(gate_row, L.gate_word, gw);
+            bwd_cols<true, kWsW>(tlane, gw, act_row, save_row, L.save_chunk);
+          } else if constexpr (PRIMARY) {   // FE_JACHEAD
+            uint32_t r[16];
+            tmem_ld16(tlane, r);
+            tmem_ld_wait();
+            const int plane = tangent_plane(tile, p.n_tiles);
+            if (valid) {
+#pragma unroll
+              for (int i = 0; i < 3; ++i) p.jac[gq * 9 + i * 3 + plane] = __uint_as_float(r[i]) + (i == plane ? 1.f : 0.f);
+            }
+          }
+        } else if (L.epi == FE_RELU) {
           fwd_cols_share<true, STASH, FOLD>(share, tlane, bias, act_row, save_row, L.save_chunk, L.n_out,
                                       STASH ? gate_row + (size_t)L.gate_word * kHalfRows : nullptr);
         } else if (L.epi == FE_WSHEAD) {
@@ -2042,6 +2111,52 @@ extern "C" HN_FV_HIDDEN int hn_mlp_fwd_warp(const hn_model_desc* desc, const voi
 }
 
 #ifndef HN_MLP_FWD_VARIANT
+template <class C>
+static int launch_fwd_tangent(const FwdParams& fp, int grid, void* stream) {
+  if (int rc = set_smem(mlp_fwd_kernel<C, true, true>, Smem<C>::TOTAL, "hn_mlp_fwd_warp_tangent: smem attr")) return rc;
+  return set_cuda_error(launch_mlp(mlp_fwd_kernel<C, true, true>, grid, Smem<C>::TOTAL, (cudaStream_t)stream, fp),
+                        "hn_mlp_fwd_warp_tangent");
+}
+
+// Jacobian of the translation warp (ModelPlan::fwd_warp_tangent): one launch of 3 x the primal's tiles, gated by the gate
+// words of the primal's warp-only stash (hn_mlp_fwd_warp with a stash); tangent_saved (3 x hn_sizes.warp_saved_bytes,
+// nullable) receives the tangents' X slabs for hn_mlp_bwd_warp_weights.
+extern "C" int hn_mlp_fwd_warp_tangent(const hn_model_desc* desc, const void* packed, const float* points, const void* primal_saved,
+                                       int64_t B, int S, float* jac, void* tangent_saved, void* stream) {
+  if (!desc || !packed || !points || !primal_saved || !jac) return set_error(-2, "hn_mlp_fwd_warp_tangent: null pointer");
+  if (int rc = check_warp_only(desc, B, S, "hn_mlp_fwd_warp_tangent")) return rc;
+  if (desc->flags & HN_FLAG_WARP_SE3)
+    return set_error(-13, "hn_mlp_fwd_warp_tangent: the Jacobian is built for the translation warp only, not for SE3");
+  const ModelPlan& plan = cached_plan(*desc);
+  FwdParams fp;
+  memset(&fp, 0, sizeof(fp));
+  fp.prog = plan.fwd_warp_tangent;
+  fp.weights = (const uint8_t*)packed + plan.layout.fwd_off;
+  fp.bias = (const float*)((const uint8_t*)packed + plan.layout.bias_off);
+  fp.glo = (const float*)((const uint8_t*)packed + plan.layout.glo_off);
+  fp.points = points;
+  fp.n = B * S; fp.S = S; fp.n_embed = desc->num_embeddings;
+  fp.view_freqs = desc->view_freqs; fp.mflags = model_flags(*desc);
+  fp.S_full = S;
+  const int64_t nt = tiles_of(fp.n);
+  if (3 * nt > 0x7fffffff) return set_error(-1, "hn_mlp_fwd_warp_tangent: too many samples");
+  fp.n_tiles = (int)(3 * nt);
+  fp.x_total = plan.info.x_warp;
+  fp.x_in_ws = plan.info.x_in0; fp.x_in_t = kNone; fp.x_in_v = kNone;
+  fp.saved = (uint8_t*)tangent_saved;
+  fp.g_total = plan.info.g_warp;
+  fp.gates = (uint32_t*)((uint8_t*)primal_saved + (size_t)(2 * kSubTiles) * nt * plan.info.x_warp * kHalfChunkBytes);
+  fp.jac = jac;
+  fp.dbg = g_dbg;
+  const int grid = (int)std::min<int64_t>(3 * nt, num_sms());
+  switch (shape_of(*desc)) {
+    case 1: return launch_fwd_tangent<Cfg1>(fp, grid, stream);
+    case 2: return launch_fwd_tangent<CfgH4>(fp, grid, stream);
+    case 3: return launch_fwd_tangent<CfgH8>(fp, grid, stream);
+    default: return set_error(-13, "hn_mlp_fwd_warp_tangent: no tangent kernel for this configuration");
+  }
+}
+
 static int mlp_bwd_impl(const hn_model_desc* desc, const void* packed, const int64_t* ids, const float* sigma,
                         const float* rgb, const float* warped, const void* saved, const float* g_sigma, const float* g_rgb,
                         const float* g_warped, int64_t B, int S, const int32_t* pos, int S_full, int level,

@@ -346,6 +346,14 @@ void build_plan(const hn_model_desc& d, ModelPlan* plan) {
       slice_program(plan->fwd_train, 0, n_ws_layers, &plan->fwd_warp_train);
       plan->fwd_warp.flags |= PF_WARP_ONLY;
       plan->fwd_warp_train.flags |= PF_WARP_ONLY;
+      if (!m.se3) {
+        plan->fwd_warp_tangent = plan->fwd_warp_train;
+        plan->fwd_warp_tangent.flags |= PF_TANGENT;
+        for (int l = 0; l < plan->fwd_warp_tangent.nlayers; ++l) {
+          Layer& L = plan->fwd_warp_tangent.layers[l];
+          L.epi = L.epi == FE_RELU ? FE_TANGENT : FE_JACHEAD;
+        }
+      }
     }
   }
   // ------------------------------------------------------------------ backward-data program

@@ -232,12 +232,17 @@ struct LogicalOp {
 // FE_LINEAR on the SE3 logit columns [0, 128) plus the sheet's logit layer (64 -> H) in columns [128, 144), whose H hyper
 // coordinates the epilogue keeps for FE_WSHEAD (the next layer's 256-wide output overwrites all of ACT).  BE_LINSHEET is
 // BE_LINEAR plus the sheet head's dY (kept since BE_TRUNKIN) written to ACT[128, 144) for the (SE3 logit | sheet logit)^T layer.
-enum FwdEpi : uint8_t { FE_RELU = 0, FE_WSHEAD, FE_BOTT, FE_RGB0A, FE_RGBHEAD, FE_SIGMA, FE_SKIPFEED, FE_LINEAR, FE_LINSHEET };
+// Tangent program (ModelPlan::fwd_warp_tangent, PF_TANGENT): FE_TANGENT replaces FE_RELU — no bias, the bf16 output masked
+// with the PRIMAL sample's gate words of the layer (Layer::gate_word is read, not written); FE_JACHEAD replaces FE_WSHEAD
+// and writes jac[n, r, c] = acc[r] + (r == c), r < 3, for the launch's input direction c.
+enum FwdEpi : uint8_t { FE_RELU = 0, FE_WSHEAD, FE_BOTT, FE_RGB0A, FE_RGBHEAD, FE_SIGMA, FE_SKIPFEED, FE_LINEAR, FE_LINSHEET,
+                        FE_TANGENT, FE_JACHEAD };
 enum BwdEpi : uint8_t { BE_MASK = 0, BE_LINEAR, BE_RGB1, BE_SKIPSTORE, BE_TRUNKIN, BE_GLO, BE_LINCOND, BE_LINSHEET };
 // PF_WARP_ONLY: a warp-stage-only program (ModelPlan::fwd_warp*, bwd_warp).  Its forward ends at the FE_WSHEAD epilogue,
 // which then writes `warped` (and the SE3 screw) but no trunk input; its data gradient starts at the head^T layer, whose
 // A operand the prologue builds from the upstream g_warped instead of from the rgb head.
-enum ProgFlags : int32_t { PF_TIN_ACT = 1, PF_WARP_ONLY = 2 };   // Program::flags
+// PF_TANGENT: the bias-free gated linear pass of the translation warp stage along one input direction (hn_mlp_fwd_warp_tangent).
+enum ProgFlags : int32_t { PF_TIN_ACT = 1, PF_WARP_ONLY = 2, PF_TANGENT = 4 };   // Program::flags
 
 struct Layer {
   uint8_t op0, nops, epi, pad;
@@ -361,6 +366,9 @@ struct ModelPlan {
   // head, and their transposes, flagged PF_WARP_ONLY (hn_mlp_fwd_warp / hn_mlp_bwd_warp_*): `apply_warp` and the
   // background loss need `warped` alone, not the template behind it.
   Program fwd_warp, fwd_warp_train, bwd_warp;
+  // Translation warp only: fwd_warp_train with FE_TANGENT / FE_JACHEAD epilogues, flagged PF_WARP_ONLY | PF_TANGENT
+  // (hn_mlp_fwd_warp_tangent): the columns of the warp's Jacobian, J[:, c] = e_c + W_head D_L W_L ... D_1 W_1 dPE/dx_c.
+  Program fwd_warp_tangent;
   WgradTable wgrad_warp;    // built per call next to `wgrad`
   LogicalOps fwd_logical, bwd_logical;
   PackTable pack;     // needs param_offsets -> built per call

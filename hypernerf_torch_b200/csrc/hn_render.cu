@@ -1284,13 +1284,25 @@ extern "C" int hn_mse_loss(const float* rgb_coarse, const float* rgb_fine, const
 // the loss warp-reduced into one atomic per warp.
 // ------------------------------------------------------------------------------------------------------
 namespace hn {
+// Barron's general robust loss of a squared residual r^2 (general_loss_with_squared_residual), through expm1 / log1p so that
+// there is no cancellation at small r^2: with l = log1p(r^2 / s^2 / b), rho = (b / a) expm1(a l / 2) and
+// d rho / d r^2 = exp((a / 2 - 1) l) / (2 s^2).  Shared by the background and the elastic loss.
+struct Barron { float a, b; };
+__device__ __forceinline__ Barron barron_of(float alpha) {
+  const float eps = FLT_EPSILON;
+  const float b = fmaxf(eps, fabsf(alpha - 2.f));
+  const float a = (alpha >= 0.f ? 1.f : -1.f) * fmaxf(eps, fabsf(alpha));
+  return {a, b};
+}
+__device__ __forceinline__ float barron_log(const Barron& k, float r2, float inv_s2) { return log1pf(r2 * inv_s2 / k.b); }
+__device__ __forceinline__ float barron_rho(const Barron& k, float l) { return (k.b / k.a) * expm1f(0.5f * k.a * l); }
+__device__ __forceinline__ float barron_drho(const Barron& k, float l, float inv_s2) { return 0.5f * inv_s2 * expf((0.5f * k.a - 1.f) * l); }
+
 __global__ void __launch_bounds__(256) background_loss_kernel(const float* __restrict__ y, const float* __restrict__ pts,
                                                               int64_t n, int cols, float alpha, float inv_s2,
                                                               float grad_scale, float* __restrict__ sums,
                                                               float* __restrict__ g) {
-  const float eps = FLT_EPSILON;
-  const float b = fmaxf(eps, fabsf(alpha - 2.f));
-  const float a = (alpha >= 0.f ? 1.f : -1.f) * fmaxf(eps, fabsf(alpha));
+  const Barron k = barron_of(alpha);
   float acc = 0.f;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     float d[3], r2 = 0.f;
@@ -1299,11 +1311,10 @@ __global__ void __launch_bounds__(256) background_loss_kernel(const float* __res
       d[c] = __ldg(y + i * cols + c) - __ldg(pts + i * 3 + c);
       r2 += d[c] * d[c];
     }
-    // rho = (b / a) ((x + 1)^(a/2) - 1), x = r^2 / s^2 / b, through expm1 / log1p: no cancellation at small x
-    const float l = log1pf(r2 * inv_s2 / b);
-    acc += (b / a) * expm1f(0.5f * a * l);
+    const float l = barron_log(k, r2, inv_s2);
+    acc += barron_rho(k, l);
     if (g != nullptr) {
-      const float drho = 0.5f * inv_s2 * expf((0.5f * a - 1.f) * l);   // d rho / d r^2
+      const float drho = barron_drho(k, l, inv_s2);
 #pragma unroll
       for (int c = 0; c < 3; ++c) g[i * cols + c] = grad_scale * drho * 2.f * d[c];
       for (int c = 3; c < cols; ++c) g[i * cols + c] = 0.f;
@@ -1325,6 +1336,131 @@ extern "C" int hn_background_loss(const float* warped, const float* points, int6
   hn::background_loss_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(warped, points, n, warped_cols, alpha,
                                                                       1.f / (scale * scale), grad_scale, sums, g_warped);
   return hn::set_cuda_error(cudaGetLastError(), "hn_background_loss");
+}
+
+
+// ------------------------------------------------------------------------------------------------------
+// hn_elastic_loss — compute_elastic_loss of Nerfies (nerfies/training.py, loss_type 'log_svals') +
+// general_loss_with_squared_residual: r^2 = sum_i log^2 max(sigma_i(J), eps) of the warp's 3 x 3 Jacobian, rho(r^2) weighted
+// by the rendering weight, with its gradient seed.  The singular values come from the eigenvalues mu_i of
+// J^T J - I = D + D^T + D^T D (D = J - I), so that log sigma_i = log1p(mu_i) / 2 keeps its relative accuracy for the
+// near-identity Jacobians of a well-behaved warp.  d r^2 / dJ = J V diag(2 l_i / lambda_i [sigma_i >= eps]) V^T
+// (lambda_i = 1 + mu_i, V the eigenvectors) is the gradient of a spectral function: defined at repeated singular values.
+// One thread per sample, the loss warp-reduced into one atomic per warp.
+// ------------------------------------------------------------------------------------------------------
+namespace hn {
+// one cyclic-Jacobi rotation of the symmetric A (upper triangle used) zeroing A[P][Q]; V accumulates the rotations
+template <int P, int Q>
+__device__ __forceinline__ void jacobi_rotate(float (&A)[3][3], float (&V)[3][3]) {
+  constexpr int R = 3 - P - Q;
+  const float apq = A[P][Q];
+  if (apq == 0.f) return;
+  const float theta = (A[Q][Q] - A[P][P]) / (2.f * apq);
+  const float at = fabsf(theta);
+  float t = at > 1e18f ? 0.5f / at : 1.f / (at + sqrtf(theta * theta + 1.f));
+  t = theta < 0.f ? -t : t;
+  const float c = rsqrtf(t * t + 1.f), s = t * c;
+  A[P][P] -= t * apq;
+  A[Q][Q] += t * apq;
+  A[P][Q] = A[Q][P] = 0.f;
+  const float arp = A[R][P], arq = A[R][Q];
+  A[R][P] = A[P][R] = c * arp - s * arq;
+  A[R][Q] = A[Q][R] = s * arp + c * arq;
+#pragma unroll
+  for (int r = 0; r < 3; ++r) {
+    const float vp = V[r][P], vq = V[r][Q];
+    V[r][P] = c * vp - s * vq;
+    V[r][Q] = s * vp + c * vq;
+  }
+}
+
+__global__ void __launch_bounds__(256) elastic_loss_kernel(const float* __restrict__ jac, const float* __restrict__ wts, int64_t n,
+                                                           float alpha, float inv_s2, float eps, float grad_scale,
+                                                           float* __restrict__ sums, float* __restrict__ g, int cols) {
+  const Barron k = barron_of(alpha);
+  const float log_eps = logf(eps), eps2 = eps * eps;
+  float acc = 0.f;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    float J[3][3], D[3][3], A[3][3], V[3][3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        J[r][c] = __ldg(jac + i * 9 + r * 3 + c);
+        D[r][c] = J[r][c] - (r == c ? 1.f : 0.f);
+        V[r][c] = r == c ? 1.f : 0.f;
+      }
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+      for (int c = 0; c < 3; ++c) A[r][c] = D[r][c] + D[c][r] + D[0][r] * D[0][c] + D[1][r] * D[1][c] + D[2][r] * D[2][c];
+    // quadratic convergence: 6 sweeps take any 3 x 3 symmetric matrix to fp32 round-off
+#pragma unroll 1
+    for (int sweep = 0; sweep < 6; ++sweep) {
+      jacobi_rotate<0, 1>(A, V);
+      jacobi_rotate<0, 2>(A, V);
+      jacobi_rotate<1, 2>(A, V);
+    }
+    // lambda_m = sigma_m^2: 1 + mu_m keeps log1p's relative accuracy near sigma = 1; a small singular value is taken as
+    // |J v_m|^2 instead, whose relative error does not grow as 1 / sigma^2 like that of 1 + mu_m
+    float l[3], f[3], r2 = 0.f;
+#pragma unroll
+    for (int m = 0; m < 3; ++m) {
+      const float mu = A[m][m];
+      float lam, lg;
+      if (mu > -0.5f) {
+        lam = 1.f + mu;
+        lg = 0.5f * log1pf(mu);
+      } else {
+        lam = 0.f;
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+          const float u = J[r][0] * V[0][m] + J[r][1] * V[1][m] + J[r][2] * V[2][m];
+          lam += u * u;
+        }
+        lg = 0.5f * logf(lam);
+      }
+      const bool open = lam >= eps2;   // sigma_m >= eps
+      l[m] = open ? lg : log_eps;
+      f[m] = open ? 2.f * l[m] / lam : 0.f;
+      r2 += l[m] * l[m];
+    }
+    const float w = __ldg(wts + i);
+    const float lb = barron_log(k, r2, inv_s2);
+    acc += w * barron_rho(k, lb);
+    if (g != nullptr) {
+      const float sc = grad_scale * w * barron_drho(k, lb, inv_s2);
+      float S[3][3];   // V diag(f) V^T
+#pragma unroll
+      for (int p = 0; p < 3; ++p)
+#pragma unroll
+        for (int q = 0; q < 3; ++q) S[p][q] = V[p][0] * f[0] * V[q][0] + V[p][1] * f[1] * V[q][1] + V[p][2] * f[2] * V[q][2];
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        float* gc = g + ((int64_t)c * n + i) * cols;
+#pragma unroll
+        for (int r = 0; r < 3; ++r) gc[r] = sc * (J[r][0] * S[0][c] + J[r][1] * S[1][c] + J[r][2] * S[2][c]);
+        for (int h = 3; h < cols; ++h) gc[h] = 0.f;
+      }
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o);
+  if ((threadIdx.x & 31) == 0) atomicAdd(sums, acc);
+}
+}  // namespace hn
+
+extern "C" int hn_elastic_loss(const float* jac, const float* weights, int64_t n, float alpha, float scale, float eps,
+                               float grad_scale, float* sums, float* g_planes, int hyper_cols, void* stream) {
+  if (!jac || !weights || !sums) return hn::set_error(-2, "hn_elastic_loss: null pointer");
+  if (n <= 0) return hn::set_error(-1, "hn_elastic_loss: n must be positive");
+  if (hyper_cols < 0) return hn::set_error(-1, "hn_elastic_loss: hyper_cols must be >= 0");
+  if (!(scale > 0.f)) return hn::set_error(-1, "hn_elastic_loss: scale must be positive");
+  if (!(eps > 0.f)) return hn::set_error(-1, "hn_elastic_loss: eps must be positive");
+  const int blocks = (int)std::min<int64_t>((n + 255) / 256, 4 * (int64_t)hn::num_sms());
+  hn::elastic_loss_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(jac, weights, n, alpha, 1.f / (scale * scale), eps, grad_scale,
+                                                                   sums, g_planes, 3 + hyper_cols);
+  return hn::set_cuda_error(cudaGetLastError(), "hn_elastic_loss");
 }
 
 

@@ -96,6 +96,45 @@ def background_loss(model, points, extra_params=None, *, noise_std=1e-3, alpha=-
     return _FusedBackground.apply(warped[:, 0, :], jittered, alpha, scale, float(weight) / float(count))
 
 
+class _FusedElastic(torch.autograd.Function):
+    @staticmethod
+    @torch.amp.custom_fwd(device_type="cuda", cast_inputs=torch.float32)
+    def forward(ctx, jac, weights, alpha, scale, eps, grad_scale):
+        J = jac.contiguous()
+        w = weights.detach().contiguous()
+        n = w.numel()
+        sums = torch.zeros(1, device=J.device, dtype=torch.float32)
+        g = torch.empty(3, n, 3, device=J.device, dtype=torch.float32) if ctx.needs_input_grad[0] else None
+        check(lib().hn_elastic_loss(ptr(J), ptr(w), n, float(alpha), float(scale), float(eps), float(grad_scale), ptr(sums),
+                                    ptr(g), 0, stream()), "hn_elastic_loss")
+        _lib.count(1)
+        ctx.save_for_backward(g)
+        ctx.shape = J.shape
+        return sums[0] * grad_scale
+
+    @staticmethod
+    @torch.amp.custom_bwd(device_type="cuda")
+    def backward(ctx, g_loss):
+        g, = ctx.saved_tensors
+        # plane c of the seed holds column c of dL/dJ
+        g_jac = None if g is None else g.permute(1, 2, 0).reshape(ctx.shape) * g_loss
+        return g_jac, None, None, None, None, None
+
+
+def elastic_loss(jacobian, weights, *, alpha=-2.0, scale=0.03, eps=1e-6, weight=1.0, global_count=None):
+    """Nerfies' elastic regularisation (compute_elastic_loss with loss_type 'log_svals' and elastic_reduce_method
+    'weight'; the torch port has none): r^2 = sum_i log^2 max(sigma_i(J), eps) of the warp's Jacobians `jacobian`
+    (B, S, 3, 3) (NerfModel.forward(..., return_warp_jacobian=True)['coarse' / 'fine']['warp_jacobian']) is penalised with
+    Barron's robust loss rho(r^2, alpha, scale), weighted by the rendering weights (B, S), which take no gradient.  Returns
+    weight * sum_{b,s} w_bs rho_bs / (global_count or B) — the reference's (weights * loss).sum(-1).mean().  One fused
+    kernel computes the loss and its gradient seed; autograd takes the seed through the warp field."""
+    if jacobian.shape[-2:] != (3, 3) or jacobian.shape[:-2] != weights.shape or weights.numel() == 0:
+        raise ValueError(f"elastic_loss needs Jacobians (..., 3, 3) and weights of the leading shape, got "
+                         f"{tuple(jacobian.shape)} and {tuple(weights.shape)}")
+    count = weights.shape[0] if global_count is None else global_count
+    return _FusedElastic.apply(jacobian, weights, alpha, scale, eps, float(weight) / float(count))
+
+
 class MSELoss(nn.Module):
     """losses.py:4-14: MSE(inputs['coarse']['rgb'], targets) [+ MSE(inputs['fine']['rgb'], targets)], mean reduction."""
 

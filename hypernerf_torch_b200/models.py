@@ -236,6 +236,119 @@ class _FusedWarp(torch.autograd.Function):
                                    for i, (slot, shape, n) in enumerate(ctx.param_meta))
 
 
+_SE3_JACOBIAN = ("the SE3 warp's Jacobian is not built: its backward needs the second derivatives of the exp map; the "
+                 "fused Jacobian covers the translation warp")
+
+
+class _FusedWarpJacobian(torch.autograd.Function):
+    """The translation warp and its Jacobian, (warped (B, S, 3 + H), jac (B, S, 3, 3)) with jac[b, s, r, c] =
+    d warped_r / d points_c (JAX jacfwd's convention), on the level-0 blob.  The forward runs the warp-only primal with a
+    stash (its ReLU gates are needed even under no_grad), then hn_mlp_fwd_warp_tangent: the bias-free pass of the warp
+    stage along each input direction, gated by the primal's gates (DESIGN.md §2e).  The backward runs the primal's backward
+    for g_warped and, for g_jac, per direction c the warp stage's data gradient on the primal's gates with
+    g_warped = (g_jac[..., c], 0) and its weight gradient on tangent plane c; biases, the GLO table and the hyper sheet take
+    no gradient from J.  Gradients go into one flat fp32 buffer, or straight into the attached train.FlatGrads."""
+
+    @staticmethod
+    @torch.amp.custom_fwd(device_type="cuda", cast_inputs=torch.float32)
+    def forward(ctx, model, window, points, ids, *params):
+        if model._se3:
+            raise NotImplementedError(_SE3_JACOBIAN)
+        B, S = points.shape[0], points.shape[1]
+        dev = points.device
+        desc = model._desc
+        packed, pe_alpha = model._packed_window(0, window)
+        pts = points.detach().to(torch.float32).contiguous()
+        ids = ids.reshape(-1).to(torch.int64).contiguous()
+        if ids.numel() != B:
+            raise ValueError(f"metadata ids must have one entry per ray, got {tuple(ids.shape)} for {B} rays")
+        sizes = model._sizes(B * S)
+        warped = torch.empty(B, S, 3 + desc.hyper_dim, device=dev, dtype=torch.float32)
+        jac = torch.empty(B, S, 3, 3, device=dev, dtype=torch.float32)
+        saved = torch.empty(sizes.warp_saved_bytes, device=dev, dtype=torch.uint8)
+        need_grad = any(ctx.needs_input_grad[4:])
+        tangent = torch.empty(3 * sizes.warp_saved_bytes, device=dev, dtype=torch.uint8) if need_grad else None
+        with _lib.timed("mlp_fwd_warp", B * S):
+            check(lib().hn_mlp_fwd_warp(C.byref(desc), ptr(packed), ptr(pts), ptr(ids), B, S, ptr(warped), ptr(saved),
+                                        None, stream()), "hn_mlp_fwd_warp")
+        with _lib.timed("mlp_fwd_warp_tangent", B * S):
+            check(lib().hn_mlp_fwd_warp_tangent(C.byref(desc), ptr(packed), ptr(pts), ptr(saved), B, S, ptr(jac),
+                                                ptr(tangent), stream()), "hn_mlp_fwd_warp_tangent")
+        _lib.count(2)
+        ctx.model, ctx.shape = model, (B, S)
+        ctx.param_meta = [(slot, p.shape, p.numel()) for slot, p in zip(model._warp_slots(), params)]
+        ctx.save_for_backward(ids, saved if need_grad else None, tangent, packed, pe_alpha)
+        ctx.set_materialize_grads(False)
+        return warped, jac
+
+    @staticmethod
+    @torch.amp.custom_bwd(device_type="cuda")
+    def backward(ctx, g_warped, g_jac):
+        ids, saved, tangent, packed, pe_alpha = ctx.saved_tensors
+        model = ctx.model
+        B, S = ctx.shape
+        n = B * S
+        if g_warped is None and g_jac is None:
+            return (None,) * (4 + len(ctx.param_meta))
+        if saved is None:
+            raise RuntimeError("the warp Jacobian's backward needs the activation stashes; forward ran without grad enabled")
+        dev = saved.device
+        direct = model._flat_grads is not None and model._flat_grads.flat.device == dev
+        if direct:
+            offs, flat_grad = model._flat_offsets(), model._flat_grads.flat
+        else:
+            offs, total = model._grad_offsets()
+            flat_grad = torch.zeros(total, device=dev, dtype=torch.float32)
+        sizes = model._sizes(n)
+        work = torch.empty(sizes.warp_workspace_bytes, device=dev, dtype=torch.uint8)
+        d, L = C.byref(model._desc), lib()
+        if g_warped is not None:
+            g_warped = g_warped.to(torch.float32).contiguous()
+            with _lib.timed("mlp_dgrad_warp", n):
+                check(L.hn_mlp_bwd_warp_data(d, ptr(packed), ptr(ids), ptr(saved), ptr(g_warped), B, S, offs,
+                                             ptr(flat_grad), ptr(work), None, None, stream()), "hn_mlp_bwd_warp_data")
+            with _lib.timed("mlp_wgrad_warp", n):
+                check(L.hn_mlp_bwd_warp_weights(d, ptr(saved), B, S, offs, ptr(flat_grad), ptr(work), ptr(pe_alpha),
+                                                stream()), "hn_mlp_bwd_warp_weights")
+            _lib.count(2)
+        if g_jac is not None:
+            H = model._desc.hyper_dim
+            planes = torch.zeros(3, n, 3 + H, device=dev, dtype=torch.float32)
+            planes[:, :, :3] = g_jac.to(torch.float32).reshape(n, 3, 3).permute(2, 0, 1)
+            warp_jacobian_backward(model, packed, ids, saved, tangent, planes, B, S, offs, flat_grad, work, pe_alpha)
+        if direct:
+            return (None,) * (4 + len(ctx.param_meta))
+        return (None,) * 4 + tuple(flat_grad[offs[slot]:offs[slot] + n_].view(shape) if ctx.needs_input_grad[4 + i] else None
+                                   for i, (slot, shape, n_) in enumerate(ctx.param_meta))
+
+
+# canonical slots that take no gradient from the Jacobian (include/hypernerf_b200.h): the GLO table, every sheet and warp bias
+_JACOBIAN_NO_GRAD_SLOTS = (0,) + tuple(range(2, 29, 2))
+
+
+def warp_jacobian_backward(model, packed, ids, saved, tangent, g_planes, B, S, offs, flat_grad, work, pe_alpha):
+    """dL/dJ (given as the three g_warped planes (3, B*S, 3 + H) of hn_elastic_loss) -> the warp-field weight gradients in
+    flat_grad (offsets `offs` by slot): per input direction c, the warp stage's data gradient on the primal stash `saved`
+    with g_warped = plane c, and the weight gradient on tangent plane c of `tangent`.  The data gradient's GLO-table output
+    (products with the zero tangent of the GLO columns) goes to a scratch table."""
+    d, L = C.byref(model._desc), lib()
+    n = B * S
+    plane_bytes = model._sizes(n).warp_saved_bytes
+    scratch_offs = (C.c_int64 * _lib.HN_NUM_PARAM_TENSORS)(*([0] + [-1] * (_lib.HN_NUM_PARAM_TENSORS - 1)))
+    scratch = torch.empty(model._desc.num_embeddings * model._desc.glo_dim, device=flat_grad.device, dtype=torch.float32)
+    w_offs = (C.c_int64 * _lib.HN_NUM_PARAM_TENSORS)(*offs)
+    for slot in _JACOBIAN_NO_GRAD_SLOTS:
+        w_offs[slot] = -1
+    for c in range(3):
+        with _lib.timed("mlp_dgrad_warp_tangent", n):
+            check(L.hn_mlp_bwd_warp_data(d, ptr(packed), ptr(ids), ptr(saved), ptr(g_planes[c]), B, S, scratch_offs,
+                                         ptr(scratch), ptr(work), None, None, stream()), "hn_mlp_bwd_warp_data")
+        with _lib.timed("mlp_wgrad_warp_tangent", n):
+            check(L.hn_mlp_bwd_warp_weights(d, tangent.data_ptr() + c * plane_bytes, B, S, w_offs, ptr(flat_grad),
+                                            ptr(work), ptr(pe_alpha), stream()), "hn_mlp_bwd_warp_weights")
+    _lib.count(6)
+
+
 class _FusedTrunk(torch.autograd.Function):
     """hn_mlp_fwd_trunk / hn_mlp_bwd_trunk: the template NeRF of one level on rows whose warped point / hyper coordinates
     are given (differentiable input).  Used for the coarse depths the fine level inherits: the warp / sheet nets are
@@ -791,8 +904,8 @@ class NerfModel(PackedWeights, nn.Module):
         None) out.  One launch of the warp stage (hn_mlp_fwd_warp) on a view whose table is the given vectors."""
         if not (self.use_warp and use_warp):
             return points, None
-        if return_warp_jacobian:
-            raise NotImplementedError  # warping.py:121-122
+        if return_warp_jacobian and self._se3:
+            raise NotImplementedError(_SE3_JACOBIAN)
         if hyper_point_override is not None:
             raise NotImplementedError('hyper_point_override is not implemented.')
         if self._forward_error is not None:
@@ -801,14 +914,16 @@ class NerfModel(PackedWeights, nn.Module):
             raise NotImplementedError("distinct warp / hyper embeddings are not built (one embedding per ray)")
         view = self._embed_view(warp_embed)
         ids = torch.arange(points.shape[0], device=points.device, dtype=torch.int64)
+        if return_warp_jacobian:   # (warped, jac (B, S, 3, 3)): warping.py:115-122
+            return _FusedWarpJacobian.apply(view, pe_alphas(extra_params), points, ids, *view._warp_params())
         return _FusedWarp.apply(view, pe_alphas(extra_params), points, ids, *view._warp_params()), None
 
     def map_spatial_points(self, points, warp_embed, extra_params, use_warp=True, return_warp_jacobian=False):
         """models.py:495-512."""
         if not (self.use_warp and use_warp):
             return points, None
-        warped, _ = self.map_points(points, warp_embed, None, extra_params, use_warp, return_warp_jacobian)
-        return warped[..., :3], None
+        warped, jac = self.map_points(points, warp_embed, None, extra_params, use_warp, return_warp_jacobian)
+        return warped[..., :3], jac
 
     def map_hyper_points(self, points, hyper_embed, extra_params, hyper_point_override=None):
         """models.py:514-543: the hyper coordinates (B, S, H); None without slicing."""
@@ -848,8 +963,8 @@ class NerfModel(PackedWeights, nn.Module):
         the positions (B,S-Ni) of the remaining depths in the sorted row): see `reuse_coarse_warp`."""
         if self._forward_error is not None:
             raise RuntimeError(self._forward_error)
-        if return_warp_jacobian:
-            raise NotImplementedError  # warping.py:121-122
+        if return_warp_jacobian and self.use_warp and self._se3:
+            raise NotImplementedError(_SE3_JACOBIAN)
         if self.use_warp and not use_warp:
             # the reference hands the raw 3-channel points to a trunk built for posenc(xyz) + posenc(hyper) channels
             raise RuntimeError("use_warp=False at call time on a model built with use_warp=True: the template expects the "
@@ -886,6 +1001,9 @@ class NerfModel(PackedWeights, nn.Module):
             known_warped, pos_known, pos_new = _inherited
             sigma, rgb, warped_points = _FusedFineLevel.apply(owner, lvl, points, viewdirs, ids, noise, noise_std, known_warped,
                                                               pos_known, pos_new, *params)
+        if return_warp_jacobian and self.use_warp:
+            # models.py:650-652: the warp field's Jacobian at this level's points (for the elastic loss)
+            _, out['warp_jacobian'] = _FusedWarpJacobian.apply(owner, lvl[1], points, ids, *owner._warp_params())
         sigma = filter_sigma(points, sigma, render_opts)
         out['warped_points'] = warped_points
         comp = model_utils.volumetric_rendering(rgb, sigma, z_vals, directions,

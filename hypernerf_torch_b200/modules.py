@@ -123,10 +123,12 @@ class TranslationField(_FusedOnly):
                        hidden_init=nn.init.xavier_normal_, output_init=functools.partial(nn.init.uniform_, b=1e-4))
 
     def forward(self, points, metadata, extra_params, return_jacobian=False):
-        """warping.py:98-125: `metadata` = embedding vectors (B, S, G); returns {'warped_points': (B, S, 3)}."""
+        """warping.py:98-125: `metadata` = embedding vectors (B, S, G); returns {'warped_points': (B, S, 3)}, plus
+        'jacobian' (B, S, 3, 3) = d warped / d points with return_jacobian."""
+        warped, jac = self._owner().map_spatial_points(points, metadata, extra_params, return_warp_jacobian=return_jacobian)
         if return_jacobian:
-            raise NotImplementedError   # warping.py:121-122
-        return {'warped_points': self._owner().map_spatial_points(points, metadata, extra_params)[0]}
+            return {'warped_points': warped, 'jacobian': jac}
+        return {'warped_points': warped}
 
 
 class SE3Field(_FusedOnly):
@@ -148,6 +150,7 @@ class SE3Field(_FusedOnly):
     def forward(self, points, metadata, extra_params, return_jacobian=False):
         """warping.py:242-272 (the metadata is not an input of this field, :223-224, but selects the hyper point that the
         fused network evaluates alongside)."""
-        if return_jacobian:
-            raise NotImplementedError   # warping.py:266-271
+        if return_jacobian:   # warping.py:266-271
+            raise NotImplementedError(
+                "the SE3 warp's Jacobian is not built: its backward needs the second derivatives of the exp map")
         return {'warped_points': self._owner().map_spatial_points(points, metadata, extra_params)[0]}

@@ -122,7 +122,7 @@ def _extra(extra_params):
 
 def train_step(model, rays, rgbs, flat_grads, global_rays=None, chunk=8192, optimizer=None, return_stats=False,
                _exchange=True, extra_params=None, _window=None, background_points=None, background_weight=1.0,
-               background_noise_std=1e-3, global_background=None):
+               background_noise_std=1e-3, global_background=None, elastic_weight=0.0, elastic_scale=0.03):
     """One data-parallel training step on this rank's ray rows (B,9) / target colours (B,3).
     Returns the local contribution to the global-mean loss (sum over ranks = the reference's loss); with
     return_stats, training_step's log entries {'train/loss', 'train/psnr'} (train.py:147-163; psnr of the fine level
@@ -131,22 +131,32 @@ def train_step(model, rays, rgbs, flat_grads, global_rays=None, chunk=8192, opti
     background_points: this rank's (P, 3) known-static points: adds HyperNeRF's background loss
     (losses.background_loss with background_weight / background_noise_std) once per step, on the step's packed weights
     and windows, scaled by 1 / global_background (default P) so that the all-reduced gradient is that of the global mean;
-    it is part of the returned loss and reported as 'train/background'."""
+    it is part of the returned loss and reported as 'train/background'.
+    elastic_weight > 0: each chunk's forward also returns the warp Jacobians of both levels, and Nerfies' elastic loss
+    elastic_weight * (E_coarse + E_fine) (losses.elastic_loss with elastic_scale, mean over global_rays) joins that chunk's
+    loss before its backward; it is part of the returned loss and reported as 'train/elastic'."""
     B = rays.shape[0]
     global_rays = B if global_rays is None else global_rays
     extra = _extra(extra_params)
     flat_grads.zero()
     total = torch.zeros((), device=rays.device, dtype=torch.float32)
     fine_sq = None
+    elastic = torch.zeros((), device=rays.device, dtype=torch.float32) if elastic_weight > 0 else None
     # the weights do not change between the chunks of one step: pack the bf16 blobs once
     with model.packed_frozen(extra, _window=_window):
         for i in range(0, B, chunk):
             rows = rays[i:i + chunk]
             tgt = rgbs[i:i + chunk]
-            out = model(model_utils.prepare_ray_dict(rows), dict(extra))
+            out = model(model_utils.prepare_ray_dict(rows), dict(extra), return_warp_jacobian=elastic is not None)
             # mean over the global batch: (sum_sq(coarse) + sum_sq(fine)) / (3 * global_rays), one fused kernel that
             # also seeds both levels' gradients (losses.py:9-14)
             loss, sums = losses.mse_coarse_fine(out, tgt, global_count=3.0 * global_rays)
+            if elastic is not None:
+                e = sum(losses.elastic_loss(lv['warp_jacobian'], lv['weights'], scale=elastic_scale, weight=elastic_weight,
+                                            global_count=global_rays) for lv in out.values() if 'warp_jacobian' in lv)
+                if torch.is_tensor(e):
+                    loss = loss + e
+                    elastic += e.detach()
             loss.backward()
             total += loss.detach()
             if return_stats:
@@ -166,6 +176,8 @@ def train_step(model, rays, rgbs, flat_grads, global_rays=None, chunk=8192, opti
         stats = {'train/loss': total, 'train/psnr': -10.0 * torch.log10(fine_sq / (3.0 * B))}
         if background is not None:
             stats['train/background'] = background
+        if elastic is not None:
+            stats['train/elastic'] = elastic
         return stats
     return total
 
@@ -319,7 +331,7 @@ def save_ckpt(model, path, epoch=0, global_step=0, optimizer=None, module_name='
 
 def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=0.0, decay_step=(20,), decay_gamma=0.1,
         chunk=8192, seed=0, ckpt_path=None, log_every=0, cuda_graph=False, extra_params=None, background_points=None,
-        background_batch_size=16384, background_weight=1.0):
+        background_batch_size=16384, background_weight=1.0, elastic_weight=0.0, elastic_scale=0.03):
     """Minimal stand-in for `Trainer.fit(NeRFSystem)` (train.py:35-233) on a ray pool that is already on the device:
     per epoch one shuffled pass over (rays (P,9), rgbs (P,3)) in batches of `batch_size` (train_dataloader,
     train.py:133-138: shuffle=True; the last short batch is kept, as DataLoader's drop_last=False does), each batch
@@ -330,11 +342,15 @@ def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=
     eagerly.  extra_params: the forward's encoding-window alphas (train_step), a dict or a callable step -> dict (a
     coarse-to-fine schedule; `step` counts from 0).  background_points: this rank's shard (Q, 3) of the known-static
     points; every step draws background_batch_size of them (with replacement, from a generator seeded with seed + 1) for
-    train_step's background loss (not with cuda_graph).  Returns a list of per-step dicts {'epoch', 'step', 'lr',
-    'train/loss', 'train/psnr'[, 'train/background']} (training_step's log)."""
+    train_step's background loss (not with cuda_graph).  elastic_weight / elastic_scale: train_step's elastic loss (not
+    with cuda_graph).  Returns a list of per-step dicts {'epoch', 'step', 'lr', 'train/loss', 'train/psnr'[,
+    'train/background'][, 'train/elastic']} (training_step's log)."""
     distributed = dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
     if background_points is not None and cuda_graph:
         raise ValueError("fit: the background loss does not run in the CUDA-graph step (GraphedTrainStep); pass "
+                         "cuda_graph=False")
+    if elastic_weight > 0 and cuda_graph:
+        raise ValueError("fit: the elastic loss does not run in the CUDA-graph step (GraphedTrainStep); pass "
                          "cuda_graph=False")
     fg = FlatGrads(model.parameters())
     model.attach_flat_grads(fg)
@@ -374,7 +390,8 @@ def fit(model, rays, rgbs, num_epochs=1, batch_size=1024, lr=5e-4, weight_decay=
                                                          device=rays.device, generator=bg_gen)]
                 stats = train_step(model, r, t, fg, global_rays=world * r.shape[0], chunk=chunk, optimizer=opt,
                                    return_stats=True, extra_params=extra, background_points=bg,
-                                   background_weight=background_weight, global_background=world * background_batch_size)
+                                   background_weight=background_weight, global_background=world * background_batch_size,
+                                   elastic_weight=elastic_weight, elastic_scale=elastic_scale)
             step += 1
             log.append({'epoch': epoch, 'step': step, 'lr': opt.param_groups[0]['lr'], **stats})
             if log_every and step % log_every == 0:

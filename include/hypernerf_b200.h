@@ -269,6 +269,27 @@ int hn_mlp_bwd_warp_weights(const hn_model_desc* desc, const void* saved, int64_
 int hn_background_loss(const float* warped, const float* points, int64_t n, int warped_cols, float alpha, float scale,
                        float grad_scale, float* sums, float* g_warped, void* stream);
 
+/* Jacobian of the translation warp, jac[b, s, r, c] = d warped_r / d points_c (r, c < 3), for the nerfies elastic loss
+ * (DESIGN.md §2e).  The forward is the bias-free gated linear pass of the warp stage along each input direction c,
+ * masked by the ReLU gates of the primal's warp-only stash `primal_saved` (hn_mlp_fwd_warp with the same blob, points,
+ * ids, B, S and a stash).  tangent_saved (3 x hn_sizes.warp_saved_bytes, plane c at c x warp_saved_bytes; NULL = Jacobian
+ * only) receives each plane's X slabs in the warp-only stash layout, gate words unwritten.  The backward of a dL/dJ = G
+ * is, per plane c: hn_mlp_bwd_warp_data on `primal_saved` with g_warped = (G[:, :, c], 0_H) (its GLO-table output is
+ * not a gradient: point it at a scratch table), then hn_mlp_bwd_warp_weights on plane c of tangent_saved with the GLO
+ * and every bias offset set to -1 (biases, the GLO table and the sheet take no gradient from J).
+ * SE3, static and no-warp descriptors are rejected (-13); B and S must be positive. */
+int hn_mlp_fwd_warp_tangent(const hn_model_desc* desc, const void* packed, const float* points, const void* primal_saved,
+                            int64_t B, int S, float* jac, void* tangent_saved, void* stream);
+
+/* compute_elastic_loss of Nerfies (loss_type 'log_svals') + general_loss_with_squared_residual, for n samples with
+ * Jacobians jac (n, 3, 3) and rendering weights (n):
+ *   r^2 = sum_i log^2 max(sigma_i(J), eps),  rho(r^2) as in hn_background_loss;  sums[0] += sum w rho (caller zeroes it);
+ *   g_planes (3, n, 3 + hyper_cols): plane c, columns r < 3 = grad_scale w d rho / d r^2 (d r^2 / dJ)[r, c], the hyper
+ *   columns 0 (NULL: no gradient) — the g_warped planes of the tangent backward.
+ * n must be positive, scale and eps positive, hyper_cols >= 0. */
+int hn_elastic_loss(const float* jac, const float* weights, int64_t n, float alpha, float scale, float eps, float grad_scale,
+                    float* sums, float* g_planes, int hyper_cols, void* stream);
+
 /* losses.py:9-14 (MSELoss: mean-MSE of coarse.rgb + fine.rgb against the target colours) fused with its gradient seed and
  * with the fine-level MSE of metrics.py:4-13 (psnr = -10 log10(mse)).  sums[0] += sum (coarse - t)^2, sums[1] += sum
  * (fine - t)^2 (caller zeroes `sums`); g_level (B,3) = 2 (pred - t) * grad_scale, grad_scale = upstream / (3 B_global).
